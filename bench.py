@@ -1,6 +1,7 @@
 """bench.py — DCCF training (samples/s) and 1000-negative evaluation (users/s) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--preset electronics]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One JSON line on stdout (rank 0).  A "step" is one training batch of the reference configuration
@@ -34,6 +35,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark leaves no __pycache__ in it
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -204,6 +206,23 @@ class L2Flusher(object):
         self.buf.fill_(self.v)
 
 
+DUMP_ARRAY_BYTES = 16 * 2 ** 20     # per array: a dump has at most eight arrays, so it stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy: float64 where the path computes in float64, float32 otherwise.  An
+    array larger than DUMP_ARRAY_BYTES keeps a fixed sample of its rows, as many as fit:
+    np.sort(np.random.RandomState(SEED).choice(n_rows, n_kept, replace=False))."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            n_kept = DUMP_ARRAY_BYTES // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.RandomState(SEED).choice(a.shape[0], n_kept, replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def dist_max(x, world):
     if world == 1:
         return x
@@ -221,9 +240,10 @@ def barrier(world):
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
-def bench_train(model, X_all, steps, warmup, world, flush):
+def bench_train(model, X_all, steps, warmup, world, flush, keep_outputs=False):
     """Returns dict with device-resident timing (CUDA events per step, L2 flushed in between, max over ranks),
-    per-stage times and the end-to-end timing from pinned host buffers."""
+    per-stage times and the end-to-end timing from pinned host buffers.  keep_outputs: also 'outputs', what the last
+    timed step returned (prediction, loss) and the parameters it left, as host arrays."""
     from dccf_b200 import kernels
     dev = next(model.parameters()).device
     n = warmup + steps
@@ -246,9 +266,14 @@ def bench_train(model, X_all, steps, warmup, world, flush):
             launches0 = kernels.LAUNCHES[0]
         flush()
         ev[i][0].record()
-        step()
+        out = step()
         ev[i][1].record()
     barrier(world)
+    outputs = None
+    if keep_outputs:            # before the back-to-back and end-to-end steps below train the model further
+        outputs = {'train_prediction': out['prediction'], 'train_loss': out['loss']}
+        outputs.update(('param_' + k.replace('.', '_'), p) for k, p in model.named_parameters())
+        outputs = {k: v.detach().cpu().numpy() for k, v in outputs.items()}
     launches = kernels.LAUNCHES[0] - launches0
     per_step = [ev[i][0].elapsed_time(ev[i][1]) for i in range(max(warmup, n_first), n)]
     total_ms = dist_max(float(np.sum(per_step)) * steps / len(per_step), world)
@@ -356,11 +381,12 @@ def bench_train(model, X_all, steps, warmup, world, flush):
     sync_s = dist_max(sync_s / max(1, n_sync), world)
     return {'total_ms': total_ms, 'stage_ms': stage_ms, 'kernels_us': kernels_us, 'timeline_step_us': timeline_step_us,
             'launches': launches, 'e2e_s': e2e_s, 'e2e_sync_s_per_step': sync_s, 'b2b_ms': b2b_ms,
-            'h2d': 2 * BATCH * 2 * 8 + 2 * BATCH * S * 8, 'd2h': 4, 'last_loss': loss}
+            'h2d': 2 * BATCH * 2 * 8 + 2 * BATCH * S * 8, 'd2h': 4, 'last_loss': loss, 'outputs': outputs}
 
 
-def bench_eval(model, n_users, warm_batches, world, rank, flush):
-    """Scores n_users x 1001 candidates in eval batches of 16384 pairs and ranks them on the device."""
+def bench_eval(model, n_users, warm_batches, world, rank, flush, keep_outputs=False):
+    """Scores n_users x 1001 candidates in eval batches of 16384 pairs and ranks them on the device.  keep_outputs:
+    also 'outputs', the predictions and metrics of the last timed pass, as host arrays."""
     from dccf_b200.models.BaseModel import candidate_layout, rank_sums_device
     dev = next(model.parameters()).device
     U, I = model.user_num, model.item_num
@@ -414,8 +440,9 @@ def bench_eval(model, n_users, warm_batches, world, rank, flush):
                                         'sample_item': si_d[a:b]})['prediction'])
             e1.record()
             ev_pairs.append((e0, e1))
-        sums, ev = rank_and_sum(torch.cat(preds), flushed=True)
-        return sums, ev_pairs + [ev]
+        pred = torch.cat(preds)
+        sums, ev = rank_and_sum(pred, flushed=True)
+        return sums, ev_pairs + [ev], pred
 
     def run_from_host(X_pin):
         """public API: ids from pinned host memory, confounders drawn on the torch CPU generator per batch
@@ -437,13 +464,16 @@ def bench_eval(model, n_users, warm_batches, world, rank, flush):
     best = None
     for _ in range(2):
         barrier(world)
-        sums, evs = run_resident()
+        sums, evs, pred = run_resident()
         barrier(world)
         s_ms = sum(a.elapsed_time(b) for a, b in evs[:-1])
         r_ms = evs[-1][0].elapsed_time(evs[-1][1])
         if best is None or s_ms + r_ms < best[0] + best[1]:
             best = (s_ms, r_ms)
     score_ms, rank_ms = best
+    outputs = None
+    if keep_outputs:            # the last resident pass: every candidate's score, metric sums @5 over this rank's users
+        outputs = {'eval_prediction': pred.cpu().numpy(), 'eval_metrics': (sums / n_users).cpu().numpy()}
     dev_ms = dist_max(score_ms + rank_ms, world)
 
     # e2e: ids from pinned host memory, confounders drawn on the CPU generator per batch (as the reference),
@@ -464,7 +494,7 @@ def bench_eval(model, n_users, warm_batches, world, rank, flush):
     return {'dev_ms': dev_ms, 'score_ms': score_ms, 'rank_ms': rank_ms, 'e2e_s': e2e_s, 'rows': rows,
             'n_batches': len(bounds), 'h2d': rows * 16 + rows * S * 8, 'd2h': 40,
             'ndcg@5': float(metrics[0]), 'recall@5': float(metrics[3]), 'precision@5': float(metrics[2]),
-            'flush_s': flush_s}
+            'flush_s': flush_s, 'outputs': outputs}
 
 
 # ------------------------------------------------------------------------------------------------
@@ -962,7 +992,15 @@ def main():
     ap.add_argument('--legs', default='all',
                     help='comma list of: config3,config4,config5,eager,noise_free,projected (default all that apply)')
     ap.add_argument('--extra-legs-only', action='store_true', help='run only the child-process legs, one JSON line each')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed training step (prediction, loss, the '
+                         'parameters it left) and the last timed evaluation pass (predictions, metrics @5) computed, '
+                         'as DIR/<name>.npy (rank 0; inputs are seeded, so two builds can be compared array by array)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the GPU path computed: not available with --impl reference')
     args.warmup = max(args.warmup, 3)
     U, I = PRESETS[args.preset]
     rank = int(os.environ.get('RANK', '0'))
@@ -1039,7 +1077,7 @@ def main():
             torch.distributed.destroy_process_group()
             sys.exit(3)
 
-    def train_eval(preset, steps, warmup, eval_users):
+    def train_eval(preset, steps, warmup, eval_users, keep_outputs=False):
         """The headline pair at one shape: (model, train result, eval result, clocks)."""
         U_, I_ = PRESETS[preset]
         model = build_model(U_, I_, dev)
@@ -1048,11 +1086,14 @@ def main():
         flush = L2Flusher(dev)
         X_all = synth_batches(warmup + steps, U_, I_, SEED + rank)
         with ClockSampler(local_rank) as clocks:
-            tr = bench_train(model, X_all, steps, warmup, world, flush)
-            evl = bench_eval(model, eval_users, 3, world, rank, flush)
+            tr = bench_train(model, X_all, steps, warmup, world, flush, keep_outputs)
+            evl = bench_eval(model, eval_users, 3, world, rank, flush, keep_outputs)
         return model, tr, evl, clocks.summary()
 
-    model, tr, evl, clk = train_eval(args.preset, args.steps, args.warmup, args.eval_users)
+    keep_outputs = bool(args.dump_outputs) and rank == 0
+    model, tr, evl, clk = train_eval(args.preset, args.steps, args.warmup, args.eval_users, keep_outputs)
+    if keep_outputs:
+        dump_outputs(args.dump_outputs, dict(tr['outputs'], **evl['outputs']))
     ms_per_step = tr['total_ms'] / args.steps
     value = world * BATCH * args.steps / (tr['total_ms'] / 1e3)
     e2e_value = world * BATCH * args.steps / tr['e2e_s']

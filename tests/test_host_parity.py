@@ -116,14 +116,12 @@ def test_initial_weights_equal_reference(golden, tmp_path, name):
 
 
 def test_model_refuses_cpu(golden, tmp_path):
-    """No CPU fallback: predict on a CPU model must fail loudly."""
+    """No CPU fallback: predict on a CPU model must fail loudly, whether or not the machine has a GPU."""
     g = golden('train_f64')
     d = str(tmp_path)
     np.save(os.path.join(d, 'g_%s.npy' % SENT), g['feat'])
     np.save(os.path.join(d, 'g.ips_expo_prob.npy'), g['expo'])
     model = _make_model(d, 'g', 40, 50)
-    if torch.cuda.is_available():
-        pytest.skip('CPU-only check')
     with pytest.raises(RuntimeError, match='CUDA only'):
         model.predict({'X': torch.from_numpy(g['X_0']), 'dropout': 0.0})
 
@@ -460,13 +458,16 @@ def test_config0_host_pipeline_digest(tmp_path):
 
 
 @pytest.mark.parametrize('fixture', ['run_recmodel', 'run_recmodel_rank0'])
-def test_whole_run_equals_reference_run(golden, tmp_path, fixture):
+def test_whole_run_equals_reference_run(golden, tmp_path, fixture, monkeypatch):
     """src/main.py's whole sequence with the mirrored classes == the same sequence of the UNMODIFIED reference
     (tests/golden/run_recmodel.npz, oracle/make_golden.py::make_run_fixture; RecModel on CPU so that every number is
     reproducible): "Test Before Training", the per-epoch train / validation / test metric lists of runner.train (i.e.
     shuffles, negatives, Adam steps with l2 + clip, evaluation, model selection and the reload of the best epoch),
     "Test After Training", the final predictions and the checkpointed parameters."""
     from dccf_b200.models.RecModel import RecModel
+    # the reference ran with no CUDA device visible (oracle/ref_harness.py::cpu_shims): so does the mirrored pipeline,
+    # which would otherwise move the batches of this CPU model to a GPU of the machine
+    monkeypatch.setattr(torch.cuda, 'device_count', lambda: 0)
     g = golden(fixture)           # rank 1: top-n recommendation (BPR, sampled negatives); rank 0: rating prediction (MSE)
     seed, rank = int(g['seed']), int(g['rank'])
     synth.write_dataset(str(tmp_path), 'toy', int(g['n_users']), int(g['n_items']), int(g['per_user']), feat_dim=64,
@@ -530,7 +531,7 @@ def test_whole_run_equals_reference_run(golden, tmp_path, fixture):
         assert np.abs(v.numpy() - g['sd_' + k]).max() <= 1e-6 * np.abs(g['sd_' + k]).max(), k
 
 
-def test_whole_dccf_run_orchestration_on_cpu(golden, tmp_path):
+def test_whole_dccf_run_orchestration_on_cpu(golden, tmp_path, monkeypatch):
     """tests/golden/run_dccf.npz (a whole DCCF run of the unmodified reference, --std 0 --dropout 0) replayed on CPU
     with the MIRRORED loader, processor and runner around a stand-in for the device math (oracle/torch_port.py, the
     eager-torch port): every shuffle, negative, confounder draw, evaluation pass, Adam step, model selection and reload
@@ -538,6 +539,7 @@ def test_whole_dccf_run_orchestration_on_cpu(golden, tmp_path):
     (The GPU path replays the same fixture in tests/test_gpu_parity.py::test_whole_dccf_run_equals_reference_run.)"""
     from oracle import dccf_oracle as O
     from oracle import torch_port
+    monkeypatch.setattr(torch.cuda, 'device_count', lambda: 0)     # CPU replay on any machine, see above
 
     class PortModel(torch_port.DCCFPort):
         append_id, include_id = True, False
