@@ -10,9 +10,8 @@ import os
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-_VARIANT = os.environ.get('DCCF_LIB_VARIANT', '')          # A/B build variants, see dccf_b200/build.py
-LIB_PATH = os.path.join(HERE, 'libdccf_b200%s.so' % (('_' + _VARIANT) if _VARIANT else ''))
-ABI_VERSION = 33
+LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
+ABI_VERSION = 34
 DIM = 64
 
 
@@ -116,7 +115,7 @@ _SIGNATURES = {
     'dccf_train_fused_smem_bytes': (ctypes.c_int64, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]),
     'dccf_train_fwd_bwd_tc': (ctypes.c_int, [ctypes.POINTER(Dims), _P, _P, _P, _P, _P, ctypes.POINTER(Expo), _P, _P, _P,
                                              ctypes.c_int64, ctypes.POINTER(Rng), ctypes.c_int32, _P, _P, _P,
-                                             ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                             ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
                                              ctypes.POINTER(BatchRef), ctypes.c_int32, _P, _P]),
     'dccf_adam_sweep': (ctypes.c_int, [_P, _P, _P, ctypes.c_int64, _P, _P, ctypes.c_int64, _P, _P,
                                        ctypes.POINTER(Adam), _P]),

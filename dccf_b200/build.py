@@ -13,17 +13,11 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 INCLUDE = os.path.join(os.path.dirname(HERE), 'include')
-# Build variants for A/B experiments on the GPU box (none by default): DCCF_LIB_VARIANT=<name> builds
-# libdccf_b200_<name>.so from the same sources with the extra -D flags of DCCF_BUILD_DEFS, e.g.
-#   DCCF_LIB_VARIANT=s3 DCCF_BUILD_DEFS="-DDCCF_TRAIN_STAGES=3 -DDCCF_ADAM_SIDE_SMEM_KB=80" python -m dccf_b200.build
-# and the same DCCF_LIB_VARIANT at run time makes dccf_b200/_lib.py load it.
-VARIANT = os.environ.get('DCCF_LIB_VARIANT', '')
-_SUFFIX = ('_' + VARIANT) if VARIANT else ''
-OBJ_DIR = os.path.join(HERE, 'build' + _SUFFIX)
-LIB_PATH = os.path.join(HERE, 'libdccf_b200%s.so' % _SUFFIX)
+OBJ_DIR = os.path.join(HERE, 'build')
+LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
 
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
-              '-Xcompiler', '-fPIC', '-Xptxas', '-v'] + (os.environ.get('DCCF_BUILD_DEFS', '').split() if VARIANT else [])
+              '-Xcompiler', '-fPIC', '-Xptxas', '-v']
 
 
 def _nvcc():

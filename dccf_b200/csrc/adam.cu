@@ -9,8 +9,6 @@
 // update is a full streaming sweep (24 B/param: read p,m,v, write p,m,v).  The sparse part of the
 // gradient arrives as records (row id + 64 floats) linked per row through head/next; records of one
 // row are summed in ascending record order so the result does not depend on atomics timing.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "backdoor.cuh"
 #include "dp_sync.cuh"
@@ -344,13 +342,11 @@ __global__ void k_csr_build(const AdamAllArgs a, int phase) {
     tl_end(13);
     for (int i = 0; i < a.n_tables; ++i) {
         const AdamTableArgs& t = a.t[i];
-        // the tables' record ranges are laid out in blocks of 256 records; a launch with narrower CTAs (256 / blockDim.x of
-        // them per block) leaves room for other kernels' CTAs beside it (dccf_adam_csr_build)
-        const int per = 256 / (int)blockDim.x;
-        const int b = (int)blockIdx.x / per - t.link_lo;
+        // the tables' record ranges are laid out in blocks of 256 records, one 256-thread CTA each
+        const int b = (int)blockIdx.x - t.link_lo;
         if (b < 0 || b >= t.link_n) continue;
         if (t.csr == nullptr) return;
-        const int64_t r = (int64_t)b * 256 + ((int)blockIdx.x % per) * blockDim.x + threadIdx.x;
+        const int64_t r = (int64_t)b * 256 + threadIdx.x;
         if (r >= t.n_rec) return;
         const int32_t pos = t.next[r];
         if (pos < 0) return;                                   // (a record no link touched)
@@ -595,10 +591,7 @@ __global__ void __launch_bounds__(256) k_link_ids(const LinkIdsArgs a) {
     tl_end(0);
 }
 
-#ifndef DCCF_ADAM_SIDE_SMEM_KB
-#define DCCF_ADAM_SIDE_SMEM_KB 120          // build-time knob, see DCCF_TRAIN_STAGES in tc_train.cu
-#endif
-constexpr int ADAM_SIDE_SMEM = DCCF_ADAM_SIDE_SMEM_KB * 1024;
+constexpr int ADAM_SIDE_SMEM = 120 * 1024;     // occupancy limiter of the side-stream sweep, see dccf_adam_untouched
 
 // L2-only loads / stores: the sweep streams 100 MB past SMs whose L1 holds the feature rows of the concurrent
 // forward — it must not evict them
@@ -880,8 +873,6 @@ __global__ void __launch_bounds__(1024) k_stage_batch(const uint64_t* __restrict
 static int marshal_sync(const char* who, const dccf_dp_sync* in, DpSync* out) {
     out->world = 1; out->rank = 0; out->n_wait = 0; out->n_done = 0;
     out->loss_parts = nullptr; out->loss_stride = 0; out->n_loss = 0; out->loss_out = nullptr;
-    static const int fence_mode = [] { const char* v = getenv("DCCF_DP_FENCE"); return v != nullptr ? atoi(v) : 1; }();   // A/B knob (dp_sync.cuh)
-    out->fence_mode = fence_mode;
     out->flags = 0;
     if (in == nullptr) return DCCF_OK;
     out->flags = in->flags;
@@ -1203,17 +1194,12 @@ extern "C" int dccf_adam_untouched(const dccf_adam_table* tables, int32_t n_tabl
             }
             attr_once.mark();
         }
-        // threads_per_cta (0 = default 224; DCCF_SIDE_THREADS overrides).  The CTA has to stay resident beside the
-        // tensor-core kernels AND the middle kernel (768 threads x 64 registers = 3/4 of the register file): 7 warps x 64
-        // registers fit, 8 do not.  Measured (tools/step_timeline.py, electronics shape, L2 flushed): 128 threads swept
+        // threads_per_cta (0 = default 224).  The CTA has to stay resident beside the tensor-core kernels AND the middle
+        // kernel (768 threads x 64 registers = 3/4 of the register file): 7 warps x 64 registers fit, 8 do not.  Measured (tools/step_timeline.py, electronics shape, L2 flushed): 128 threads swept
         // the tables in 46 us — the longest chain of the step once k_link_ids had left the forward's way; a launch
         // that did not fit beside the middle kernel (160 / 192 threads at 70 registers) held that kernel back until the
         // sweep had finished (+15 us).
-        int side_threads = (threads_per_cta >= 32 && threads_per_cta <= 256) ? (threads_per_cta / 32) * 32 : 224;
-        {
-            const char* v = getenv("DCCF_SIDE_THREADS");
-            if (v != nullptr && atoi(v) >= 32 && atoi(v) <= 256) side_threads = (atoi(v) / 32) * 32;
-        }
+        const int side_threads = (threads_per_cta >= 32 && threads_per_cta <= 256) ? (threads_per_cta / 32) * 32 : 224;
         k_adam_untouched<<<(unsigned)blocks, side_threads, ADAM_SIDE_SMEM, (cudaStream_t)stream_>>>(a);
         DCCF_CHECK_LAUNCH("k_adam_untouched");
     }
@@ -1231,13 +1217,9 @@ extern "C" int dccf_adam_csr_build(const dccf_adam_table* tables, int32_t n_tabl
     for (int i = 0; i < n_tables; ++i)
         DCCF_CHECK_ARG(tables[i].csr != nullptr || (int64_t)tables[i].n_seg * tables[i].seg_len == 0, "dccf_adam_csr_build: table %d has records but no CSR buffers", i);
     if (link_blocks == 0) return DCCF_OK;
-    // CTA width: 256, or (DCCF_CSR_THREADS = 64 / 128) narrower CTAs that fit beside the middle kernel and the side sweep
-    static const int csr_threads = [] { const char* v = getenv("DCCF_CSR_THREADS"); const int t = v != nullptr ? atoi(v) : 256;
-                                        return (t == 64 || t == 128) ? t : 256; }();
-    const unsigned ctas = (unsigned)link_blocks * (256 / csr_threads);
-    k_csr_build<<<ctas, csr_threads, 0, stream>>>(a, 0);
+    k_csr_build<<<(unsigned)link_blocks, 256, 0, stream>>>(a, 0);
     DCCF_CHECK_LAUNCH("k_csr_build");
-    k_csr_build<<<ctas, csr_threads, 0, stream>>>(a, 1);
+    k_csr_build<<<(unsigned)link_blocks, 256, 0, stream>>>(a, 1);
     DCCF_CHECK_LAUNCH("k_csr_build");
     return DCCF_OK;
 }

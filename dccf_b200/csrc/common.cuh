@@ -76,16 +76,11 @@ __host__ __device__ __forceinline__ RngKey make_rng_key(uint64_t seed, uint64_t 
     return k;
 }
 
-// Rounds: 10, as curand's Philox4_32_10 behind the reference's normal_().  -DDCCF_PHILOX_ROUNDS=7 (the fewest rounds
-// that pass BigCrush, Salmon et al. table 2) exists only to MEASURE what the generator costs (build variant, see
-// dccf_b200/build.py); it defines a different stream and is not a product configuration.
-#ifndef DCCF_PHILOX_ROUNDS
-#define DCCF_PHILOX_ROUNDS 10
-#endif
+// Rounds: 10, as curand's Philox4_32_10 behind the reference's normal_().
 __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                uint32_t k0, uint32_t k1) {
 #pragma unroll
-    for (int r = 0; r < DCCF_PHILOX_ROUNDS; ++r) {
+    for (int r = 0; r < 10; ++r) {
         // one 32x32->64 multiply (IMAD.WIDE.U32) per product instead of a high and a low multiply
         uint32_t hi0, lo0, hi1, lo1;
         asm("{\n\t.reg .b64 t;\n\tmul.wide.u32 t, %2, %3;\n\tmov.b64 {%0, %1}, t;\n\t}" : "=r"(lo0), "=r"(hi0) : "r"(PHILOX_M0), "r"(c0));

@@ -53,14 +53,14 @@ constexpr int DP_PIECE4 = 256;
 // writes to the peers' memory over NVLink in large transactions.  (The first version stored from the SMs, one 16-byte
 // store per thread and peer: measured on 8 x B200, a rank's 7 MB of outgoing segments drained at ~115 GB/s and the last
 // peer saw the dW / db segment 24 us after the push kernel had ended.)  Lane p then waits for ITS copies to complete and
-// publishes the CTA's arrival on peer p with a release store: one arrival flag per (source rank, source CTA) on every
-// peer, no grid-wide counter, no second fence.  The consumer waits for all of a push's flags.
+// publishes the CTA's arrival on peer p with a relaxed store (lean protocol, dp_sync.cuh): one arrival flag per (source
+// rank, source CTA) on every peer, no grid-wide counter, no second fence.  The consumer waits for all of a push's flags.
 // FOLD: some ranges of the segment are sums of partial buffers (dW / db): sixteen float4 loads in flight per thread — a
 // register budget the plain pushes (ids, gradient records: they run beside the dW kernel and the sweep) do not pay for
 template <bool FOLD>
 __global__ void __launch_bounds__(256) k_dp_push(const float* __restrict__ send, int64_t seg, DpPeers peers, int world,
                                                  int rank, int64_t flag_off, const int32_t* __restrict__ epoch_dev,
-                                                 int32_t* cta_counter, const DpFolds folds, const bool strict) {
+                                                 int32_t* cta_counter, const DpFolds folds) {
     __shared__ __align__(128) float4 piece[DP_PIECE4];
     // debug timeline slot by what is pushed: 8 ids (small segment), 10 gradient records, 11 dW / db / loss (folded partials)
     const int tl_slot = folds.n > 0 ? 11 : (seg < 16384 ? 8 : 10);
@@ -69,7 +69,9 @@ __global__ void __launch_bounds__(256) k_dp_push(const float* __restrict__ send,
     // (the peers' consumed flags are requested together with the epoch: one round trip instead of two on the way to the
     // first copy)
     const int32_t* consumed = reinterpret_cast<const int32_t*>(peers.base[rank] + flag_off) + DP_FLAG_CONSUMED;
-    const int32_t seen = (!strict && (int)threadIdx.x < world) ? ld_relaxed_sys(consumed + threadIdx.x) : (int32_t)0x80000000;
+    // (world <= DP_MAX_WORLD already; the constant bound, tested first, keeps ptxas at 23 / 112 registers instead of 26 / 114)
+    const int32_t seen = ((int)threadIdx.x < DP_MAX_WORLD && (int)threadIdx.x < world) ? ld_relaxed_sys(consumed + threadIdx.x)
+                                                                                       : (int32_t)0x80000000;
     const int32_t epoch = __ldg(epoch_dev) + 1;
     // a consumer launched as a programmatic dependent (dccf_adam_touched, DCCF_DP_SYNC_OVERLAP_PUSH) may start once every
     // CTA of this push is resident and has read the channel's epoch (the consumer's last CTA advances it)
@@ -107,7 +109,7 @@ __global__ void __launch_bounds__(256) k_dp_push(const float* __restrict__ send,
         }
         if (!waited) {
             // peers have finished reading what this rank pushed last step (checked once per CTA, after the first loads)
-            if ((int)threadIdx.x < world && seen < epoch - 1) spin_until(consumed + threadIdx.x, epoch - 1, strict);
+            if ((int)threadIdx.x < world && seen < epoch - 1) spin_until(consumed + threadIdx.x, epoch - 1, false);
             waited = true;
         }
         tc::fence_proxy_async_smem();        // this thread's shared-memory writes -> visible to the bulk-copy engine
@@ -125,8 +127,7 @@ __global__ void __launch_bounds__(256) k_dp_push(const float* __restrict__ send,
         if (FOLD) { tl_begin(15); tl_end(15); }
         asm volatile("fence.proxy.async;" ::: "memory");
         int32_t* flag = reinterpret_cast<int32_t*>(peers.base[threadIdx.x] + flag_off) + rank * DP_MAX_CTAS + blockIdx.x;
-        if (strict) st_release_sys(flag, epoch);
-        else st_relaxed_sys(flag, epoch);        // (the copies it announces are complete: lean protocol, dp_sync.cuh)
+        st_relaxed_sys(flag, epoch);         // (the copies it announces are complete: lean protocol, dp_sync.cuh)
     }
     tl_end(tl_slot);
 }
@@ -181,7 +182,6 @@ static int dp_push_impl(const float* send, int64_t seg_floats, const uint64_t* p
     DCCF_CHECK_ARG(seg_floats > 0 && seg_floats % 4 == 0, "dccf_dp_push: segment length must be a positive multiple of 4 floats");
     DCCF_CHECK_ARG(rank >= 0 && rank < world, "dccf_dp_push: rank %d outside [0,%d)", rank, world);
     const int64_t ctas = dp_push_ctas(seg_floats);
-    static const bool strict = [] { const char* v = getenv("DCCF_DP_FENCE"); return v != nullptr && atoi(v) == 2; }();
     static PerDeviceOnce carve_once;      // (same carveout as its neighbours in the step, see dccf_adam_link_ids)
     if (carve_once.need()) {
         cudaFuncSetAttribute(k_dp_push<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -189,9 +189,9 @@ static int dp_push_impl(const float* send, int64_t seg_floats, const uint64_t* p
         carve_once.mark();
     }
     if (folds.n > 0)
-        k_dp_push<true><<<(unsigned)ctas, 256, 0, stream>>>(send, seg_floats, peers, world, rank, flag_off, epoch_dev, cta_counter, folds, strict);
+        k_dp_push<true><<<(unsigned)ctas, 256, 0, stream>>>(send, seg_floats, peers, world, rank, flag_off, epoch_dev, cta_counter, folds);
     else
-        k_dp_push<false><<<(unsigned)ctas, 256, 0, stream>>>(send, seg_floats, peers, world, rank, flag_off, epoch_dev, cta_counter, folds, strict);
+        k_dp_push<false><<<(unsigned)ctas, 256, 0, stream>>>(send, seg_floats, peers, world, rank, flag_off, epoch_dev, cta_counter, folds);
     DCCF_CHECK_LAUNCH("k_dp_push");
     return DCCF_OK;
 }

@@ -46,7 +46,6 @@ __device__ __forceinline__ void st_relaxed_sys(int32_t* p, int32_t v) {
 //   consumer -> producer, consumed flag (write-after-read): the readers' loads have returned before the last CTA's
 //     relaxed store is issued (gpu-scope fence + atomic counter between them); the producer polls it relaxed and its
 //     copies are control-dependent on what it saw.
-// DCCF_DP_FENCE=2 restores the strict forms everywhere (acquire loads, release stores, fence.sc.sys) for comparison.
 // Spin until *p >= want.  A peer that died (or never reaches this step) must not leave this GPU spinning for ever:
 // after 60 s — four orders of magnitude beyond any legitimate wait, start-up skew included — the kernel traps, the
 // process sees a CUDA error and the job fails loudly instead of hanging the box.
@@ -72,7 +71,6 @@ struct DpSync {
     int64_t loss_stride;
     int32_t n_loss;
     int32_t flags;               // dccf_dp_sync.flags
-    int32_t fence_mode;          // 1 (default) lean protocol, see above; 0 fence.acq_rel.sys after the flags; 2 strict everywhere
     float* loss_out;
 };
 
@@ -109,11 +107,7 @@ __device__ __forceinline__ void dp_wait_inline(const DpSync& s, const uint32_t m
                 __nanosleep(64);
             }
         } while (!__syncthreads_and(ok));
-        if (threadIdx.x == 0) {
-            if (s.fence_mode == 1) asm volatile("fence.acq_rel.gpu;" ::: "memory");
-            else if (s.fence_mode == 2) __threadfence_system();
-            else asm volatile("fence.acq_rel.sys;" ::: "memory");
-        }
+        if (threadIdx.x == 0) asm volatile("fence.acq_rel.gpu;" ::: "memory");
         __syncthreads();
     }
 }
@@ -139,8 +133,7 @@ __device__ __forceinline__ void dp_done_inline(const DpSync& s) {
         const DpChannel& c = s.done[t / s.world];
         const int peer = t % s.world;
         int32_t* flag = reinterpret_cast<int32_t*>(c.base[peer] + c.flag_off) + DP_FLAG_CONSUMED + s.rank;
-        if (s.fence_mode == 2) st_release_sys(flag, *c.epoch_dev + 1);
-        else st_relaxed_sys(flag, *c.epoch_dev + 1);
+        st_relaxed_sys(flag, *c.epoch_dev + 1);
     }
     __syncthreads();
     if (t < s.n_done) *s.done[t].epoch_dev += 1;

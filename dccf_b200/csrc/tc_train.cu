@@ -16,8 +16,6 @@
 //   16-byte store into the same K-major core-matrix layout the forward uses (no MN-major descriptors).
 //   dpre comes from the record role of k_bpr_bwd (bpr_bwd.cu), which also produces the embedding-gradient
 //   records and the loss.  The bias gradient falls out of the same GEMM through a column of ones at k = K.
-#include <stdlib.h>
-
 #include "backdoor.cuh"
 #include "common.cuh"
 #include "tc_common.cuh"
@@ -25,19 +23,9 @@
 
 namespace dccf {
 
-// Ring depth of the two training contractions.  Build-time knob (python -m dccf_b200.build with
-// DCCF_BUILD_DEFS="-DDCCF_TRAIN_STAGES=3 -DDCCF_ADAM_SIDE_SMEM_KB=80" DCCF_LIB_VARIANT=s3): a third stage decouples the 16
-// producer warps from the MMA issuer (DESIGN.md §8 item 1) but needs 144 KB, so the side-stream sweep's shared-memory
-// occupancy limiter has to shrink with it.  Default: the evaluation scorer's depth.
-#ifndef DCCF_TRAIN_STAGES
-#define DCCF_TRAIN_STAGES TC_STAGES
-#endif
-// Producers generate two stages per trip (four independent Philox chains per thread instead of two); wants a
-// three-stage ring.  Build-time knob like the above.
-#ifndef DCCF_TRAIN_PAIR
-#define DCCF_TRAIN_PAIR 0
-#endif
-constexpr int TT_STAGES = DCCF_TRAIN_STAGES;
+// Ring depth of the two training contractions: the evaluation scorer's depth.  (A third stage, with the side-stream
+// sweep's shared-memory limiter shrunk to make room for its 144 KB, was measured and rejected: DESIGN.md §8.)
+constexpr int TT_STAGES = TC_STAGES;
 constexpr uint32_t TT_SMEM_BYTES = TT_STAGES * TC_STAGE_BYTES + 256;
 static_assert(TT_SMEM_BYTES <= 227 * 1024, "training ring does not fit the shared memory of an SM");
 
@@ -120,7 +108,6 @@ struct TrainFwdParams {
     const int64_t* batch_cursor; //   whose base addresses are batch_ptrs[0..1] (the staged copies are written concurrently)
     const float* noise;          // mode 1
     float* pre_part;             // [n_ksplits][N][D]
-    float* x_save;               // optional [ceil(N/128)*128 * F], tile-major: Feat[i_r] + eps_r as multiplied, for the dW kernel
     int32_t* err_flag;
     int64_t n_rows;
     int32_t n_items, F, S, A, R;
@@ -130,7 +117,7 @@ struct TrainFwdParams {
 };
 
 template <int NOISE_MODE>
-__global__ void __launch_bounds__(TC_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_fwd_tc(const TrainFwdParams prm) {
+__global__ void __launch_bounds__(TC_NT, 2) k_train_fwd_tc(const TrainFwdParams prm) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + TT_STAGES * TC_STAGE_BYTES);
     uint64_t* empty_bar = full_bar + TT_STAGES;
@@ -192,7 +179,7 @@ __global__ void __launch_bounds__(TC_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_fwd_tc
 #pragma unroll
             for (int q = 0; q < 2; ++q) v[q] = ldg4(src + 4 * q);
         };
-        // chunk c's noise added to its table values (and the optional copy for the dW kernel)
+        // chunk c's noise added to its table values
         auto add_noise = [&](int c, float4 (&v)[2]) {
             const int k0 = c * TC_KC;
             if (k0 < D) return;
@@ -206,13 +193,6 @@ __global__ void __launch_bounds__(TC_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_fwd_tc
                     v[q].x = __fadd_rn(v[q].x, e.x); v[q].y = __fadd_rn(v[q].y, e.y);
                     v[q].z = __fadd_rn(v[q].z, e.z); v[q].w = __fadd_rn(v[q].w, e.w);
                 }
-            }
-            if (prm.x_save != nullptr) {
-                // tile-major copy of what is multiplied: [row tile][feature chunk][kq][row][8 floats] — a warp
-                // (32 consecutive rows, one kq) stores 1 KB contiguous
-                float* dst = prm.x_save + ((((size_t)blockIdx.x * (prm.F / TC_KC) + (size_t)(f0 / TC_KC)) * 4 + kq) * TC_BM + row) * 8;
-#pragma unroll
-                for (int q = 0; q < 2; ++q) st4(dst + 4 * q, v[q]);
             }
         };
         // stage i of this CTA's sequence: wait until the MMAs that read its slot have completed, store, publish
@@ -228,25 +208,6 @@ __global__ void __launch_bounds__(TC_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_fwd_tc
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(&full_bar[s]);
         };
-#if DCCF_TRAIN_PAIR
-        // Two stages per trip: their four Philox / Box-Muller chains are independent, so the scheduler interleaves them
-        // (the producer loop is bound by the LATENCY of its dependent chains at 4 warps per scheduler, not by issue
-        // slots: seven Philox rounds instead of ten bought 4 %), and the loads of the NEXT pair are in flight meanwhile.
-        float4 v0[2], v1[2];
-        if (n_local > 0) fetch(c_lo, v0);
-        if (n_local > 1) fetch(c_lo + 1, v1);
-        for (int i = 0; i < n_local; i += 2) {
-            const bool two = i + 1 < n_local;
-            float4 n0[2], n1[2];
-            if (i + 2 < n_local) fetch(c_lo + i + 2, n0);
-            if (i + 3 < n_local) fetch(c_lo + i + 3, n1);
-            add_noise(c_lo + i, v0);
-            if (two) add_noise(c_lo + i + 1, v1);
-            commit(i, v0);
-            if (two) commit(i + 1, v1);
-            v0[0] = n0[0]; v0[1] = n0[1]; v1[0] = n1[0]; v1[1] = n1[1];
-        }
-#else
         float4 v[2];
         if (n_local > 0) fetch(c_lo, v);
         for (int i = 0; i < n_local; ++i) {
@@ -257,7 +218,6 @@ __global__ void __launch_bounds__(TC_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_fwd_tc
             commit(i, v);
             if (i + 1 < n_local) { v[0] = vn[0]; v[1] = vn[1]; }
         }
-#endif
     } else if (warp == TC_PRODUCERS / 32) {
         // ===== MMA issuer =====
         if (lane == 0) {
@@ -288,9 +248,6 @@ __global__ void __launch_bounds__(TC_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_fwd_tc
         __syncwarp();
     }
 
-    // (DCCF_PDL_CHAIN: the middle kernel may have been launched as a programmatic dependent: its CTAs can be placed from
-    // here on, they wait for this grid's completion before they read anything)
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     // ===== epilogue: the 16 producer warps; warp w reads TMEM lanes 32*(w%4).. (the only ones it may touch) and
     // columns 16*(w/4)..: one 16-column slice of 32 rows of the partial pre-activations of this K split =====
     if (warp < TC_PRODUCERS / 32) {
@@ -447,10 +404,6 @@ __global__ void __maxnreg__(64) k_train_mid(const TrainMidParams prm) {
     float* pred_s = w_s + npc * Z;                  // [2]
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    // (DCCF_PDL_CHAIN: launched as a programmatic dependent of the partial-product kernel; the dW kernel behind this one
-    // may be placed as soon as SMs free up — both no-ops in a plain launch)
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     tl_begin(3);
     const int hw = tid >> 4, sub = tid & 15;
     const int64_t jt = blockIdx.x;
@@ -648,7 +601,6 @@ struct TrainBwdParams {
     const int64_t* sample_item;
     const float* noise;          // mode 1
     const float* dpre_rows;      // [N, D]
-    const float* x_rows;         // optional: the forward's tile-major Feat + eps copy (else regenerated here)
     float* gW_part;              // [n_splits][D][K]
     float* gb_part;              // [n_splits][D]
     const float* loss_terms;     // optional [n_loss_terms]: summed into out_loss by CTA (0,0) (fused step)
@@ -676,7 +628,7 @@ __device__ __forceinline__ void quad_transpose(float4& a, int j) {
 }
 
 template <int NOISE_MODE>
-__global__ void __launch_bounds__(TB_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_bwd_tc(const TrainBwdParams prm) {
+__global__ void __launch_bounds__(TB_NT, 2) k_train_bwd_tc(const TrainBwdParams prm) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + TT_STAGES * TC_STAGE_BYTES);
     uint64_t* empty_bar = full_bar + TT_STAGES;
@@ -703,9 +655,6 @@ __global__ void __launch_bounds__(TB_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_bwd_tc
     __syncthreads();
     tc::tc_fence_after_sync();
     const uint32_t tmem_base = *tmem_slot;
-    // (DCCF_PDL_CHAIN: barriers and tensor memory were set up while the middle kernel was still running; its outputs are
-    // read from here on)
-    asm volatile("griddepcontrol.wait;" ::: "memory");
 
     if (warp < TC_PRODUCERS / 32) {
         // ===== producers =====
@@ -731,9 +680,8 @@ __global__ void __launch_bounds__(TB_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_bwd_tc
             }
             const int64_t r = rb + rq * 4 + j;
             const bool live = r < row_hi;
-            const bool need_ids = live && (prm.x_rows == nullptr || mt == 0);
             int32_t fi = 0, it = 0;
-            if (need_ids) {
+            if (live) {
                 const uint32_t p = (uint32_t)r / (uint32_t)prm.R;
                 fi = checked_id(prm.X[2 * (int64_t)p + 1], prm.n_items, nullptr);
                 if (mt == 0) {
@@ -750,19 +698,13 @@ __global__ void __launch_bounds__(TB_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_bwd_tc
                         v[t] = ldg4(prm.E_item + (size_t)it * D + col);
                     } else if (col < prm.K) {
                         const int f = col - D;
-                        if (prm.x_rows != nullptr) {
-                            // the forward's tile-major copy (see k_train_fwd_tc)
-                            const size_t tile = (size_t)(r >> 7);
-                            v[t] = ldg4(prm.x_rows + (((tile * (prm.F / TC_KC) + (size_t)(f >> 5)) * 4 + ((f >> 3) & 3)) * TC_BM + (size_t)(r & 127)) * 8 + (f & 7));
-                        } else {
-                            v[t] = ldg4(prm.Feat + (size_t)fi * prm.F + f);
-                            if (NOISE_MODE != 0) {
-                                float4 e;
-                                if (NOISE_MODE == 1) e = ldg4(prm.noise + (size_t)r * prm.F + f);
-                                else e = noise_quad(key_noise, (uint32_t)r, (uint32_t)(f / 4), prm.noise_std);
-                                v[t].x = __fadd_rn(v[t].x, e.x); v[t].y = __fadd_rn(v[t].y, e.y);
-                                v[t].z = __fadd_rn(v[t].z, e.z); v[t].w = __fadd_rn(v[t].w, e.w);
-                            }
+                        v[t] = ldg4(prm.Feat + (size_t)fi * prm.F + f);
+                        if (NOISE_MODE != 0) {
+                            float4 e;
+                            if (NOISE_MODE == 1) e = ldg4(prm.noise + (size_t)r * prm.F + f);
+                            else e = noise_quad(key_noise, (uint32_t)r, (uint32_t)(f / 4), prm.noise_std);
+                            v[t].x = __fadd_rn(v[t].x, e.x); v[t].y = __fadd_rn(v[t].y, e.y);
+                            v[t].z = __fadd_rn(v[t].z, e.z); v[t].w = __fadd_rn(v[t].w, e.w);
                         }
                     } else if (col == prm.K) {
                         v[t].x = 1.f;                 // the column of ones: its output row is the bias gradient
@@ -792,23 +734,6 @@ __global__ void __launch_bounds__(TB_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_bwd_tc
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(&full_bar[s]);
         };
-#if DCCF_TRAIN_PAIR
-        // two stages per trip: the operands of the NEXT pair (four independent Philox chains, the loads behind their id
-        // lookups) are produced while this pair is transposed, stored and multiplied — see k_train_fwd_tc
-        float4 v0[2], v1[2], dv0, dv1;
-        if (n_st > 0) fetch(0, v0, dv0);
-        if (n_st > 1) fetch(1, v1, dv1);
-        for (int st = 0; st < n_st; st += 2) {
-            const bool two = st + 1 < n_st;
-            float4 n0[2], n1[2], dn0, dn1;
-            if (st + 2 < n_st) fetch(st + 2, n0, dn0);
-            if (st + 3 < n_st) fetch(st + 3, n1, dn1);
-            commit(st, v0, dv0);
-            if (two) commit(st + 1, v1, dv1);
-            v0[0] = n0[0]; v0[1] = n0[1]; dv0 = dn0;
-            v1[0] = n1[0]; v1[1] = n1[1]; dv1 = dn1;
-        }
-#else
         float4 v[2], dv;
         if (n_st > 0) fetch(0, v, dv);
         for (int st = 0; st < n_st; ++st) {
@@ -820,7 +745,6 @@ __global__ void __launch_bounds__(TB_NT, DCCF_TRAIN_PAIR ? 1 : 2) k_train_bwd_tc
                 v[0] = vn[0]; v[1] = vn[1]; dv = dvn;
             }
         }
-#endif
         // the scalar loss of the fused step: per-term values summed in a fixed order (lane-strided, then a shuffle
         // tree) by one warp that is idle during the epilogue
         if (warp == 4 && mt == 0 && sp == 0 && prm.loss_terms != nullptr) {
@@ -884,34 +808,10 @@ int bpr_bwd_launch(const dccf_dims* dims, const float* E_user, const float* E_it
                    float* gW_part, float* gb_part, float* gu_rec, float* gi_rec, int32_t* rec_keys_u, int32_t* rec_keys_i,
                    float* dpre_rows, bool with_gw, cudaStream_t stream);
 
-static int env_int(const char* name) {
-    const char* v = getenv(name);
-    return (v != nullptr && v[0] != '\0') ? atoi(v) : 0;
-}
-
-// DCCF_PDL_CHAIN=1: the middle kernel and the dW kernel of the fused step are launched as programmatic dependents of the
-// kernel before them (cudaLaunchAttributeProgrammaticStreamSerialization): each waits (griddepcontrol.wait) before it
-// reads its predecessor's outputs, so only launch latency and the CTA prologues overlap.
-static bool pdl_chain() {
-    static const bool on = [] { const char* v = getenv("DCCF_PDL_CHAIN"); return v != nullptr && atoi(v) != 0; }();
-    return on;
-}
-template <typename Kern, typename Prm>
-static void launch_maybe_programmatic(Kern k, dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool programmatic, const Prm& prm) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = programmatic ? 1 : 0;
-    cudaLaunchKernelEx(&cfg, k, prm);       // (errors are picked up by DCCF_CHECK_LAUNCH at the call site)
-}
-
 static int32_t fwd_ksplits_for(int64_t n_rows, int n_chunks) {
     if (n_rows <= 0) return 1;
     const int64_t tiles = (n_rows + TC_BM - 1) / TC_BM;
-    int64_t ks = env_int("DCCF_TC_KSPLITS");
-    if (ks <= 0) ks = 148 / tiles;                 // about one CTA per SM
+    int64_t ks = 148 / tiles;                      // about one CTA per SM
     if (ks > 8) ks = 8;
     if (ks > n_chunks) ks = n_chunks;
     if (ks < 1) ks = 1;
@@ -920,8 +820,7 @@ static int32_t fwd_ksplits_for(int64_t n_rows, int n_chunks) {
 
 static void bwd_geometry(int64_t n_rows, int K, int32_t* n_mtiles, int32_t* n_splits, int32_t* rows_per_split) {
     const int mt = (K + 1 + TC_BM - 1) / TC_BM;    // columns of [x | 1]
-    int64_t want = env_int("DCCF_TC_BWD_SPLITS");
-    if (want <= 0) want = 148 / mt;
+    int64_t want = 148 / mt;
     if (want < 1) want = 1;
     int64_t rps = (n_rows + want - 1) / want;
     rps = ((rps + TC_KC - 1) / TC_KC) * TC_KC;
@@ -982,7 +881,7 @@ extern "C" int32_t dccf_train_bwd_splits(int64_t n_rows, int32_t feat_dim) {
 // W images + partial products of every (row tile, K split)
 static int launch_fwd_tc(const dccf_dims* dims, const float* E_item, const float* Feat, const float* W, const int64_t* X,
                          const int64_t* sample_item, int64_t n_pairs, const dccf_rng* rng, float* ws_wimg,
-                         bool w_image_valid, float* ws_pre_part, float* x_save, int32_t* err_flag, int32_t* n_ks_out,
+                         bool w_image_valid, float* ws_pre_part, int32_t* err_flag, int32_t* n_ks_out,
                          cudaStream_t stream, const dccf_batch_ref* batch = nullptr, bool programmatic = false) {
     const int F = dims->feat_dim, K = D + F, Z = dims->n_samples + 1, R = Z * dims->n_attr;
     const int64_t n_rows = n_pairs * R;
@@ -1001,7 +900,7 @@ static int launch_fwd_tc(const dccf_dims* dims, const float* E_item, const float
     TrainFwdParams prm;
     prm.E_item = E_item; prm.Feat = Feat; prm.gWimg = ws_wimg; prm.X = X; prm.sample_item = sample_item;
     prm.batch_ptrs = batch ? batch->epoch_ptrs_dev : nullptr; prm.batch_cursor = batch ? batch->cursor_dev : nullptr;
-    prm.noise = rng->noise; prm.pre_part = ws_pre_part; prm.x_save = x_save; prm.err_flag = err_flag; prm.n_rows = n_rows;
+    prm.noise = rng->noise; prm.pre_part = ws_pre_part; prm.err_flag = err_flag; prm.n_rows = n_rows;
     prm.n_items = dims->n_items; prm.F = F; prm.S = dims->n_samples; prm.A = dims->n_attr; prm.R = R;
     prm.n_chunks = K / TC_KC; prm.noise_std = rng->noise_std;
     prm.rng.seed = rng->seed; prm.rng.offset = rng->offset; prm.rng.offset_dev = rng->offset_dev;
@@ -1031,8 +930,8 @@ static int launch_fwd_tc(const dccf_dims* dims, const float* E_item, const float
 // gW / gb partial tiles from the dpre rows (+ the scalar loss of the fused step)
 static int launch_bwd_tc(const dccf_dims* dims, const float* E_item, const float* Feat, const int64_t* X,
                          const int64_t* sample_item, int64_t n_pairs, const dccf_rng* rng, const float* ws_dpre,
-                         const float* x_rows, float* gW_part, float* gb_part, const float* loss_terms, int64_t n_loss_terms,
-                         float loss_scale, float* out_loss, cudaStream_t stream, bool programmatic = false) {
+                         float* gW_part, float* gb_part, const float* loss_terms, int64_t n_loss_terms,
+                         float loss_scale, float* out_loss, cudaStream_t stream) {
     static PerDeviceOnce attr_once;
     if (attr_once.need()) {
         int rc = opt_in_smem(k_train_bwd_tc<0>, "dccf_train_bwd_tc");
@@ -1044,7 +943,7 @@ static int launch_bwd_tc(const dccf_dims* dims, const float* E_item, const float
     const int F = dims->feat_dim, K = D + F, Z = dims->n_samples + 1, R = Z * dims->n_attr;
     TrainBwdParams prm;
     prm.E_item = E_item; prm.Feat = Feat; prm.X = X; prm.sample_item = sample_item; prm.noise = rng->noise;
-    prm.dpre_rows = ws_dpre; prm.x_rows = x_rows; prm.gW_part = gW_part; prm.gb_part = gb_part; prm.n_rows = n_pairs * R;
+    prm.dpre_rows = ws_dpre; prm.gW_part = gW_part; prm.gb_part = gb_part; prm.n_rows = n_pairs * R;
     prm.loss_terms = loss_terms; prm.out_loss = out_loss; prm.n_loss_terms = n_loss_terms; prm.loss_scale = loss_scale;
     prm.n_items = dims->n_items; prm.F = F; prm.S = dims->n_samples; prm.A = dims->n_attr; prm.R = R; prm.K = K;
     prm.noise_std = rng->noise_std;
@@ -1053,9 +952,9 @@ static int launch_bwd_tc(const dccf_dims* dims, const float* E_item, const float
     bwd_geometry(prm.n_rows, K, &n_mtiles, &n_splits, &prm.rows_per_split);
     const dim3 grid((unsigned)n_mtiles, (unsigned)n_splits);
     switch (rng->noise_mode) {
-        case 0: launch_maybe_programmatic(k_train_bwd_tc<0>, grid, dim3(TB_NT), TT_SMEM_BYTES, stream, programmatic, prm); break;
-        case 1: launch_maybe_programmatic(k_train_bwd_tc<1>, grid, dim3(TB_NT), TT_SMEM_BYTES, stream, programmatic, prm); break;
-        default: launch_maybe_programmatic(k_train_bwd_tc<2>, grid, dim3(TB_NT), TT_SMEM_BYTES, stream, programmatic, prm); break;
+        case 0: k_train_bwd_tc<0><<<grid, TB_NT, TT_SMEM_BYTES, stream>>>(prm); break;
+        case 1: k_train_bwd_tc<1><<<grid, TB_NT, TT_SMEM_BYTES, stream>>>(prm); break;
+        default: k_train_bwd_tc<2><<<grid, TB_NT, TT_SMEM_BYTES, stream>>>(prm); break;
     }
     DCCF_CHECK_LAUNCH("k_train_bwd_tc");
     return DCCF_OK;
@@ -1091,7 +990,7 @@ extern "C" int dccf_train_fwd_tc(const dccf_dims* dims, const float* E_user, con
     if (n_pairs <= 0) return DCCF_OK;
     const int Z = dims->n_samples + 1, R = Z * dims->n_attr;
     int32_t n_ks = 1;
-    rc = launch_fwd_tc(dims, E_item, Feat, W, X, sample_item, n_pairs, rng, ws_wimg, false, ws_pre_part, nullptr, err_flag,
+    rc = launch_fwd_tc(dims, E_item, Feat, W, X, sample_item, n_pairs, rng, ws_wimg, false, ws_pre_part, err_flag,
                        &n_ks, stream);
     if (rc != DCCF_OK) return rc;
 
@@ -1122,7 +1021,7 @@ extern "C" int dccf_train_bwd_tc(const dccf_dims* dims, const float* E_user, con
                             save_w, out_loss, nullptr, nullptr, gu_rec, gi_rec, rec_keys_u, rec_keys_i, ws_dpre, false,
                             stream);
     if (rc != DCCF_OK || n_pairs <= 0) return rc;
-    return launch_bwd_tc(dims, E_item, Feat, X, sample_item, n_pairs, rng, ws_dpre, nullptr, gW_part, gb_part, nullptr, 0,
+    return launch_bwd_tc(dims, E_item, Feat, X, sample_item, n_pairs, rng, ws_dpre, gW_part, gb_part, nullptr, 0,
                          1.f, nullptr, stream);
 }
 
@@ -1135,7 +1034,7 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
                                      const float* W, const float* b, const dccf_expo* expo, const int64_t* X,
                                      const int64_t* sample_item, const float* Y, int64_t n_pairs, const dccf_rng* rng,
                                      int32_t loss_mode, float* out_pred, float* out_loss, float* ws_wimg,
-                                     int32_t w_image_valid, float* ws_pre_part, float* ws_dpre, float* ws_x, float* ws_loss_terms,
+                                     int32_t w_image_valid, float* ws_pre_part, float* ws_dpre, float* ws_loss_terms,
                                      float* gW_part, float* gb_part, float* gu_rec, float* gi_rec, int32_t* rec_keys_u,
                                      int32_t* rec_keys_i, float* save_h, float* save_w, const float* expo_e,
                                      const float* expo_den, const dccf_batch_ref* batch, int32_t phases, int32_t* err_flag,
@@ -1171,7 +1070,7 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     }
     int32_t n_ks = fwd_ksplits_for(n_pairs * R, K / TC_KC);
     if (phases & 1) {
-        rc = launch_fwd_tc(dims, E_item, Feat, W, X, sample_item, n_pairs, rng, ws_wimg, w_image_valid != 0, ws_pre_part, ws_x,
+        rc = launch_fwd_tc(dims, E_item, Feat, W, X, sample_item, n_pairs, rng, ws_wimg, w_image_valid != 0, ws_pre_part,
                            err_flag, &n_ks, stream, batch, (phases & 8) != 0);
         if (rc != DCCF_OK) return rc;
     }
@@ -1191,11 +1090,11 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     mid.rng.seed = rng->seed; mid.rng.offset = rng->offset; mid.rng.offset_dev = rng->offset_dev;
     const int64_t n_terms = (loss_mode == 0) ? n_pairs / 2 : n_pairs;
     if (phases & 2) {
-        launch_maybe_programmatic(k_train_mid, dim3((unsigned)n_terms), dim3(TM_NT), smem, stream, pdl_chain(), mid);
+        k_train_mid<<<(unsigned)n_terms, TM_NT, smem, stream>>>(mid);
         DCCF_CHECK_LAUNCH("k_train_mid");
     }
     if (!(phases & 4)) return DCCF_OK;
 
-    return launch_bwd_tc(dims, E_item, Feat, X, sample_item, n_pairs, rng, ws_dpre, ws_x, gW_part, gb_part, ws_loss_terms,
-                         n_terms, loss_mode == 0 ? 1.f : 1.f / (float)n_pairs, out_loss, stream, pdl_chain());
+    return launch_bwd_tc(dims, E_item, Feat, X, sample_item, n_pairs, rng, ws_dpre, gW_part, gb_part, ws_loss_terms,
+                         n_terms, loss_mode == 0 ? 1.f : 1.f / (float)n_pairs, out_loss, stream);
 }

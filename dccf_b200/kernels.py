@@ -185,7 +185,7 @@ def train_fused_supported(n_samples, n_attr, loss_mode):
 
 
 def train_fwd_bwd_tc(dims, E_user, E_item, Feat, W, b, expo, X, sample_item, Y, rng, loss_mode, out_pred, out_loss,
-                     ws_wimg, w_image_valid, ws_pre_part, ws_dpre, ws_x, ws_loss_terms, gW_part, gb_part, gu_rec, gi_rec,
+                     ws_wimg, w_image_valid, ws_pre_part, ws_dpre, ws_loss_terms, gW_part, gb_part, gu_rec, gi_rec,
                      rec_keys_u, rec_keys_i, save_h=None, save_w=None, expo_e=None, expo_den=None, err_flag=None, phases=7,
                      batch=None):
     """Forward + BPR/MSE loss + backward of a training step: partial products, fused per-loss-term middle kernel,
@@ -202,7 +202,7 @@ def train_fwd_bwd_tc(dims, E_user, E_item, Feat, W, b, expo, X, sample_item, Y, 
     check(lib.dccf_train_fwd_bwd_tc(ctypes.byref(dims), ptr(E_user), ptr(E_item), ptr(Feat), ptr(W), ptr(b),
                                     ctypes.byref(expo), ptr(X), ptr(sample_item), ptr(Y), n_pairs, ctypes.byref(rng),
                                     int(loss_mode), ptr(out_pred), ptr(out_loss), ptr(ws_wimg), int(bool(w_image_valid)),
-                                    ptr(ws_pre_part), ptr(ws_dpre), ptr(ws_x), ptr(ws_loss_terms), ptr(gW_part), ptr(gb_part),
+                                    ptr(ws_pre_part), ptr(ws_dpre), ptr(ws_loss_terms), ptr(gW_part), ptr(gb_part),
                                     ptr(gu_rec), ptr(gi_rec), ptr(rec_keys_u), ptr(rec_keys_i), ptr(save_h), ptr(save_w),
                                     ptr(expo_e), ptr(expo_den), ctypes.byref(ref) if ref is not None else None, int(phases),
                                     ptr(err_flag), stream_ptr()),

@@ -261,10 +261,6 @@ class DCCF(DMF):
     use_tensor_cores_train = True
     # forward + loss + backward as dccf_train_fwd_bwd_tc (one fused kernel between the two contractions)
     use_fused_step = True
-    # True: the forward stores the rows Feat + eps it multiplied (tile-major, coalesced) and the dW kernel reads
-    # them back instead of regenerating the noise.  Measured: the dW kernel gains 1 us (it is not bound by the
-    # generation), the forward loses 3 us to the 17 MB of extra stores beside the Adam sweep: off.
-    reuse_noise_rows = os.environ.get('DCCF_REUSE_X', '0') != '0'
     tc_min_rows = 128 * 148
     # noise-free inference (--std 0, dropout 0, no explicit noise / mask) as a pure gather over the projected item
     # tables (dccf_score_gather) instead of the K = D + F contraction: 1.9e-7 from the general FP32 scorer and green
@@ -449,7 +445,6 @@ class DCCF(DMF):
             self.mlp[0].weight.data, self.mlp[0].bias.data, self._expo(), call['X'], call['sample_item'], Y, call['rng'],
             loss_mode, pred, rec['loss'], self._buf('ws_wimg', (kernels.train_w_image_floats(F),), torch.float32),
             w_image_valid, self._buf('ws_pre_part', (n_ks, N, D), torch.float32), self._buf('ws_dpre', (N, D), torch.float32),
-            self._buf('ws_x', ((N + 127) // 128 * 128, F), torch.float32) if self.reuse_noise_rows else None,
             self._buf('ws_loss_terms', (P,), torch.float32), rec['gW_part'], rec['gb_part'], rec['gu_rec'],
             rec['gi_rec'], rec['keys_u'], rec['keys_i'], None, None, expo_e, expo_den, self._err_flag)
         pdl = 8 if (programmatic and w_image_valid) else 0     # phase 1 beside the kernel launched just before it
@@ -769,8 +764,6 @@ class DCCF(DMF):
 
     # fused step with the optimizer split around the backward: the Adam sweep of the rows the (global) batch does not
     # touch runs on a second stream while the forward and backward run (dccf_adam_link_ids / _untouched / _touched)
-    use_split_adam = os.environ.get('DCCF_SPLIT_ADAM', '1') != '0'
-    overlap_split_adam = os.environ.get('DCCF_SPLIT_OVERLAP', '1') != '0'
 
     def _sweep_threads(self, dp):
         """Launch shape of the untouched-row Adam sweep: one small CTA per SM hidden beside the tensor-core kernels and
@@ -788,7 +781,7 @@ class DCCF(DMF):
         return (W._version, W.data_ptr(), self._param_epoch)
 
     def _split_step_ok(self, loss_mode, P=None):
-        if not (self.use_split_adam and self._fused_step_ok(loss_mode)):
+        if not self._fused_step_ok(loss_mode):
             return False
         if self._dp is None:
             return True
@@ -803,21 +796,6 @@ class DCCF(DMF):
                             group=self._dp['group'], use_p2p=self._dp.get('p2p', True))
             self._dp['ids'][P] = ix
         return ix
-
-    # k_link_ids also requests what the step will touch into L2 (rows of the tables and their Adam moments, the true
-    # items' feature rows, W with its moments and operand images): DCCF_L2_PREFETCH=0 switches it off (A/B)
-    l2_prefetch = os.environ.get('DCCF_L2_PREFETCH', '1') != '0'
-    dp_fold_sync = os.environ.get('DCCF_DP_FOLD', '1') != '0'
-    # with the folded synchronisation: table rows are swept while this rank's dW / db push is still running (A/B: =0)
-    dp_overlap_push = os.environ.get('DCCF_DP_OVERLAP_PUSH', '1') != '0'
-    # where dccf_adam_csr_build runs: beside | after_mid | before_sweep (default: by world size, see _fused_split_step)
-    csr_place = os.environ.get('DCCF_CSR_PLACE') or None
-    # data-parallel training over a device-resident epoch: every rank's ids of the WHOLE epoch (chunk) are all-gathered
-    # once, outside the steps, so no step waits for an id exchange (DCCF_DP_EPOCH_IDS=0: one id exchange per step)
-    dp_epoch_ids = os.environ.get('DCCF_DP_EPOCH_IDS', '1') != '0'
-    # k_link_ids (record lists, staging of a resident batch, exposure softmax) on the side stream, beside the forward
-    # instead of ahead of it (DCCF_LINK_BESIDE=0: ahead, as in round 1)
-    link_beside_forward = os.environ.get('DCCF_LINK_BESIDE', '1') != '0'
 
     def _fused_split_step(self, call, loss_mode, Y, opt, hp, w_image_valid, overlap, counters=None, stage=None,
                           epoch_ids=None):
@@ -839,7 +817,6 @@ class DCCF(DMF):
         if opt.__dict__.get('cta_counter') is None:
             opt.cta_counter = torch.zeros(1, dtype=torch.int32, device=self.uid_embeddings.weight.device)
         main = torch.cuda.current_stream()
-        overlap = overlap and self.overlap_split_adam
         expo_e = self._buf('ws_expo_e', (P, self.sample_num + 1), torch.float32)
         expo_den = self._buf('ws_expo_den', (P,), torch.float32)
         dp = 'exchange' in rec
@@ -849,27 +826,22 @@ class DCCF(DMF):
 
         # The exposure softmax of the local pairs (read by the middle kernel) and, on one GPU, the record lists: first,
         # on the main stream.  (On the side stream this kernel would run beside the first CTAs of the partial-product
-        # kernel — measured: that kernel then takes 22 us instead of 13.)
+        # kernel — measured: that kernel then takes 22 us instead of 13.)  k_link_ids also requests what the step will
+        # touch into L2: rows of the tables and their Adam moments, the true items' feature rows, W with its moments and
+        # operand images.
         eu, ei = self.uid_embeddings.weight.data, self.iid_embeddings.weight.data
         W = self.mlp[0].weight.data
-        pf_user = (eu, opt.exp_avg['E_user'], opt.exp_avg_sq['E_user']) if self.l2_prefetch else None
-        pf_item = (ei, opt.exp_avg['E_item'], opt.exp_avg_sq['E_item']) if self.l2_prefetch else None
+        pf_user = (eu, opt.exp_avg['E_user'], opt.exp_avg_sq['E_user'])
+        pf_item = (ei, opt.exp_avg['E_item'], opt.exp_avg_sq['E_item'])
         rec_rows = (self._ws['rec_row_u'], self._ws['rec_row_i']) if csr else None      # (allocated by _step_tables)
-        extra = None
-        if not dp and (self.l2_prefetch or stage is not None or csr):
+        if not dp:
             extra = kernels.make_link_extra(
                 stage=stage, prefetch_user=pf_user, prefetch_item=pf_item, rec_rows=rec_rows,
-                prefetch_feat=self.feature_embedding if self.l2_prefetch else None,
-                prefetch_dense=(wimg, W, opt.exp_avg['W'], opt.exp_avg_sq['W']) if self.l2_prefetch else None)
-        elif dp and (stage is not None or self.l2_prefetch):
+                prefetch_feat=self.feature_embedding, prefetch_dense=(wimg, W, opt.exp_avg['W'], opt.exp_avg_sq['W']))
+        else:
             # data parallel: the local launch stages the batch (device-resident epoch) and evaluates the exposure softmax;
             # the record lists of the GLOBAL step are linked on the side stream
-            extra = kernels.make_link_extra(stage=stage, prefetch_feat=self.feature_embedding if self.l2_prefetch else None,
-                                            prefetch_dense=(wimg,) if self.l2_prefetch else None)
-
-        def link_local():
-            kernels.adam_link_ids(self._dims(), call['X'], call['sample_item'], opt.head_u, next_u, opt.head_i, next_i,
-                                  self._expo(), expo_e, expo_den, n_seg=0 if dp else 1, extra=extra)
+            extra = kernels.make_link_extra(stage=stage, prefetch_feat=self.feature_embedding, prefetch_dense=(wimg,))
 
         # The forward needs nothing this launch produces except — with a device-resident epoch — the staged ids, and
         # those it can read from the epoch arrays itself (dccf_batch_ref): it is launched as a PROGRAMMATIC DEPENDENT of
@@ -877,35 +849,29 @@ class DCCF(DMF):
         # forward does not complete before this kernel has, so the middle kernel still finds the exposure softmax and
         # the staged ids.  (A first version put this launch on the side stream: same overlap, but a graph with two root
         # nodes and a cross-stream edge into the middle kernel started 3 us later and left 2 us wider gaps.)
-        beside = overlap and self.link_beside_forward and w_image_valid
+        beside = overlap and w_image_valid
         batch = (stage[0], stage[1]) if (stage is not None and beside) else None
-        link_local()
-
-        # data parallel, folded synchronisation (DCCF_DP_FOLD=0: the round-1 sequence push / wait / consume / done as
-        # separate launches): consumers wait for the peers' segments in their own prologue and their last CTA hands the
-        # buffers back — four launches fewer on the main stream of every step
-        fold = dp and self.dp_fold_sync
+        kernels.adam_link_ids(self._dims(), call['X'], call['sample_item'], opt.head_u, next_u, opt.head_i, next_i,
+                              self._expo(), expo_e, expo_den, n_seg=0 if dp else 1, extra=extra)
 
         def link_global():
-            # data parallel: every rank's ids, then the record lists of the GLOBAL step
+            # data parallel: every rank's ids, then the record lists of the GLOBAL step.  The synchronisation is folded
+            # into the consumers: they wait for the peers' segments in their own prologue and their last CTA hands the
+            # buffers back.
             pf = dict(prefetch_user=pf_user, prefetch_item=pf_item,
-                      prefetch_dense=(W, opt.exp_avg['W'], opt.exp_avg_sq['W'])) if self.l2_prefetch else {}
+                      prefetch_dense=(W, opt.exp_avg['W'], opt.exp_avg_sq['W']))
             if epoch_ids is not None:
                 # every rank's ids of the whole epoch were gathered once (begin_resident_epoch): no id exchange in the step
                 kernels.adam_link_ids(self._dims(), None, None, opt.head_u, next_u, opt.head_i, next_i, n_pairs=P,
                                       n_seg=ex.world, seg_stride=0, user_seg=-1 if ex.user_records else ex.rank,
                                       extra=kernels.make_link_extra(epoch_global=epoch_ids, rec_rows=rec_rows, **pf))
                 return
-            if fold:
-                ix.push()
-                if opt.__dict__.get('link_counter') is None:
-                    opt.link_counter = torch.zeros(1, dtype=torch.int32, device=eu.device)
-                ids = ix.recv.view(torch.int64)
-                extra_g = kernels.make_link_extra(sync=kernels.make_dp_sync(ix.world, ix.rank, wait=(ix,), done=(ix,)),
-                                                  counter=opt.link_counter, rec_rows=rec_rows, **pf)
-            else:
-                ids = ix.exchange().view(torch.int64)
-                extra_g = kernels.make_link_extra(rec_rows=rec_rows, **pf) if (pf or csr) else None
+            ix.push()
+            if opt.__dict__.get('link_counter') is None:
+                opt.link_counter = torch.zeros(1, dtype=torch.int32, device=eu.device)
+            ids = ix.recv.view(torch.int64)
+            extra_g = kernels.make_link_extra(sync=kernels.make_dp_sync(ix.world, ix.rank, wait=(ix,), done=(ix,)),
+                                              counter=opt.link_counter, rec_rows=rec_rows, **pf)
             kernels.adam_link_ids(self._dims(), ids, ids[ix.si_off_i64:], opt.head_u, next_u, opt.head_i, next_i,
                                   n_pairs=P, n_seg=ix.world, seg_stride=ix.seg_i64,
                                   user_seg=-1 if ex.user_records else ix.rank, extra=extra_g)
@@ -923,57 +889,32 @@ class DCCF(DMF):
             with torch.cuda.stream(side):
                 if dp:                      # the id exchange waits for the peers: never on the critical path
                     link_global()
-                # The CSR ranges of the step's record lists (two small launches; the touched-row sweep that needs them
-                # runs after the backward).  'beside' (default): on a third stream as soon as the lists are linked, beside
-                # the sweep and the forward — done before the middle kernel starts at 1-2 ranks.  At 8 ranks (8 x the
-                # records) they are still resident when the middle kernel wants its SMs (sweep CTA + CSR CTA + middle
-                # CTA exceed the register file) and that kernel ends 7 us later than on one GPU; the alternatives measured
-                # on 8 x B200 move the cost instead of removing it — 'after_mid' (a fourth stream, once the middle
-                # kernel has ended, beside the dW kernel and the record push: the dW kernel then takes 27 us instead of 23,
-                # 107.6 us per step against 105.4), DCCF_CSR_THREADS=64 (narrower CTAs: 106.5), 'before_sweep' (ahead of
-                # the sweep on this stream: the sweep then runs under the dW kernel, +6 us at 2 ranks).
-                csr_place = self.csr_place or 'beside'
-                if not csr or (csr_place == 'after_mid' and not dp):
-                    csr_place = 'beside' if csr else None
-                if csr_place == 'before_sweep':
-                    kernels.adam_csr_build(tables)
-                elif csr_place is not None:
+                if csr:
                     linked = torch.cuda.Event()
                     linked.record(side)
                 kernels.adam_untouched(tables, hp, self._sweep_threads(dp and epoch_ids is None))
-                if dp and not fold and epoch_ids is None:
-                    ix.done()
                 done.record(side)
+            # The CSR ranges of the step's record lists (two small launches; the touched-row sweep that needs them runs
+            # after the backward): on a third stream as soon as the lists are linked, beside the sweep and the forward —
+            # done before the middle kernel starts at 1-2 ranks.  At 8 ranks they are still resident when the middle
+            # kernel wants its SMs and that kernel ends 7 us later than on one GPU; the other placements measured on
+            # 8 x B200 moved that cost instead of removing it (DESIGN.md §8).
             csr_done = None
-            if csr_place == 'beside':
+            if csr:
                 csr_done = torch.cuda.Event()
                 ship.wait_event(linked)
                 with torch.cuda.stream(ship):
                     kernels.adam_csr_build(tables)
                     csr_done.record(ship)
-            elif csr_place == 'after_mid':
-                csr_done = torch.cuda.Event()
-                if d.get('_aux_stream') is None:
-                    d['_aux_stream'] = torch.cuda.Stream(device=main.device)
-                aux = d['_aux_stream']
             if dp:
                 mid_done, shipped = torch.cuda.Event(), torch.cuda.Event()
 
                 def between(phase):        # noqa: E306  the gradient records leave while the dW kernel runs
                     if phase == 2:
                         mid_done.record(main)
-                        if csr_place == 'after_mid':
-                            aux.wait_event(mid_done)
-                            aux.wait_event(linked)
-                            with torch.cuda.stream(aux):
-                                kernels.adam_csr_build(tables)
-                                csr_done.record(aux)
                         ship.wait_event(mid_done)
                         with torch.cuda.stream(ship):
-                            if fold:
-                                ex.rec.push()
-                            else:
-                                ex.exchange_records()
+                            ex.rec.push()
                             shipped.record(ship)
         else:
             if dp:
@@ -981,20 +922,11 @@ class DCCF(DMF):
             kernels.adam_untouched(tables, hp, self._sweep_threads(dp and epoch_ids is None))
             if csr:
                 kernels.adam_csr_build(tables)
-            if dp and not fold and epoch_ids is None:
-                ix.done()
         pred, rec = self._launch_fwd_bwd(call, loss_mode, Y, rec=rec, w_image_valid=w_image_valid, expo_e=expo_e,
                                          expo_den=expo_den, between=between, batch=batch, programmatic=beside)
         sync = None
-        joined = False
         if dp:
-            if not overlap:
-                if fold:
-                    ex.rec.push()
-                else:
-                    ex.exchange_records()
-            overlap_push = fold and self.dp_overlap_push
-            if overlap and overlap_push:
+            if overlap:
                 # The touched-row sweep is launched as a programmatic dependent of the dW / db push and starts beside it:
                 # everything else it depends on (record push, side sweep, CSR ranges) is joined BEFORE the push, which
                 # is then its only — programmatic — predecessor.  (All three end long before the dW kernel does.)
@@ -1002,17 +934,15 @@ class DCCF(DMF):
                 main.wait_event(done)
                 if csr_done is not None:
                     main.wait_event(csr_done)
-                joined = True
-            self._exchange_dense(rec, push_only=fold)
-            if overlap and not joined:
-                main.wait_event(shipped)
-            if fold:
-                total = self._buf('dp_total_loss', (1,), torch.float32)
-                a_loss, _ = ex.off['loss']
-                sync = kernels.make_dp_sync(ex.world, ex.rank, wait=(ex.rec, ex.dense), done=(ex.rec, ex.dense),
-                                            loss=(ex.dense.recv[a_loss:], ex.dense.seg, ex.world, total),
-                                            flags=kernels.DP_SYNC_OVERLAP_PUSH if (overlap_push and overlap) else 0)
-        if overlap and not joined:
+            else:
+                ex.rec.push()
+            self._exchange_dense(rec, push_only=True)
+            total = self._buf('dp_total_loss', (1,), torch.float32)
+            a_loss, _ = ex.off['loss']
+            sync = kernels.make_dp_sync(ex.world, ex.rank, wait=(ex.rec, ex.dense), done=(ex.rec, ex.dense),
+                                        loss=(ex.dense.recv[a_loss:], ex.dense.seg, ex.world, total),
+                                        flags=kernels.DP_SYNC_OVERLAP_PUSH if overlap else 0)
+        elif overlap:
             main.wait_event(done)
             if csr_done is not None:
                 main.wait_event(csr_done)
@@ -1020,11 +950,7 @@ class DCCF(DMF):
         kernels.adam_touched(tables, dense, hp, True, wimg, 0, D + F, opt.cta_counter, step_dev, offset_dev, sync=sync,
                              advance_cursor_dev=stage[1] if stage is not None else None)
         if dp:
-            if fold:
-                return pred, total[0]
-            loss = ex.total_loss()
-            ex.done()
-            return pred, loss
+            return pred, total[0]
         return pred, rec['loss'][0]
 
     def train_step(self, feed_dict, opt=None, stage_events=None):
@@ -1113,19 +1039,16 @@ class DCCF(DMF):
             loss_mode = 0 if rank_mode == 1 else 1
             Yg = g['Y'] if rank_mode != 1 else None
             split = self._split_step_ok(loss_mode, P)
-            # a batch read from a device-resident epoch: fetched by k_link_ids itself on one GPU (each linking thread
-            # copies the id it links), by a launch of its own otherwise (the id exchange pushes the staged buffers)
-            # the id exchange pushes the staged buffers; with the epoch-wide id gather (dp_epoch_ids) there is none)
-            epoch_ids = staged and split and self._dp is not None and self.dp_epoch_ids
-            stage_in_link = staged and split and (self._dp is None or epoch_ids)
-            if staged and not stage_in_link:
+            # a batch read from a device-resident epoch: fetched by k_link_ids itself in the split step (each linking
+            # thread copies the id it links; data parallel, every rank's ids of the whole epoch were gathered once, so
+            # the step has no id exchange), by a launch of its own otherwise
+            epoch_ids = staged and split and self._dp is not None
+            if staged and not split:
                 kernels.stage_batch(g['epoch_ptrs'], g['cursor'], P, S, g['X'], g['si'])
             if split:
                 # the W operand images are kept current by dccf_adam_touched (checked before every replay)
-                stage = None
-                if stage_in_link:
-                    stage = (g['epoch_ptrs'], g['cursor'], g['X'], g['si'], g['stage_counter'])
-                g['epoch_ids'] = bool(epoch_ids)
+                stage = (g['epoch_ptrs'], g['cursor'], g['X'], g['si'], g['stage_counter']) if staged else None
+                g['epoch_ids'] = epoch_ids
                 pred, loss = self._fused_split_step(call, loss_mode, Yg, opt, hp, True, overlap=True,
                                                     counters=(g['step_dev'], g['offset_dev']), stage=stage,
                                                     epoch_ids=(g['epoch_ptrs'], g['cursor']) if epoch_ids else None)
@@ -1142,8 +1065,7 @@ class DCCF(DMF):
         # later, larger call would replace and free), the optimizer state and the exchange buffers stay referenced
         # from the graph entry for as long as the graph can be replayed.
         keep = {'ws': dict(self._ws), 'opt': opt, 'err_flag': self._err_flag,
-                'streams': (self.__dict__.get('_side_stream'), self.__dict__.get('_ship_stream'),
-                            self.__dict__.get('_aux_stream'))}
+                'streams': (self.__dict__.get('_side_stream'), self.__dict__.get('_ship_stream'))}
         if self._dp is not None:
             keep['dp'] = (dict(self._dp.get('ex', {})), dict(self._dp.get('ids', {})))
         g.update({'graph': graph, 'pred': pred, 'loss': loss, 'call': call, 'keep_alive': keep,

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 33
+#define DCCF_ABI_VERSION 34
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -192,8 +192,7 @@ int dccf_train_bwd_tc(const dccf_dims* dims, const float* E_user, const float* E
  * d loss / d pred, dpre rows, embedding-gradient records — with BPR a CTA owns the positive pair j and its
  * negative j + P/2), then the dW / db tiles (whose CTA (0,0) also sums the loss terms in a fixed order).
  *   w_image_valid != 0: ws_wimg already holds the operand images of the current W (dccf_adam_step wrote them)
- *   ws_x [ceil(N/128)*128 * F] optional workspace: the forward stores the rows Feat[i] + eps it multiplied (tile-major)
- *        and the dW kernel reads them back (L2-resident) instead of regenerating the noise; NULL: regenerated
+ *   the dW kernel regenerates the rows Feat[i] + eps the forward multiplied (same noise stream), it stores none
  *   ws_loss_terms [P/2] (BPR) or [P] (MSE) workspace;  save_h / save_w optional (NULL: not written)
  *   expo_e [P, Z] / expo_den [P] optional: the exposure softmax precomputed by dccf_adam_link_ids
  *   phases: mask of 1 = the partial products, 2 = the middle kernel, 4 = the dW / db tiles (7 = everything; same
@@ -202,7 +201,8 @@ int dccf_train_bwd_tc(const dccf_dims* dims, const float* E_user, const float* E
  *        + 8: the partial-product kernel is launched as a PROGRAMMATIC DEPENDENT of the kernel before it on the stream
  *        (cudaLaunchAttributeProgrammaticStreamSerialization): it starts as soon as that kernel — dccf_adam_link_ids,
  *        which signals griddepcontrol.launch_dependents first thing — has started, reads nothing it writes (use
- *        `batch` when the ids are being staged by it) and does not complete before it has; needs w_image_valid
+ *        `batch` when the ids are being staged by it) and does not complete before it has; needs w_image_valid.
+ *        The middle kernel and the dW / db kernel are always plain launches
  *   batch (optional): the partial-product kernel (phase 1) takes its ids from batch *cursor_dev of a device-resident
  *        epoch (epoch_ptrs_dev[0..1] = base addresses of X_epoch [n, P, 2] / sample_epoch [n, P, S], the arrays
  *        dccf_link_extra's staging reads) instead of X / sample_item — it then does not have to wait for the launch
@@ -216,7 +216,7 @@ int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user, const floa
                           const float* W, const float* b, const dccf_expo* expo, const int64_t* X,
                           const int64_t* sample_item, const float* Y, int64_t n_pairs, const dccf_rng* rng,
                           int32_t loss_mode, float* out_pred, float* out_loss, float* ws_wimg,
-                          int32_t w_image_valid, float* ws_pre_part, float* ws_dpre, float* ws_x, float* ws_loss_terms,
+                          int32_t w_image_valid, float* ws_pre_part, float* ws_dpre, float* ws_loss_terms,
                           float* gW_part, float* gb_part, float* gu_rec, float* gi_rec, int32_t* rec_keys_u,
                           int32_t* rec_keys_i, float* save_h, float* save_w, const float* expo_e,
                           const float* expo_den, const dccf_batch_ref* batch, int32_t phases, int32_t* err_flag,

@@ -109,26 +109,24 @@ def test_gather_scorer_schedule_emulated(P, S, A, ipsmf):
 # ---------------------------------------------------------------------------------------------------------
 # Index arithmetic of two optimizer kernels whose launch shapes changed late in round 2 (adam.cu)
 # ---------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize('cta_threads', [256, 128, 64])
 @pytest.mark.parametrize('n_rec', [(1, 1), (256, 2816), (2048, 22528), (300, 0), (257, 513)])
-def test_csr_build_narrow_ctas_visit_every_record_once(cta_threads, n_rec):
+def test_csr_build_ctas_visit_every_record_once(n_rec):
     """k_csr_build: the tables' record ranges are laid out in blocks of 256 records (link_lo / link_n, marshal_adam);
-    dccf_adam_csr_build may launch 256 / blockDim.x narrower CTAs per block (DCCF_CSR_THREADS).  Transcription of the
-    kernel's mapping blockIdx.x, threadIdx.x -> (table, record): every record of every table exactly once, nothing else."""
+    dccf_adam_csr_build launches one 256-thread CTA per block.  Transcription of the kernel's mapping blockIdx.x,
+    threadIdx.x -> (table, record): every record of every table exactly once, nothing else."""
     tables, lo = [], 0
     for n in n_rec:                                   # marshal_adam: link_n = ceil(n_rec / 256) blocks per table
         link_n = (n + 255) // 256
         tables.append({'n_rec': n, 'link_lo': lo, 'link_n': link_n})
         lo += link_n
     link_blocks = lo
-    per = 256 // cta_threads
     seen = [np.zeros(t['n_rec'], dtype=np.int64) for t in tables]
-    for block in range(link_blocks * per):            # ctas = link_blocks * (256 / csr_threads)
+    for block in range(link_blocks):
         for i, t in enumerate(tables):
-            b = block // per - t['link_lo']
+            b = block - t['link_lo']
             if b < 0 or b >= t['link_n']:
                 continue
-            r = b * 256 + (block % per) * cta_threads + np.arange(cta_threads)
+            r = b * 256 + np.arange(256)
             r = r[r < t['n_rec']]
             seen[i][r] += 1
             break                                     # (the kernel returns after the table that owns the block)

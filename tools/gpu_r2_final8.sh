@@ -1,7 +1,5 @@
 #!/bin/bash
-# Round 2, final 8-GPU call: two short runs to place dccf_adam_csr_build at 8 ranks (after the middle kernel on a fourth
-# stream / beside the sweep with 64-thread CTAs; beside with 256-thread CTAs measured 104.5 us per step in call U), then the
-# full bench line (every leg) with the faster of the two.
+# Round 2, final 8-GPU call: the full bench line (every leg) at 8 ranks.
 mkdir -p gpurun_out
 TR="python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29533"
 show() {
@@ -19,25 +17,5 @@ except Exception as e:
     print(sys.argv[1], 'parse failed', e)
 P
 }
-DCCF_CSR_PLACE=after_mid timeout 300 $TR bench.py --gpus 8 --steps 50 --warmup 5 --no-extra-legs --eval-users 128 > gpurun_out/bench_r2_dp8_after_mid.json 2> gpurun_out/bench_r2_dp8_after_mid.err; echo rc=$?; show gpurun_out/bench_r2_dp8_after_mid.json
-DCCF_CSR_PLACE=beside DCCF_CSR_THREADS=64 timeout 300 $TR bench.py --gpus 8 --steps 50 --warmup 5 --no-extra-legs --eval-users 128 > gpurun_out/bench_r2_dp8_beside64.json 2> gpurun_out/bench_r2_dp8_beside64.err; echo rc=$?; show gpurun_out/bench_r2_dp8_beside64.json
-BEST=$(python - <<'P'
-import json
-def ms(p):
-    try:
-        return json.loads(open(p).read().strip().splitlines()[-1])['ms_per_step']
-    except Exception:
-        return 1e9
-a, b = ms('gpurun_out/bench_r2_dp8_after_mid.json'), ms('gpurun_out/bench_r2_dp8_beside64.json')
-best = min((a, 'after_mid'), (b, 'beside64'), (0.10452, 'beside'))
-print(best[1])
-P
-)
-echo "BEST=$BEST"
-case $BEST in
-  after_mid) export DCCF_CSR_PLACE=after_mid;;
-  beside64) export DCCF_CSR_PLACE=beside DCCF_CSR_THREADS=64;;
-  *) export DCCF_CSR_PLACE=beside;;
-esac
 DCCF_BENCH_RANK_TIMELINES=1 timeout 900 $TR bench.py --gpus 8 --steps 100 --warmup 5 > gpurun_out/bench_r2_dp8.json 2> gpurun_out/bench_r2_dp8.err; echo rc=$?; grep '"rank"' gpurun_out/bench_r2_dp8.err | cut -c1-700 | head -3; tail -c 300 gpurun_out/bench_r2_dp8.err; show gpurun_out/bench_r2_dp8.json
 nvidia-smi --query-gpu=index,clocks.sm,clocks.max.sm,power.draw,temperature.gpu --format=csv,noheader | head -3

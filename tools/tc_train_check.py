@@ -63,11 +63,10 @@ def run(path, t, X, si, F, S, A, rng, time_it=0):
     gW_part, gb_part = torch.zeros(ns, D, K, **f32), torch.zeros(ns, D, **f32)
     if path == 'fused':
         terms = torch.zeros(P, **f32)
-        xs = torch.zeros((N + 127) // 128 * 128, F, **f32)
 
         def step():
             kernels.train_fwd_bwd_tc(dims, t['E_user'], t['E_item'], t['Feat'], t['W'], t['b'], expo, X, si, None, rng, 0,
-                                     pred, loss, wimg, False, pre_part, dpre, xs, terms, gW_part, gb_part, gu, gi, ku, ki,
+                                     pred, loss, wimg, False, pre_part, dpre, terms, gW_part, gb_part, gu, gi, ku, ki,
                                      save_h, save_w, None, None, None)
         step()
         torch.cuda.synchronize()
