@@ -11,7 +11,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
-ABI_VERSION = 34
+ABI_VERSION = 35
 DIM = 64
 
 
@@ -41,7 +41,7 @@ class Rng(ctypes.Structure):
 class Adam(ctypes.Structure):
     _fields_ = [('lr', ctypes.c_double), ('beta1', ctypes.c_double), ('beta2', ctypes.c_double),
                 ('eps', ctypes.c_double), ('l2', ctypes.c_double), ('weight_decay', ctypes.c_double),
-                ('clip', ctypes.c_double), ('step', ctypes.c_int32), ('_pad', ctypes.c_int32),
+                ('clip', ctypes.c_double), ('step', ctypes.c_int32), ('rule', ctypes.c_int32),
                 ('step_dev', ctypes.c_void_p)]
 
 

@@ -5,8 +5,9 @@
 //   clip_grad_value_(params, 50)          src/runners/BaseRunner.py:185
 //   Adam(lr, weight_decay=l2).step()      src/runners/BaseRunner.py:100,187  (torch 2.11 optim/adam.py,
 //                                         _multi_tensor_adam, non-capturable branch)
+//   or SGD / Adagrad(lr, weight_decay=l2)  src/runners/BaseRunner.py:83-98 (rule_elem below)
 // which together put a non-zero gradient on EVERY row of both embedding tables each step, so the
-// update is a full streaming sweep (24 B/param: read p,m,v, write p,m,v).  The sparse part of the
+// update is a full streaming sweep (Adam 24 B/param: read p,m,v, write p,m,v; Adagrad 16; GD 8).  The sparse part of the
 // gradient arrives as records (row id + 64 floats) linked per row through head/next; records of one
 // row are summed in ascending record order so the result does not depend on atomics timing.
 #include "common.cuh"
@@ -70,6 +71,62 @@ __device__ __forceinline__ void adam_elem(float& p, float& m, float& v, float g_
     asm("sqrt.approx.f32 %0, %1;" : "=f"(sq) : "f"(v));
     const float denom = fmaf(sq, s.inv_bc2_sqrt, s.eps);
     p = fmaf(s.step_size, __fdividef(m, denom), p);              // param.addcdiv_(exp_avg, denom, value = step_size)
+}
+
+// The optimizer rule (dccf_adam.rule) is a compile-time parameter of the step kernels below.  A rule streams only the
+// state it has: Adam exp_avg (m) and exp_avg_sq (v), Adagrad state_sum (in m), GD none.
+enum : int { RULE_ADAM = 0, RULE_GD = 1, RULE_ADAGRAD = 2 };
+template <int R> constexpr bool rule_has_m = R != RULE_GD;
+template <int R> constexpr bool rule_has_v = R == RULE_ADAM;
+
+// GD and Adagrad need no per-step constant beyond lr (lr_decay = 0): step_size = -lr
+template <int R> __device__ __forceinline__ AdamScalars resolve_rule(const AdamHost& h) {
+    if constexpr (R == RULE_ADAM) {
+        return resolve_adam(h);
+    } else {
+        AdamScalars s = {};
+        s.step_size = (float)(-h.lr);
+        s.eps = h.eps;
+        s.two_l2 = 2.0f * h.l2;
+        s.wd = h.wd;
+        s.clip = h.clip;
+        return s;
+    }
+}
+
+template <int R> __device__ __forceinline__ void rule_elem(float& p, float& m, float& v, float g_sparse, const AdamScalars& s) {
+    if constexpr (R == RULE_ADAM) {
+        adam_elem(p, m, v, g_sparse, s);
+    } else {
+        float g = __fadd_rn(g_sparse, __fmul_rn(s.two_l2, p));   // same preamble as adam_elem
+        if (s.clip > 0.f) g = fminf(fmaxf(g, -s.clip), s.clip);
+        g = fmaf(s.wd, p, g);                                    // weight_decay: g + wd * p
+        if constexpr (R == RULE_GD) {
+            p = fmaf(s.step_size, g, p);                         // SGD: param.add_(g, alpha = -lr)
+        } else {
+            m = fmaf(g, g, m);                                   // Adagrad: state_sum.addcmul_(g, g, value = 1)
+            // std = sqrt(state_sum) + eps ; p += -lr * g / std.  Since state_sum >= g^2, |g| / std <= 1 and the step is
+            // at most lr; MUFU.SQRT and MUFU.RCP (<= 2 ulp each) perturb it by ~4e-7 relative, i.e. by ~4e-7 * lr in p —
+            // far below the 1e-5 parity bound.  state_sum itself is exact IEEE arithmetic.
+            float sq;
+            asm("sqrt.approx.f32 %0, %1;" : "=f"(sq) : "f"(m));
+            p = fmaf(s.step_size, __fdividef(g, __fadd_rn(sq, s.eps)), p);
+        }
+    }
+}
+
+template <int R> __device__ __forceinline__ void rule_elem4(float4& p, float4& m, float4& v, const float4& g,
+                                                            const AdamScalars& s) {
+    rule_elem<R>(p.x, m.x, v.x, g.x, s); rule_elem<R>(p.y, m.y, v.y, g.y, s);
+    rule_elem<R>(p.z, m.z, v.z, g.z, s); rule_elem<R>(p.w, m.w, v.w, g.w, s);
+}
+
+// loads / stores of one state tensor that are compiled away for a rule without it
+template <bool On> __device__ __forceinline__ float4 ld4_if(const float* p) {
+    if constexpr (On) return ld4(p); else return make_float4(0.f, 0.f, 0.f, 0.f);
+}
+template <bool On> __device__ __forceinline__ void st4_if(float* p, const float4& v) {
+    if constexpr (On) st4(p, v);
 }
 
 // Records may arrive in n_seg segments of seg_len records each (one segment per data-parallel rank after the
@@ -365,9 +422,10 @@ __global__ void k_csr_build(const AdamAllArgs a, int phase) {
     }
 }
 
-__global__ void __launch_bounds__(256, 4) k_adam_all(const AdamAllArgs a) {
+template <int R> __device__ __forceinline__ void step_all(const AdamAllArgs& a) {
+    constexpr bool HM = rule_has_m<R>, HV = rule_has_v<R>;
     __shared__ int32_t list_s[16][2][ADAM_LIST_CAP];   // per half-warp: record indices as linked / in ascending order
-    const AdamScalars s = resolve_adam(a.hp);
+    const AdamScalars s = resolve_rule<R>(a.hp);
     const int bid = (int)blockIdx.x;
     for (int i = 0; i < a.n_tables; ++i) {
         const AdamTableArgs& t = a.t[i];
@@ -382,8 +440,8 @@ __global__ void __launch_bounds__(256, 4) k_adam_all(const AdamAllArgs a) {
             const int64_t r0 = 4 * w + half, r1 = r0 + 2;
             const bool v0 = r0 < t.n_rows, v1 = r1 < t.n_rows;
             const size_t o0 = (size_t)(v0 ? r0 : 0) * D + sub * 4, o1 = (size_t)(v1 ? r1 : 0) * D + sub * 4;
-            float4 p0 = ld4(t.table + o0), m0 = ld4(t.m + o0), q0 = ld4(t.v + o0);
-            float4 p1 = ld4(t.table + o1), m1 = ld4(t.m + o1), q1 = ld4(t.v + o1);
+            float4 p0 = ld4(t.table + o0), m0 = ld4_if<HM>(t.m + o0), q0 = ld4_if<HV>(t.v + o0);
+            float4 p1 = ld4(t.table + o1), m1 = ld4_if<HM>(t.m + o1), q1 = ld4_if<HV>(t.v + o1);
             const int32_t h0 = v0 ? t.head[r0] : -1;
             const int32_t h1 = v1 ? t.head[r1] : -1;
             __syncwarp();  // every lane holds its list heads before any lane resets them
@@ -400,14 +458,12 @@ __global__ void __launch_bounds__(256, 4) k_adam_all(const AdamAllArgs a) {
                 if (sub == 0) t.head[r1] = -1;
             }
             if (v0) {
-                adam_elem(p0.x, m0.x, q0.x, g0.x, s); adam_elem(p0.y, m0.y, q0.y, g0.y, s);
-                adam_elem(p0.z, m0.z, q0.z, g0.z, s); adam_elem(p0.w, m0.w, q0.w, g0.w, s);
-                st4(t.table + o0, p0); st4(t.m + o0, m0); st4(t.v + o0, q0);
+                rule_elem4<R>(p0, m0, q0, g0, s);
+                st4(t.table + o0, p0); st4_if<HM>(t.m + o0, m0); st4_if<HV>(t.v + o0, q0);
             }
             if (v1) {
-                adam_elem(p1.x, m1.x, q1.x, g1.x, s); adam_elem(p1.y, m1.y, q1.y, g1.y, s);
-                adam_elem(p1.z, m1.z, q1.z, g1.z, s); adam_elem(p1.w, m1.w, q1.w, g1.w, s);
-                st4(t.table + o1, p1); st4(t.m + o1, m1); st4(t.v + o1, q1);
+                rule_elem4<R>(p1, m1, q1, g1, s);
+                st4(t.table + o1, p1); st4_if<HM>(t.m + o1, m1); st4_if<HV>(t.v + o1, q1);
             }
         }
         return;
@@ -420,13 +476,19 @@ __global__ void __launch_bounds__(256, 4) k_adam_all(const AdamAllArgs a) {
         for (int64_t e = (int64_t)b * blockDim.x + threadIdx.x; e < d.n; e += stride) {
             float g = 0.f;
             for (int32_t k = 0; k < d.n_parts; ++k) g += __ldg(d.g_parts + (size_t)k * d.part_stride + e);
-            float p = d.p[e], m = d.m[e], v = d.v[e];
-            adam_elem(p, m, v, g, s);
-            d.p[e] = p; d.m[e] = m; d.v[e] = v;
+            float p = d.p[e], m = HM ? d.m[e] : 0.f, v = HV ? d.v[e] : 0.f;
+            rule_elem<R>(p, m, v, g, s);
+            d.p[e] = p;
+            if constexpr (HM) d.m[e] = m;
+            if constexpr (HV) d.v[e] = v;
         }
         return;
     }
 }
+
+__global__ void __launch_bounds__(256, 4) k_adam_all(const AdamAllArgs a) { step_all<RULE_ADAM>(a); }
+__global__ void __launch_bounds__(256, 4) k_gd_all(const AdamAllArgs a) { step_all<RULE_GD>(a); }
+__global__ void __launch_bounds__(256, 4) k_adagrad_all(const AdamAllArgs a) { step_all<RULE_ADAGRAD>(a); }
 
 // ---------------------------------------------------------------------------------------------
 // The same step split around the backward pass, so that the HBM-bound sweep of the rows a step does NOT touch
@@ -598,9 +660,17 @@ constexpr int ADAM_SIDE_SMEM = 120 * 1024;     // occupancy limiter of the side-
 __device__ __forceinline__ float4 ldcg4(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ void stcg4(float* p, const float4& v) { __stcg(reinterpret_cast<float4*>(p), v); }
 
-__global__ void __maxnreg__(64) k_adam_untouched(const AdamAllArgs a) {
+template <bool On> __device__ __forceinline__ float4 ldcg4_if(const float* p) {
+    if constexpr (On) return ldcg4(p); else return make_float4(0.f, 0.f, 0.f, 0.f);
+}
+template <bool On> __device__ __forceinline__ void stcg4_if(float* p, const float4& v) {
+    if constexpr (On) stcg4(p, v);
+}
+
+template <int R> __device__ __forceinline__ void step_untouched(const AdamAllArgs& a) {
+    constexpr bool HM = rule_has_m<R>, HV = rule_has_v<R>;
     tl_begin(1);
-    const AdamScalars s = resolve_adam(a.hp);
+    const AdamScalars s = resolve_rule<R>(a.hp);
     const int bid = (int)blockIdx.x;
     for (int i = 0; i < a.n_tables; ++i) {
         const AdamTableArgs& t = a.t[i];
@@ -617,7 +687,9 @@ __global__ void __maxnreg__(64) k_adam_untouched(const AdamAllArgs a) {
         auto request = [&](int64_t r) {
             if (r >= t.n_rows || (sub & 7) != 0) return;              // one lane per 128-byte line
             const size_t o = (size_t)r * D + sub * 4;
-            prefetch_l2(t.table + o); prefetch_l2(t.m + o); prefetch_l2(t.v + o);
+            prefetch_l2(t.table + o);
+            if constexpr (HM) prefetch_l2(t.m + o);
+            if constexpr (HV) prefetch_l2(t.v + o);
         };
         bool v0 = 4 * warp < t.n_rows && row_ok(4 * warp + half), v1 = 4 * warp < t.n_rows && row_ok(4 * warp + half + 2);
         for (int64_t w = warp; 4 * w < t.n_rows; w += n_warps) {
@@ -628,17 +700,16 @@ __global__ void __maxnreg__(64) k_adam_untouched(const AdamAllArgs a) {
             const bool nv0 = row_ok(n0), nv1 = row_ok(n1);
             const size_t o0 = (size_t)(v0 ? r0 : 0) * D + sub * 4, o1 = (size_t)(v1 ? r1 : 0) * D + sub * 4;
             float4 p0, m0, q0, p1, m1, q1;
-            if (v0) { p0 = ldcg4(t.table + o0); m0 = ldcg4(t.m + o0); q0 = ldcg4(t.v + o0); }
-            if (v1) { p1 = ldcg4(t.table + o1); m1 = ldcg4(t.m + o1); q1 = ldcg4(t.v + o1); }
+            if (v0) { p0 = ldcg4(t.table + o0); m0 = ldcg4_if<HM>(t.m + o0); q0 = ldcg4_if<HV>(t.v + o0); }
+            if (v1) { p1 = ldcg4(t.table + o1); m1 = ldcg4_if<HM>(t.m + o1); q1 = ldcg4_if<HV>(t.v + o1); }
+            const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
             if (v0) {
-                adam_elem(p0.x, m0.x, q0.x, 0.f, s); adam_elem(p0.y, m0.y, q0.y, 0.f, s);
-                adam_elem(p0.z, m0.z, q0.z, 0.f, s); adam_elem(p0.w, m0.w, q0.w, 0.f, s);
-                stcg4(t.table + o0, p0); stcg4(t.m + o0, m0); stcg4(t.v + o0, q0);
+                rule_elem4<R>(p0, m0, q0, zero, s);
+                stcg4(t.table + o0, p0); stcg4_if<HM>(t.m + o0, m0); stcg4_if<HV>(t.v + o0, q0);
             }
             if (v1) {
-                adam_elem(p1.x, m1.x, q1.x, 0.f, s); adam_elem(p1.y, m1.y, q1.y, 0.f, s);
-                adam_elem(p1.z, m1.z, q1.z, 0.f, s); adam_elem(p1.w, m1.w, q1.w, 0.f, s);
-                stcg4(t.table + o1, p1); stcg4(t.m + o1, m1); stcg4(t.v + o1, q1);
+                rule_elem4<R>(p1, m1, q1, zero, s);
+                stcg4(t.table + o1, p1); stcg4_if<HM>(t.m + o1, m1); stcg4_if<HV>(t.v + o1, q1);
             }
             v0 = nv0; v1 = nv1;
         }
@@ -647,6 +718,10 @@ __global__ void __maxnreg__(64) k_adam_untouched(const AdamAllArgs a) {
         return;
     }
 }
+
+__global__ void __maxnreg__(64) k_adam_untouched(const AdamAllArgs a) { step_untouched<RULE_ADAM>(a); }
+__global__ void __maxnreg__(64) k_gd_untouched(const AdamAllArgs a) { step_untouched<RULE_GD>(a); }
+__global__ void __maxnreg__(64) k_adagrad_untouched(const AdamAllArgs a) { step_untouched<RULE_ADAGRAD>(a); }
 
 struct WImageArgs {
     float* img;          // operand images of W for the tensor-core forward of the NEXT step (tc_train.cu), or null
@@ -685,7 +760,8 @@ __device__ __forceinline__ void touched_cta_done(const AdamAllArgs& a, const WIm
     }
 }
 
-__global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const WImageArgs wi, const DpSync sync) {
+template <int R> __device__ __forceinline__ void step_touched(const AdamAllArgs& a, const WImageArgs& wi, const DpSync& sync) {
+    constexpr bool HM = rule_has_m<R>, HV = rule_has_v<R>;
     __shared__ int32_t list_s[16][2][ADAM_LIST_CAP];
     tl_begin(5);
     const int bid = (int)blockIdx.x;
@@ -703,7 +779,7 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
         dp_wait_inline(sync, mask);
         if (sync.n_wait > 0 && (mask & 2u)) { tl_begin(12); tl_end(12); }
     }
-    const AdamScalars s = resolve_adam(a.hp);
+    const AdamScalars s = resolve_rule<R>(a.hp);
     for (int i = 0; i < a.n_tables; ++i) {
         const AdamTableArgs& t = a.t[i];
         const int b = bid - t.block_lo;
@@ -731,8 +807,8 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
                 const int32_t offA = t.csr_off[rowA], offB = t.csr_off[rowB];
                 __syncwarp(half_mask);      // every lane of the half-warp has read the heads before lane 0 resets them
                 const size_t oA = (size_t)rowA * D + sub * 4, oB = (size_t)rowB * D + sub * 4;
-                float4 pA = ld4(t.table + oA), mA = ld4(t.m + oA), qA = ld4(t.v + oA);
-                float4 pB = ld4(t.table + oB), mB = ld4(t.m + oB), qB = ld4(t.v + oB);
+                float4 pA = ld4(t.table + oA), mA = ld4_if<HM>(t.m + oA), qA = ld4_if<HV>(t.v + oA);
+                float4 pB = ld4(t.table + oB), mB = ld4_if<HM>(t.m + oB), qB = ld4_if<HV>(t.v + oB);
                 const int32_t fA = __ldcg(t.csr + offA), fB = __ldcg(t.csr + offB);
                 float4 gA, gB;
                 if (nA == 1 && nB == 1) {   // the common case: both single records, both loads in flight
@@ -746,13 +822,11 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
                     t.head[rowA] = -1;
                     if (two) t.head[rowB] = -1;
                 }
-                adam_elem(pA.x, mA.x, qA.x, gA.x, s); adam_elem(pA.y, mA.y, qA.y, gA.y, s);
-                adam_elem(pA.z, mA.z, qA.z, gA.z, s); adam_elem(pA.w, mA.w, qA.w, gA.w, s);
-                st4(t.table + oA, pA); st4(t.m + oA, mA); st4(t.v + oA, qA);
+                rule_elem4<R>(pA, mA, qA, gA, s);
+                st4(t.table + oA, pA); st4_if<HM>(t.m + oA, mA); st4_if<HV>(t.v + oA, qA);
                 if (two) {
-                    adam_elem(pB.x, mB.x, qB.x, gB.x, s); adam_elem(pB.y, mB.y, qB.y, gB.y, s);
-                    adam_elem(pB.z, mB.z, qB.z, gB.z, s); adam_elem(pB.w, mB.w, qB.w, gB.w, s);
-                    st4(t.table + oB, pB); st4(t.m + oB, mB); st4(t.v + oB, qB);
+                    rule_elem4<R>(pB, mB, qB, gB, s);
+                    st4(t.table + oB, pB); st4_if<HM>(t.m + oB, mB); st4_if<HV>(t.v + oB, qB);
                 }
             }
             touched_cta_done(a, wi, sync);
@@ -771,15 +845,14 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
             if (row < 0) continue;          // (uniform over the half-warp: all 16 lanes read the same key and head)
             __syncwarp(half_mask);          // every lane of the half-warp has read the head before lane 0 resets it
             const size_t o = (size_t)row * D + sub * 4;
-            float4 p = ld4(t.table + o), m = ld4(t.m + o), q = ld4(t.v + o);
+            float4 p = ld4(t.table + o), m = ld4_if<HM>(t.m + o), q = ld4_if<HV>(t.v + o);
             if (csr && n_list == 1) first = __ldcg(t.csr + off);
             const float4 g = csr ? gather_row_grad_csr(t, first, off, n_list, sub, half_mask,
                                                        list_s[threadIdx.x >> 4][0], list_s[threadIdx.x >> 4][1])
                                  : gather_row_grad(t, (int32_t)r, sub, half_mask, list_s[threadIdx.x >> 4][0], list_s[threadIdx.x >> 4][1]);
             if (sub == 0) t.head[row] = -1;
-            adam_elem(p.x, m.x, q.x, g.x, s); adam_elem(p.y, m.y, q.y, g.y, s);
-            adam_elem(p.z, m.z, q.z, g.z, s); adam_elem(p.w, m.w, q.w, g.w, s);
-            st4(t.table + o, p); st4(t.m + o, m); st4(t.v + o, q);
+            rule_elem4<R>(p, m, q, g, s);
+            st4(t.table + o, p); st4_if<HM>(t.m + o, m); st4_if<HV>(t.v + o, q);
         }
         touched_cta_done(a, wi, sync);
         return;
@@ -791,7 +864,7 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
         const int64_t stride = (int64_t)d.block_n * blockDim.x;
         const bool image = wi.img != nullptr && wi.tensor == i;
         for (int64_t e = (int64_t)b * blockDim.x + threadIdx.x; e < d.n; e += stride) {
-            float p = d.p[e], m = d.m[e], v = d.v[e];
+            float p = d.p[e], m = HM ? d.m[e] : 0.f, v = HV ? d.v[e] : 0.f;
             // partials added in ascending order, up to sixteen loads in flight at a time (the dW kernel of the reference
             // shape leaves 20: a rolled tail loop waited for the last four one L2 round trip after the other)
             float g = 0.f;
@@ -804,8 +877,10 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
                 for (int q = 0; q < 16; ++q)
                     if (k + q < d.n_parts) g += t16[q];
             }
-            adam_elem(p, m, v, g, s);
-            d.p[e] = p; d.m[e] = m; d.v[e] = v;
+            rule_elem<R>(p, m, v, g, s);
+            d.p[e] = p;
+            if constexpr (HM) d.m[e] = m;
+            if constexpr (HV) d.v[e] = v;
             if (image) {
                 // same layout as k_prep_w_image (tc_train.cu): 32-wide K chunks of [hi 8 KB | lo 8 KB], 8x4 core matrices
                 const int n = (int)(e / wi.K), k = (int)(e - (int64_t)n * wi.K);
@@ -820,6 +895,16 @@ __global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const
         touched_cta_done(a, wi, sync);
         return;
     }
+}
+
+__global__ void __launch_bounds__(256) k_adam_touched(const AdamAllArgs a, const WImageArgs wi, const DpSync sync) {
+    step_touched<RULE_ADAM>(a, wi, sync);
+}
+__global__ void __launch_bounds__(256) k_gd_touched(const AdamAllArgs a, const WImageArgs wi, const DpSync sync) {
+    step_touched<RULE_GD>(a, wi, sync);
+}
+__global__ void __launch_bounds__(256) k_adagrad_touched(const AdamAllArgs a, const WImageArgs wi, const DpSync sync) {
+    step_touched<RULE_ADAGRAD>(a, wi, sync);
 }
 
 __global__ void k_state_advance(int32_t* step_dev, uint64_t* offset_dev, uint64_t inc) {
@@ -904,11 +989,31 @@ static int check_hp(const dccf_adam* hp, AdamHost* out, const char* who) {
     DCCF_CHECK_ARG(hp != nullptr, "%s: null hyper-parameter struct", who);
     DCCF_CHECK_ARG(hp->step_dev != nullptr || hp->step >= 1, "%s: step must be >= 1 (got %d)", who, hp->step);
     DCCF_CHECK_ARG(hp->beta1 >= 0.0 && hp->beta1 < 1.0 && hp->beta2 >= 0.0 && hp->beta2 < 1.0, "%s: betas out of range", who);
+    DCCF_CHECK_ARG(hp->rule == RULE_ADAM || hp->rule == RULE_GD || hp->rule == RULE_ADAGRAD,
+                   "%s: unknown optimizer rule %d (0 Adam, 1 GD, 2 Adagrad)", who, hp->rule);
     out->lr = hp->lr; out->beta1 = hp->beta1; out->beta2 = hp->beta2;
     out->eps = (float)hp->eps; out->l2 = (float)hp->l2; out->wd = (float)hp->weight_decay; out->clip = (float)hp->clip;
     out->step = hp->step; out->step_dev = hp->step_dev;
     return DCCF_OK;
 }
+
+// the per-tensor entry points implement Adam only
+static int check_hp_adam(const dccf_adam* hp, AdamHost* out, const char* who) {
+    int rc = check_hp(hp, out, who);
+    if (rc != DCCF_OK) return rc;
+    DCCF_CHECK_ARG(hp->rule == RULE_ADAM, "%s: Adam only (rule %d); use dccf_adam_step for GD / Adagrad", who, hp->rule);
+    return DCCF_OK;
+}
+
+// kernel of each rule, indexed by dccf_adam.rule
+typedef void (*StepKernel)(AdamAllArgs);
+typedef void (*TouchedKernel)(AdamAllArgs, WImageArgs, DpSync);
+static const StepKernel k_all_of[3] = {k_adam_all, k_gd_all, k_adagrad_all};
+static const StepKernel k_untouched_of[3] = {k_adam_untouched, k_gd_untouched, k_adagrad_untouched};
+static const TouchedKernel k_touched_of[3] = {k_adam_touched, k_gd_touched, k_adagrad_touched};
+static const char* const all_name[3] = {"k_adam_all", "k_gd_all", "k_adagrad_all"};
+static const char* const untouched_name[3] = {"k_adam_untouched", "k_gd_untouched", "k_adagrad_untouched"};
+static const char* const touched_name[3] = {"k_adam_touched", "k_gd_touched", "k_adagrad_touched"};
 
 }  // namespace dccf
 
@@ -920,7 +1025,7 @@ extern "C" int dccf_adam_sweep_seg(float* table, float* m, float* v, int64_t n_t
                                    void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     AdamHost h;
-    int rc = check_hp(hp, &h, "dccf_adam_sweep");
+    int rc = check_hp_adam(hp, &h, "dccf_adam_sweep");
     if (rc != DCCF_OK) return rc;
     DCCF_CHECK_ARG(table && m && v && head, "dccf_adam_sweep: null buffer");
     DCCF_CHECK_ARG(n_seg >= 0 && seg_len >= 0, "dccf_adam_sweep: negative record layout");
@@ -970,7 +1075,7 @@ extern "C" int dccf_adam_dense(float* p, float* m, float* v, int64_t n, const fl
                                int64_t part_stride, const dccf_adam* hp, void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     AdamHost h;
-    int rc = check_hp(hp, &h, "dccf_adam_dense");
+    int rc = check_hp_adam(hp, &h, "dccf_adam_dense");
     if (rc != DCCF_OK) return rc;
     DCCF_CHECK_ARG(p && m && v, "dccf_adam_dense: null buffer");
     DCCF_CHECK_ARG(n_parts == 0 || g_parts, "dccf_adam_dense: null gradient buffer");
@@ -999,6 +1104,8 @@ static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t 
                         int32_t* link_blocks_out) {
     int rc = check_hp(hp, &a.hp, who);
     if (rc != DCCF_OK) return rc;
+    // state tensors the rule reads and writes: Adam m and v, Adagrad m (state_sum), GD none
+    const bool need_m = hp->rule != RULE_GD, need_v = hp->rule == RULE_ADAM;
     DCCF_CHECK_ARG(n_tables >= 0 && n_tables <= ADAM_MAX_T && n_dense >= 0 && n_dense <= ADAM_MAX_T,
                    "%s: at most %d tables and %d dense tensors per call", who, ADAM_MAX_T, ADAM_MAX_T);
     DCCF_CHECK_ARG((n_tables == 0 || tables) && (n_dense == 0 || dense), "%s: null descriptor array", who);
@@ -1010,7 +1117,7 @@ static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t 
     const int64_t budget = (mode == 1) ? 148 : 148 * 8;   // CTAs for the table sweeps, shared in proportion to the row counts (mode 3: the wide untouched-row sweep)
     for (int i = 0; i < n_tables; ++i) {
         const dccf_adam_table& t = tables[i];
-        DCCF_CHECK_ARG(t.table && t.m && t.v && t.head, "%s: table %d has a null buffer", who, i);
+        DCCF_CHECK_ARG(t.table && t.head && (t.m || !need_m) && (t.v || !need_v), "%s: table %d has a null buffer (rule %d)", who, i, hp->rule);
         const int64_t n_rec = (int64_t)t.n_seg * t.seg_len;
         DCCF_CHECK_ARG(t.n_seg >= 0 && t.seg_len >= 0, "%s: table %d has a negative record layout", who, i);
         DCCF_CHECK_ARG(n_rec == 0 || (t.rec_keys && t.rec_grads && t.next), "%s: table %d has records but a null record buffer", who, i);
@@ -1047,7 +1154,7 @@ static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t 
     }
     for (int i = 0; i < n_dense; ++i) {
         const dccf_adam_tensor& d = dense[i];
-        DCCF_CHECK_ARG(d.p && d.m && d.v, "%s: dense tensor %d has a null buffer", who, i);
+        DCCF_CHECK_ARG(d.p && (d.m || !need_m) && (d.v || !need_v), "%s: dense tensor %d has a null buffer (rule %d)", who, i, hp->rule);
         DCCF_CHECK_ARG(d.n_parts == 0 || d.g_parts, "%s: dense tensor %d has a null gradient", who, i);
         AdamDenseArgs& o = a.d[i];
         o.p = d.p; o.m = d.m; o.v = d.v; o.n = d.n > 0 ? d.n : 0; o.g_parts = d.g_parts; o.n_parts = d.n_parts;
@@ -1073,8 +1180,8 @@ extern "C" int dccf_adam_step(const dccf_adam_table* tables, int32_t n_tables, c
         DCCF_CHECK_LAUNCH("k_link_all");
     }
     if (blocks > 0) {
-        k_adam_all<<<(unsigned)blocks, 256, 0, stream>>>(a);
-        DCCF_CHECK_LAUNCH("k_adam_all");
+        k_all_of[hp->rule]<<<(unsigned)blocks, 256, 0, stream>>>(a);
+        DCCF_CHECK_LAUNCH(all_name[hp->rule]);
     }
     return DCCF_OK;
 }
@@ -1174,9 +1281,10 @@ extern "C" int dccf_adam_untouched(const dccf_adam_table* tables, int32_t n_tabl
     const bool wide = threads_per_cta < 0;
     int rc = marshal_adam("dccf_adam_untouched", local, n_tables, nullptr, 0, hp, wide ? 3 : 1, a, &blocks, &link_blocks);
     if (rc != DCCF_OK) return rc;
+    const StepKernel kernel = k_untouched_of[hp->rule];
     if (blocks > 0 && wide) {
-        k_adam_untouched<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(a);
-        DCCF_CHECK_LAUNCH("k_adam_untouched");
+        kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream_>>>(a);
+        DCCF_CHECK_LAUNCH(untouched_name[hp->rule]);
         return DCCF_OK;
     }
     if (blocks > 0) {
@@ -1184,15 +1292,15 @@ extern "C" int dccf_adam_untouched(const dccf_adam_table* tables, int32_t n_tabl
         // memory, ~48 K registers per CTA).  Two sweep CTAs on one SM would leave no room for such a CTA and push it
         // into a second wave, so every sweep CTA reserves (and never touches) 120 KB of dynamic shared memory:
         // at most one per SM, and 120 + 96 KB still fit the 227 KB of an SM.
-        static PerDeviceOnce attr_once;
-        if (attr_once.need()) {
-            cudaError_t e = cudaFuncSetAttribute(k_adam_untouched, cudaFuncAttributeMaxDynamicSharedMemorySize, ADAM_SIDE_SMEM);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(k_adam_untouched, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        static PerDeviceOnce attr_once[3];
+        if (attr_once[hp->rule].need()) {
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ADAM_SIDE_SMEM);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
             if (e != cudaSuccess) {
                 set_error("dccf_adam_untouched: cannot opt in to %d bytes of shared memory: %s", ADAM_SIDE_SMEM, cudaGetErrorString(e));
                 return DCCF_ERR_CUDA;
             }
-            attr_once.mark();
+            attr_once[hp->rule].mark();
         }
         // threads_per_cta (0 = default 224).  The CTA has to stay resident beside the tensor-core kernels AND the middle
         // kernel (768 threads x 64 registers = 3/4 of the register file): 7 warps x 64 registers fit, 8 do not.  Measured (tools/step_timeline.py, electronics shape, L2 flushed): 128 threads swept
@@ -1200,8 +1308,8 @@ extern "C" int dccf_adam_untouched(const dccf_adam_table* tables, int32_t n_tabl
         // that did not fit beside the middle kernel (160 / 192 threads at 70 registers) held that kernel back until the
         // sweep had finished (+15 us).
         const int side_threads = (threads_per_cta >= 32 && threads_per_cta <= 256) ? (threads_per_cta / 32) * 32 : 224;
-        k_adam_untouched<<<(unsigned)blocks, side_threads, ADAM_SIDE_SMEM, (cudaStream_t)stream_>>>(a);
-        DCCF_CHECK_LAUNCH("k_adam_untouched");
+        kernel<<<(unsigned)blocks, side_threads, ADAM_SIDE_SMEM, (cudaStream_t)stream_>>>(a);
+        DCCF_CHECK_LAUNCH(untouched_name[hp->rule]);
     }
     return DCCF_OK;
 }
@@ -1212,6 +1320,7 @@ extern "C" int dccf_adam_csr_build(const dccf_adam_table* tables, int32_t n_tabl
     int32_t blocks = 0, link_blocks = 0;
     dccf_adam hp;
     hp.lr = 0; hp.beta1 = 0.9; hp.beta2 = 0.999; hp.eps = 0; hp.l2 = 0; hp.weight_decay = 0; hp.clip = 0; hp.step = 1; hp.step_dev = nullptr;
+    hp.rule = RULE_GD;      // (this launch reads no optimizer state: validated as the rule without any)
     int rc = marshal_adam("dccf_adam_csr_build", tables, n_tables, nullptr, 0, &hp, 2, a, &blocks, &link_blocks);
     if (rc != DCCF_OK) return rc;
     for (int i = 0; i < n_tables; ++i)
@@ -1253,10 +1362,11 @@ extern "C" int dccf_adam_touched(const dccf_adam_table* tables, int32_t n_tables
         k_link_all<<<(unsigned)link_blocks, 256, 0, stream>>>(a);
         DCCF_CHECK_LAUNCH("k_link_all");
     }
-    static PerDeviceOnce carve_once;
-    if (carve_once.need()) {
-        cudaFuncSetAttribute(k_adam_touched, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        carve_once.mark();
+    const TouchedKernel kernel = k_touched_of[hp->rule];
+    static PerDeviceOnce carve_once[3];
+    if (carve_once[hp->rule].need()) {
+        cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        carve_once[hp->rule].mark();
     }
     if (blocks > 0) {
         cudaLaunchConfig_t cfg = {};
@@ -1266,12 +1376,12 @@ extern "C" int dccf_adam_touched(const dccf_adam_table* tables, int32_t n_tables
         attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = ((ds.flags & DCCF_DP_SYNC_OVERLAP_PUSH) && ds.n_wait >= 2 && already_linked) ? 1 : 0;
-        cudaError_t le = cudaLaunchKernelEx(&cfg, k_adam_touched, a, wi, ds);
+        cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, a, wi, ds);
         if (le != cudaSuccess) {
-            set_error("k_adam_touched: launch failed: %s", cudaGetErrorString(le));
+            set_error("%s: launch failed: %s", touched_name[hp->rule], cudaGetErrorString(le));
             return DCCF_ERR_CUDA;
         }
-        DCCF_CHECK_LAUNCH("k_adam_touched");
+        DCCF_CHECK_LAUNCH(touched_name[hp->rule]);
     }
     return DCCF_OK;
 }

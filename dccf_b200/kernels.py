@@ -54,11 +54,16 @@ def make_rng(noise=None, mask=None, noise_std=0.0, p_drop=0.0, seed=0, offset=0,
     return r
 
 
-def make_adam(lr, l2, weight_decay, step=1, step_dev=None, beta1=0.9, beta2=0.999, eps=1e-8, clip=50.0):
+RULE_ADAM, RULE_GD, RULE_ADAGRAD = 0, 1, 2
+
+
+def make_adam(lr, l2, weight_decay, step=1, step_dev=None, beta1=0.9, beta2=0.999, eps=1e-8, clip=50.0, rule=RULE_ADAM):
+    """dccf_adam: hyper-parameters of the optimizer step; rule 0 Adam, 1 GD, 2 Adagrad (include/dccf_b200.h)."""
     a = Adam()
     a.lr, a.beta1, a.beta2, a.eps = float(lr), float(beta1), float(beta2), float(eps)
     a.l2, a.weight_decay, a.clip = float(l2), float(weight_decay), float(clip)
     a.step = int(step)
+    a.rule = int(rule)
     a.step_dev = ptr(step_dev).value if step_dev is not None else None
     return a
 
@@ -243,12 +248,15 @@ def adam_dense(p, m, v, g_parts, n_parts, part_stride, hp):
 
 
 def adam_table(table, m, v, rec_keys, rec_grads, n_seg, seg_len, key_seg_stride, grad_seg_stride, head, nxt, csr=None):
-    """csr = (rec_row [n_rec], csr_off [n_rows], csr [2 * n_rec], csr_pool [2]) int32 tensors: CSR record lists (counting
-    link + dccf_adam_csr_build) instead of linked lists."""
+    """m / v: the optimizer rule's state (None where the rule has none).  csr = (rec_row [n_rec], csr_off [n_rows],
+    csr [2 * n_rec], csr_pool [2]) int32 tensors: CSR record lists (counting link + dccf_adam_csr_build) instead of
+    linked lists."""
     t = AdamTable()
     if csr is not None:
         t.rec_row, t.csr_off, t.csr, t.csr_pool = (ptr(x).value for x in csr)
-    t.table, t.m, t.v = ptr(table).value, ptr(m).value, ptr(v).value
+    t.table = ptr(table).value
+    t.m = ptr(m).value if m is not None else None
+    t.v = ptr(v).value if v is not None else None
     t.n_rows = table.shape[0]
     t.rec_keys = ptr(rec_keys).value if rec_keys is not None else None
     t.rec_grads = ptr(rec_grads).value if rec_grads is not None else None
@@ -261,7 +269,9 @@ def adam_table(table, m, v, rec_keys, rec_grads, n_seg, seg_len, key_seg_stride,
 
 def adam_tensor(p, m, v, g_parts, n_parts, part_stride):
     t = AdamTensor()
-    t.p, t.m, t.v = ptr(p).value, ptr(m).value, ptr(v).value
+    t.p = ptr(p).value
+    t.m = ptr(m).value if m is not None else None
+    t.v = ptr(v).value if v is not None else None
     t.n = p.numel()
     t.g_parts = ptr(g_parts).value if g_parts is not None else None
     t.n_parts, t.part_stride = int(n_parts), int(part_stride)
@@ -269,7 +279,7 @@ def adam_tensor(p, m, v, g_parts, n_parts, part_stride):
 
 
 def adam_step(tables, dense, hp):
-    """l2 + clip + Adam over every tensor of the model in two launches (dccf_adam_step)."""
+    """l2 + clip + the optimizer rule of `hp` over every tensor of the model in two launches (dccf_adam_step)."""
     lib = _lib.load()
     ta = (AdamTable * max(1, len(tables)))(*tables)
     da = (AdamTensor * max(1, len(dense)))(*dense)
@@ -312,7 +322,7 @@ def make_link_extra(stage=None, prefetch_user=None, prefetch_item=None, prefetch
                     sync=None, counter=None, rec_rows=None, epoch_global=None):
     """Extras of dccf_adam_link_ids.  stage = (epoch_ptrs_dev, cursor_dev, X_out, si_out, counter): the batch is read
     from a device-resident epoch (replaces dccf_stage_batch).  prefetch_user / prefetch_item = up to three [rows, D]
-    tensors each (parameter, exp_avg, exp_avg_sq), prefetch_feat = Feat, prefetch_dense = up to four tensors: what the
+    tensors each (parameter and the optimizer state it has), prefetch_feat = Feat, prefetch_dense = up to four tensors: what the
     step will touch, requested into L2 ahead of its use.  epoch_global = (epoch_ptrs_dev with six slots, cursor_dev): the
     data-parallel link reads every rank's ids of the current batch from an epoch-wide gather (no per-step id exchange)."""
     e = LinkExtra()
@@ -358,7 +368,7 @@ def adam_link_ids(dims, X, sample_item, head_user, next_user, head_item, next_it
 
 
 def adam_untouched(tables, hp, threads=0):
-    """l2 + clip + Adam over the rows no record of this step refers to (head == -1): one launch, <= 148 CTAs of
+    """l2 + clip + the optimizer rule over the rows no record of this step refers to (head == -1): one launch, <= 148 CTAs of
     `threads` threads (0 = the library's default)."""
     lib = _lib.load()
     ta = (AdamTable * max(1, len(tables)))(*tables)
@@ -368,7 +378,7 @@ def adam_untouched(tables, hp, threads=0):
 
 def adam_touched(tables, dense, hp, already_linked=False, w_image=None, w_image_tensor=0, w_image_K=0, cta_counter=None,
                  advance_step_dev=None, advance_offset_dev=None, sync=None, advance_cursor_dev=None):
-    """Adam over the touched rows and the dense tensors (one launch, two when the records still need linking).
+    """The optimizer rule over the touched rows and the dense tensors (one launch, two when the records still need linking).
     sync (make_dp_sync): data-parallel step — wait for the peers' gradient segments in the kernel's prologue, total loss
     and hand-back of the exchange buffers by its last CTA."""
     lib = _lib.load()

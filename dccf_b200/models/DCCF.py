@@ -29,38 +29,66 @@ from .DMF import DMF
 
 
 class FusedAdamState(object):
-    """Optimizer state of the fused path: exp_avg / exp_avg_sq per parameter, step count, and the
-    persistent per-row list heads of the gradient-record scatter.  Stands where the reference keeps a
-    torch.optim.Adam in `model.optimizer` (src/runners/BaseRunner.py:168-169)."""
+    """Optimizer state of the fused path: the rule's state per parameter, step count, and the persistent per-row
+    list heads of the gradient-record scatter.  Stands where the reference keeps its torch optimizer in
+    `model.optimizer` (src/runners/BaseRunner.py:83-107,168-169).  kind: 'adam' (exp_avg / exp_avg_sq), 'gd'
+    (torch.optim.SGD without momentum: no state) or 'adagrad' (state_sum); eps defaults to torch's value per kind."""
 
-    def __init__(self, model, lr, l2, weight_decay, beta1=0.9, beta2=0.999, eps=1e-8, clip=50.0):
+    RULES = {'adam': kernels.RULE_ADAM, 'gd': kernels.RULE_GD, 'adagrad': kernels.RULE_ADAGRAD}
+
+    def __init__(self, model, lr, l2, weight_decay, kind='adam', beta1=0.9, beta2=0.999, eps=None, clip=50.0):
+        if kind not in self.RULES:
+            raise ValueError('unknown fused optimizer %r (adam, gd, adagrad)' % (kind,))
+        self.kind, self.rule = kind, self.RULES[kind]
         self.lr, self.l2, self.weight_decay = lr, l2, weight_decay
-        self.beta1, self.beta2, self.eps, self.clip = beta1, beta2, eps, clip
+        self.beta1, self.beta2, self.clip = beta1, beta2, clip
+        self.eps = eps if eps is not None else (1e-10 if kind == 'adagrad' else 1e-8)
         self.step_count = 0
         self.params = {'E_user': model.uid_embeddings.weight, 'E_item': model.iid_embeddings.weight,
                        'W': model.mlp[0].weight, 'b': model.mlp[0].bias}
-        self.exp_avg = {k: torch.zeros_like(p.data) for k, p in self.params.items()}
-        self.exp_avg_sq = {k: torch.zeros_like(p.data) for k, p in self.params.items()}
+        if kind == 'adam':
+            self.exp_avg = {k: torch.zeros_like(p.data) for k, p in self.params.items()}
+            self.exp_avg_sq = {k: torch.zeros_like(p.data) for k, p in self.params.items()}
+        elif kind == 'adagrad':
+            self.state_sum = {k: torch.zeros_like(p.data) for k, p in self.params.items()}
         dev = model.uid_embeddings.weight.device
         self.head_u = torch.full((model.uid_embeddings.weight.shape[0],), -1, dtype=torch.int32, device=dev)
         self.head_i = torch.full((model.item_num,), -1, dtype=torch.int32, device=dev)
 
-    def hp(self, step=None):
+    def _state_names(self):
+        return {'adam': ('exp_avg', 'exp_avg_sq'), 'gd': (), 'adagrad': ('state_sum',)}[self.kind]
+
+    def state_of(self, k):
+        """(m, v) of parameter k as the kernels take them (dccf_adam_table / _tensor), None where the rule has none."""
+        if self.kind == 'adam':
+            return self.exp_avg[k], self.exp_avg_sq[k]
+        if self.kind == 'adagrad':
+            return self.state_sum[k], None
+        return None, None
+
+    def hp(self, step=None, step_dev=None):
         return kernels.make_adam(self.lr, self.l2, self.weight_decay, step=self.step_count if step is None else step,
-                                 beta1=self.beta1, beta2=self.beta2, eps=self.eps, clip=self.clip)
+                                 step_dev=step_dev, beta1=self.beta1, beta2=self.beta2, eps=self.eps, clip=self.clip,
+                                 rule=self.rule)
 
     def zero_grad(self):
         pass
 
     def state_dict(self):
-        return {'step': self.step_count, 'exp_avg': self.exp_avg, 'exp_avg_sq': self.exp_avg_sq,
-                'lr': self.lr, 'l2': self.l2, 'weight_decay': self.weight_decay}
+        sd = {'step': self.step_count, 'kind': self.kind, 'lr': self.lr, 'l2': self.l2,
+              'weight_decay': self.weight_decay}
+        for n in self._state_names():
+            sd[n] = getattr(self, n)
+        return sd
 
     def load_state_dict(self, sd):
-        """Resume: moments and step count of a saved run (SURVEY.md §8f-4; the reference resumes weights only)."""
-        for k in self.exp_avg:
-            self.exp_avg[k].copy_(sd['exp_avg'][k])
-            self.exp_avg_sq[k].copy_(sd['exp_avg_sq'][k])
+        """Resume: state and step count of a saved run (SURVEY.md §8f-4; the reference resumes weights only)."""
+        kind = sd.get('kind', 'adam')
+        if kind != self.kind:
+            raise ValueError('cannot load the state of a fused %s optimizer into a fused %s optimizer' % (kind, self.kind))
+        for n in self._state_names():
+            for k, t in getattr(self, n).items():
+                t.copy_(sd[n][k])
         self.step_count = int(sd['step'])
         self.lr, self.l2, self.weight_decay = sd['lr'], sd['l2'], sd['weight_decay']
 
@@ -475,7 +503,8 @@ class DCCF(DMF):
         if st['optimizer'] is not None:
             if not isinstance(self.optimizer, FusedAdamState):
                 self.optimizer = self.make_fused_optimizer(lr=st['optimizer']['lr'], l2=st['optimizer']['l2'],
-                                                           weight_decay=st['optimizer']['weight_decay'])
+                                                           weight_decay=st['optimizer']['weight_decay'],
+                                                           kind=st['optimizer'].get('kind', 'adam'))
             self.optimizer.load_state_dict(st['optimizer'])
         self._rng_offset = int(st['rng_offset'])
         self._param_epoch += 1                      # projected tables / operand images of the old weights are stale
@@ -676,9 +705,12 @@ class DCCF(DMF):
         return ex
 
     # ---- fused training step -----------------------------------------------------------------
-    def make_fused_optimizer(self, lr, l2, weight_decay=None, **kw):
+    def make_fused_optimizer(self, lr, l2, weight_decay=None, kind='adam', **kw):
+        """State of the fused step for kind 'adam', 'gd' or 'adagrad' (torch.optim.Adam / SGD / Adagrad with
+        weight_decay, as src/runners/BaseRunner.py:83-107 builds them)."""
         self._check_ready()
-        return FusedAdamState(self, lr=lr, l2=l2, weight_decay=l2 if weight_decay is None else weight_decay, **kw)
+        return FusedAdamState(self, lr=lr, l2=l2, weight_decay=l2 if weight_decay is None else weight_decay, kind=kind,
+                              **kw)
 
     # record lists of the split optimizer step as CSR ranges (counting link + dccf_adam_csr_build off the critical path)
     # instead of linked lists: DCCF_ADAM_CSR=0 restores the lists (A/B; same summation order, same bits)
@@ -699,7 +731,7 @@ class DCCF(DMF):
         Z, D = self.sample_num + 1, self.ui_vector_size
         W, b = self.mlp[0].weight.data, self.mlp[0].bias.data
         eu, ei = self.uid_embeddings.weight.data, self.iid_embeddings.weight.data
-        ea, es = opt.exp_avg, opt.exp_avg_sq
+        su, si, sW, sb = (opt.state_of(k) for k in ('E_user', 'E_item', 'W', 'b'))
         dp = 'exchange' in rec
         world = rec['exchange'].world if dp else 1
         n_u = (world if (dp and rec['exchange'].user_records) else 1) * P
@@ -711,23 +743,23 @@ class DCCF(DMF):
             ex = rec['exchange']
             rseg, dseg = ex.seg_of('gi'), ex.seg_of('gW')
             if ex.user_records:
-                user = kernels.adam_table(eu, ea['E_user'], es['E_user'], ex.recv_part('keys_u'), ex.recv_part('gu'), world, P,
+                user = kernels.adam_table(eu, *su, ex.recv_part('keys_u'), ex.recv_part('gu'), world, P,
                                           rseg, rseg, opt.head_u, next_u, csr=csr_u)
             else:
-                user = kernels.adam_table(eu, ea['E_user'], es['E_user'], rec['keys_u'], rec['gu_rec'], 1, P, P, P * D,
+                user = kernels.adam_table(eu, *su, rec['keys_u'], rec['gu_rec'], 1, P, P, P * D,
                                           opt.head_u, next_u, csr=csr_u)
             tables = [user,
-                      kernels.adam_table(ei, ea['E_item'], es['E_item'], ex.recv_part('keys_i'), ex.recv_part('gi'),
+                      kernels.adam_table(ei, *si, ex.recv_part('keys_i'), ex.recv_part('gi'),
                                          world, P * Z, rseg, rseg, opt.head_i, next_i, csr=csr_i)]
-            dense = [kernels.adam_tensor(W, ea['W'], es['W'], ex.recv_part('gW'), world, dseg),
-                     kernels.adam_tensor(b, ea['b'], es['b'], ex.recv_part('gb'), world, dseg)]
+            dense = [kernels.adam_tensor(W, *sW, ex.recv_part('gW'), world, dseg),
+                     kernels.adam_tensor(b, *sb, ex.recv_part('gb'), world, dseg)]
             return tables, dense
-        tables = [kernels.adam_table(eu, ea['E_user'], es['E_user'], rec['keys_u'], rec['gu_rec'], 1, P, P, P * D,
+        tables = [kernels.adam_table(eu, *su, rec['keys_u'], rec['gu_rec'], 1, P, P, P * D,
                                      opt.head_u, next_u, csr=csr_u),
-                  kernels.adam_table(ei, ea['E_item'], es['E_item'], rec['keys_i'], rec['gi_rec'], 1, P * Z, P * Z,
+                  kernels.adam_table(ei, *si, rec['keys_i'], rec['gi_rec'], 1, P * Z, P * Z,
                                      P * Z * D, opt.head_i, next_i, csr=csr_i)]
-        dense = [kernels.adam_tensor(W, ea['W'], es['W'], rec['gW_part'], rec['n_splits'], W.numel()),
-                 kernels.adam_tensor(b, ea['b'], es['b'], rec['gb_part'], rec['n_splits'], b.numel())]
+        dense = [kernels.adam_tensor(W, *sW, rec['gW_part'], rec['n_splits'], W.numel()),
+                 kernels.adam_tensor(b, *sb, rec['gb_part'], rec['n_splits'], b.numel())]
         return tables, dense
 
     def _exchange_dense(self, rec, push_only=False):
@@ -765,14 +797,16 @@ class DCCF(DMF):
     # fused step with the optimizer split around the backward: the Adam sweep of the rows the (global) batch does not
     # touch runs on a second stream while the forward and backward run (dccf_adam_link_ids / _untouched / _touched)
 
-    def _sweep_threads(self, dp):
-        """Launch shape of the untouched-row Adam sweep: one small CTA per SM hidden beside the tensor-core kernels and
+    def _sweep_threads(self, dp, opt):
+        """Launch shape of the untouched-row sweep: one small CTA per SM hidden beside the tensor-core kernels and
         the middle kernel (0 = the library's default, 224 threads: the widest CTA whose registers fit beside the middle
         kernel's) while the tables are small enough for that to finish in time; -1 = the wide, full-occupancy sweep once
-        the sweep itself bounds the step (scaled configuration: 24 B x 64 x 10^6..10^7 rows per step — at the ~3 TB/s
-        of the narrow launch that is milliseconds)."""
+        the sweep itself bounds the step (scaled configuration with Adam: 24 B x 64 x 10^6..10^7 rows per step — at the
+        ~3 TB/s of the narrow launch that is milliseconds).  Bytes per parameter: the parameter and each state tensor
+        of the rule, read and written (Adam 24, Adagrad 16, GD 8)."""
         rows = self.uid_embeddings.weight.shape[0] + self.item_num
-        if rows * self.ui_vector_size * 24 > 400e6:
+        bytes_per_param = 8 * (1 + sum(t is not None for t in opt.state_of('E_item')))
+        if rows * self.ui_vector_size * bytes_per_param > 400e6:
             return -1
         return 0
 
@@ -827,17 +861,19 @@ class DCCF(DMF):
         # The exposure softmax of the local pairs (read by the middle kernel) and, on one GPU, the record lists: first,
         # on the main stream.  (On the side stream this kernel would run beside the first CTAs of the partial-product
         # kernel — measured: that kernel then takes 22 us instead of 13.)  k_link_ids also requests what the step will
-        # touch into L2: rows of the tables and their Adam moments, the true items' feature rows, W with its moments and
+        # touch into L2: rows of the tables and their optimizer state, the true items' feature rows, W with its state and
         # operand images.
         eu, ei = self.uid_embeddings.weight.data, self.iid_embeddings.weight.data
         W = self.mlp[0].weight.data
-        pf_user = (eu, opt.exp_avg['E_user'], opt.exp_avg_sq['E_user'])
-        pf_item = (ei, opt.exp_avg['E_item'], opt.exp_avg_sq['E_item'])
+        # (only the tensors the optimizer rule has)
+        pf_user = tuple(t for t in (eu,) + opt.state_of('E_user') if t is not None)
+        pf_item = tuple(t for t in (ei,) + opt.state_of('E_item') if t is not None)
+        pf_W = tuple(t for t in (W,) + opt.state_of('W') if t is not None)
         rec_rows = (self._ws['rec_row_u'], self._ws['rec_row_i']) if csr else None      # (allocated by _step_tables)
         if not dp:
             extra = kernels.make_link_extra(
                 stage=stage, prefetch_user=pf_user, prefetch_item=pf_item, rec_rows=rec_rows,
-                prefetch_feat=self.feature_embedding, prefetch_dense=(wimg, W, opt.exp_avg['W'], opt.exp_avg_sq['W']))
+                prefetch_feat=self.feature_embedding, prefetch_dense=(wimg,) + pf_W)
         else:
             # data parallel: the local launch stages the batch (device-resident epoch) and evaluates the exposure softmax;
             # the record lists of the GLOBAL step are linked on the side stream
@@ -859,7 +895,7 @@ class DCCF(DMF):
             # into the consumers: they wait for the peers' segments in their own prologue and their last CTA hands the
             # buffers back.
             pf = dict(prefetch_user=pf_user, prefetch_item=pf_item,
-                      prefetch_dense=(W, opt.exp_avg['W'], opt.exp_avg_sq['W']))
+                      prefetch_dense=pf_W)
             if epoch_ids is not None:
                 # every rank's ids of the whole epoch were gathered once (begin_resident_epoch): no id exchange in the step
                 kernels.adam_link_ids(self._dims(), None, None, opt.head_u, next_u, opt.head_i, next_i, n_pairs=P,
@@ -892,7 +928,7 @@ class DCCF(DMF):
                 if csr:
                     linked = torch.cuda.Event()
                     linked.record(side)
-                kernels.adam_untouched(tables, hp, self._sweep_threads(dp and epoch_ids is None))
+                kernels.adam_untouched(tables, hp, self._sweep_threads(dp and epoch_ids is None, opt))
                 done.record(side)
             # The CSR ranges of the step's record lists (two small launches; the touched-row sweep that needs them runs
             # after the backward): on a third stream as soon as the lists are linked, beside the sweep and the forward —
@@ -919,7 +955,7 @@ class DCCF(DMF):
         else:
             if dp:
                 link_global()
-            kernels.adam_untouched(tables, hp, self._sweep_threads(dp and epoch_ids is None))
+            kernels.adam_untouched(tables, hp, self._sweep_threads(dp and epoch_ids is None, opt))
             if csr:
                 kernels.adam_csr_build(tables)
         pred, rec = self._launch_fwd_bwd(call, loss_mode, Y, rec=rec, w_image_valid=w_image_valid, expo_e=expo_e,
@@ -1030,8 +1066,7 @@ class DCCF(DMF):
                                generate_noise=self.std > 0, generate_mask=p_drop > 0)
         call = {'X': g['X'], 'sample_item': g['si'], 'rng': rng, 'noise': None, 'mask': None, 'P': P,
                 'N': P * (S + 1) * self.attribute_num}
-        hp = kernels.make_adam(opt.lr, opt.l2, opt.weight_decay, step=1, step_dev=g['step_dev'], beta1=opt.beta1,
-                               beta2=opt.beta2, eps=opt.eps, clip=opt.clip)
+        hp = opt.hp(step=1, step_dev=g['step_dev'])
         torch.cuda.synchronize()
         graph = torch.cuda.CUDAGraph()
         launches_before = kernels.LAUNCHES[0]

@@ -3,10 +3,10 @@
 Same flags, constructor, `train / fit / predict / evaluate / check / eva_termination`, same log lines and
 model-selection rules.  Differences are confined to where the time goes:
 
-  * `fit` — when the optimizer is Adam and the model offers `train_step` (dccf_b200's DCCF), each batch
-    is ONE fused step (forward, loss, l2 term, backward, clip(+-50), Adam; BaseRunner.py:175-188) with no
-    autograd and no host synchronisation; the loss of the last batch is read back once per epoch.
-    Any other optimizer/model goes through the reference's autograd sequence unchanged.
+  * `fit` — when the model offers `train_step` (dccf_b200's DCCF), each batch is ONE fused step (forward, loss,
+    l2 term, backward, clip(+-50), GD / Adagrad / Adam step; BaseRunner.py:175-188) with no autograd and no host
+    synchronisation; the loss of the last batch is read back once per epoch.  Any other model goes through the
+    reference's autograd sequence and torch optimizer unchanged.
   * `predict` — predictions stay on the device across batches and are re-ordered to data order with one
     vectorised scatter instead of a Python dict with one entry per row (BaseRunner.py:148-156).
   * `evaluate` — ranking metrics come from the dccf_rank_eval kernel on the device-resident predictions.
@@ -62,8 +62,8 @@ class BaseRunner(object):
 
     # ---- optimizer ---------------------------------------------------------------------------
     def _build_optimizer(self, model):
-        """SGD / Adagrad / Adam, all with weight_decay = l2 (BaseRunner.py:83-107).  Adam on a model that has
-        the fused step keeps its state in a FusedAdamState instead of torch.optim.Adam."""
+        """SGD / Adagrad / Adam, all with weight_decay = l2 (BaseRunner.py:83-107).  On a model that has the fused
+        step, the state of each lives in the fused optimizer state (make_fused_optimizer) instead of a torch optimizer."""
         name = self.optimizer_name.lower()
         if name == 'adam':
             logging.info('Optimizer: Adam')
@@ -72,9 +72,15 @@ class BaseRunner(object):
             return torch.optim.Adam(model.parameters(), lr=self.learning_rate, weight_decay=self.l2_weight)
         if name == 'adagrad':
             logging.info('Optimizer: Adagrad')
+            if hasattr(model, 'make_fused_optimizer'):
+                return model.make_fused_optimizer(lr=self.learning_rate, l2=self.l2_weight, weight_decay=self.l2_weight,
+                                                  kind='adagrad')
             return torch.optim.Adagrad(model.parameters(), lr=self.learning_rate, weight_decay=self.l2_weight)
         if name == 'gd':
             logging.info('Optimizer: GD')
+            if hasattr(model, 'make_fused_optimizer'):
+                return model.make_fused_optimizer(lr=self.learning_rate, l2=self.l2_weight, weight_decay=self.l2_weight,
+                                                  kind='gd')
             return torch.optim.SGD(model.parameters(), lr=self.learning_rate, weight_decay=self.l2_weight)
         logging.error('Unknown Optimizer: ' + self.optimizer_name)
         assert self.optimizer_name in ['GD', 'Adagrad', 'Adam']
@@ -204,7 +210,8 @@ class BaseRunner(object):
         suspended = None
         if world > 1:
             if not (fused and hasattr(model, 'begin_resident_epoch') and data_processor.rank == 1):
-                raise RuntimeError('data-parallel training (torchrun) needs the fused Adam step of DCCF with --rank 1')
+                raise RuntimeError('data-parallel training (torchrun) supports only the fused step of DCCF (GD, '
+                                   'Adagrad or Adam) with --rank 1: not other models, torch optimizers or --rank 0')
             from ..dist import sync_host_rng
             sync_host_rng(model)            # sharded evaluation left the ranks' generators at different positions
         if fused and hasattr(model, 'begin_resident_epoch') and (len(batches) > 2 or world > 1) \

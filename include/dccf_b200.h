@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 34
+#define DCCF_ABI_VERSION 35
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -222,11 +222,19 @@ int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user, const floa
                           const float* expo_den, const dccf_batch_ref* batch, int32_t phases, int32_t* err_flag,
                           void* stream);
 
-/* ---- (c) part 2: l2 + clip + Adam, dense over every row --------------------------------- */
+/* ---- (c) part 2: l2 + clip + optimizer (Adam, GD, Adagrad), dense over every row ---------- */
 /* Replaces model.l2()*l2 (BaseRunner.py:181, BaseModel.py:179-187), clip_grad_value_
- * (BaseRunner.py:185) and torch.optim.Adam(weight_decay=l2).step (BaseRunner.py:100,187):
- *   g = clamp(g_sparse + 2*l2*p, -clip, clip) + wd*p ; m,v,p updated as torch 2.11
- *   optim/adam.py (_multi_tensor_adam, non-capturable branch).
+ * (BaseRunner.py:185) and the optimizer step (BaseRunner.py:83-107,187), every optimizer with
+ * weight_decay = l2:
+ *   g = clamp(g_sparse + 2*l2*p, -clip, clip) + wd*p
+ * then, by dccf_adam.rule:
+ *   0 Adam     m,v,p updated as torch 2.11 optim/adam.py (_multi_tensor_adam, non-capturable branch)
+ *   1 GD       torch.optim.SGD, momentum 0:   p = p - lr*g                        (no state)
+ *   2 Adagrad  torch.optim.Adagrad, lr_decay 0, initial_accumulator_value 0:
+ *              s = s + g*g ; p = p - lr*g / (sqrt(s) + eps)                       (state_sum s in `m`)
+ * The update is dense: rows without gradient records step with g_sparse = 0.  A rule reads and
+ * writes only its own state; the state pointers it does not have may be NULL.  Only
+ * dccf_adam_step, dccf_adam_untouched and dccf_adam_touched take rule != 0.
  * Embedding-table variant: the gradient arrives as n_rec records (row id + D floats); records
  * with equal ids are summed in ascending record order (deterministic).
  *   head  int32[n_table_rows], persistent, must be -1 everywhere on entry; is -1 again on exit
@@ -238,7 +246,7 @@ typedef struct dccf_adam {
     double weight_decay;/* Adam weight_decay               (--l2) */
     double clip;        /* clip_grad_value_ bound, 50; <= 0 disables */
     int32_t step;       /* t = 1,2,... */
-    int32_t _pad;
+    int32_t rule;       /* 0 Adam (a zero-initialised struct), 1 GD, 2 Adagrad */
     const int32_t* step_dev; /* optional DEVICE pointer overriding `step` (graph replay) */
 } dccf_adam;
 
@@ -263,7 +271,7 @@ int dccf_adam_dense(float* p, float* m, float* v, int64_t n, const float* g_part
  * embedding tables with segmented records and up to 4 dense tensors with partial-sum gradients.  Same
  * arithmetic and summation order as the per-tensor entry points above. */
 typedef struct dccf_adam_table {
-    float* table; float* m; float* v;
+    float* table; float* m; float* v;  /* m / v: the rule's state (see dccf_adam.rule) */
     int64_t n_rows;
     const int32_t* rec_keys; const float* rec_grads;
     int32_t n_seg; int32_t _pad;

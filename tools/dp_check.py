@@ -1,6 +1,12 @@
 """Multi-GPU check, run under torchrun (world >= 2): a data-parallel fused step over W ranks equals the
 single-GPU step on the concatenated batch, replicas stay bit-identical, user-sharded evaluation equals the
-single-GPU evaluation.  Prints 'DP CHECK OK' on rank 0."""
+single-GPU evaluation.  Prints 'DP CHECK OK' on rank 0.
+
+    torchrun --nproc-per-node 2 tools/dp_check.py [--optimizer adam|gd|adagrad]
+
+--optimizer: the fused optimizer of both runs (default adam); its state (exp_avg for Adam, state_sum for Adagrad) is
+compared as well."""
+import argparse
 import os
 import sys
 
@@ -35,6 +41,9 @@ def close(a, b, tol, what):
 
 
 def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--optimizer', choices=('adam', 'gd', 'adagrad'), default='adam')
+    kind = ap.parse_args().optimizer
     rank, world, local = int(os.environ['RANK']), int(os.environ['WORLD_SIZE']), int(os.environ['LOCAL_RANK'])
     torch.cuda.set_device(local)
     dist.init_process_group('nccl', device_id=torch.device('cuda', local))
@@ -50,7 +59,7 @@ def main():
     rows = (pairs[:, None] * R + np.arange(R)[None, :]).reshape(-1)
     model = make_model(params, S, A, std)
     model.enable_data_parallel(p2p=os.environ.get('DCCF_DP_P2P', '1') == '1')
-    model.optimizer = model.make_fused_optimizer(lr=1e-3, l2=1e-4)
+    model.optimizer = model.make_fused_optimizer(lr=1e-3, l2=1e-4, kind=kind)
     steps = 2
     for t in range(steps):
         fd = {'X': torch.from_numpy(X[pairs]).cuda(), 'rank': 1, 'train': True, 'dropout': drop,
@@ -67,7 +76,7 @@ def main():
         assert torch.equal(t, ref), 'rank %d diverged from rank 0 on %s' % (rank, k)
     # equals the single-GPU step on the whole batch
     single = make_model(params, S, A, std)
-    single.optimizer = single.make_fused_optimizer(lr=1e-3, l2=1e-4)
+    single.optimizer = single.make_fused_optimizer(lr=1e-3, l2=1e-4, kind=kind)
     for t in range(steps):
         fd = {'X': torch.from_numpy(X).cuda(), 'rank': 1, 'train': True, 'dropout': drop, 'Y': torch.zeros(P).cuda(),
               'sample_item': torch.from_numpy(si), 'noise': torch.from_numpy(noise),
@@ -79,8 +88,10 @@ def main():
     for k in ('E_user', 'E_item', 'b'):
         close(got[k], want[k], 1e-5, k)
     close(got['W'], want['W'], 5e-4, 'W')
-    for k in ('E_user', 'E_item', 'W', 'b'):
-        close(model.optimizer.exp_avg[k].cpu().numpy(), single.optimizer.exp_avg[k].cpu().numpy(), 1e-5, 'exp_avg ' + k)
+    state = {'adam': 'exp_avg', 'adagrad': 'state_sum', 'gd': None}[kind]
+    for k in (('E_user', 'E_item', 'W', 'b') if state else ()):
+        close(getattr(model.optimizer, state)[k].cpu().numpy(), getattr(single.optimizer, state)[k].cpu().numpy(), 1e-5,
+              state + ' ' + k)
 
     say(rank, 'equality with the single-GPU step ok')
     # DP steps on the library's own rng streams keep the replicas identical too
@@ -115,7 +126,7 @@ def main():
     assert np.abs(np.array(got_m) - np.array(want_m)).max() < 1e-9, (got_m, want_m)
     dist.barrier()
     if rank == 0:
-        print('DP CHECK OK world=%d' % world)
+        print('DP CHECK OK world=%d optimizer=%s' % (world, kind))
     dist.destroy_process_group()
 
 
