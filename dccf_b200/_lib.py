@@ -11,7 +11,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
-ABI_VERSION = 35
+ABI_VERSION = 36
 DIM = 64
 
 

@@ -164,6 +164,10 @@ __global__ void __launch_bounds__(TC_NT, 2) k_train_fwd_tc(const TrainFwdParams 
     __syncthreads();
     tc::tc_fence_after_sync();
     const uint32_t tmem_base = *tmem_slot;
+    // The middle kernel may be launched as a programmatic dependent of this one (phases bit 16): its CTAs may be placed
+    // from here on.  They read this grid's outputs only after their griddepcontrol.wait, which returns when this grid has
+    // COMPLETED — and this grid does not complete before the kernel before it has (the wait at the end).
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
     if (warp < TC_PRODUCERS / 32) {
         // ===== producers =====
@@ -366,6 +370,8 @@ struct TrainMidParams {
     const float* pre_part;
     const float* expo_e;         // optional [P, Z] + expo_den [P]: the exposure softmax of every pair, precomputed from
     const float* expo_den;       // the ids on another stream (dccf_adam_link_ids); null: evaluated here
+    const uint64_t* batch_ptrs;  // optional (with batch_cursor): the user ids read before griddepcontrol.wait come from
+    const int64_t* batch_cursor; //   batch *batch_cursor of the device-resident epoch, as in k_train_fwd_tc
     float* out_pred;
     float* loss_terms;
     float* dpre_rows;
@@ -412,6 +418,14 @@ __global__ void __maxnreg__(64) k_train_mid(const TrainMidParams prm) {
     auto pair_of = [&](int q) { return q == 0 ? jt : p_second; };
     const uint32_t half_mask = (lane & 16) ? 0xffff0000u : 0x0000ffffu;
 
+    // Launched as a programmatic dependent of the partial-product kernel (phases bit 16), this CTA may start while that
+    // kernel runs (only on an SM without one of its CTAs: 768 x 64 registers do not fit beside its 576 x 56).  Until
+    // griddepcontrol.wait it reads only state that existed before the step: W, b, E_user (the user rows are touched
+    // rows, which only k_adam_touched writes, after the step's dW kernel), the RNG key and, through the batch cursor,
+    // the ids of a device-resident epoch.  The staged X, expo_e / expo_den and pre_part are read after the wait, which
+    // returns when the partial-product kernel has completed — and that kernel does not complete before k_adam_link_ids,
+    // which writes them, has (its own wait).  Both instructions are no-ops in a plain launch.
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     // W_i: loaded now, parked in registers, stored to shared memory after the first phase (only the last one reads it)
     float4 wreg[2];
 #pragma unroll
@@ -420,14 +434,18 @@ __global__ void __maxnreg__(64) k_train_mid(const TrainMidParams prm) {
         if (i < D * D / 4) wreg[t] = ldg4(prm.W + (size_t)(i / (D / 4)) * prm.K + (i % (D / 4)) * 4);
     }
     const float4 bia = ldg4(prm.bias + sub * 4);
-    // the user rows of the CTA's (at most two) pairs, columns 4*sub .. 4*sub+3
-    const int32_t u0 = checked_id(prm.X[2 * jt] - prm.user_base, prm.n_users, prm.err_flag);
-    const int32_t u1 = checked_id(prm.X[2 * p_second] - prm.user_base, prm.n_users, prm.err_flag);
-    const float4 eu0 = ldg4(prm.E_user + (size_t)u0 * D + sub * 4);
-    const float4 eu1 = ldg4(prm.E_user + (size_t)u1 * D + sub * 4);
     RngKey key_drop = make_rng_key(0, 0, DOMAIN_DROPOUT);
     if (prm.mask_mode == 2) key_drop = resolve_rng_key(prm.rng, DOMAIN_DROPOUT);
     const size_t part_stride = (size_t)prm.n_rows * D;
+    // the user rows of the CTA's (at most two) pairs, columns 4*sub .. 4*sub+3
+    const int64_t* Xu = prm.X;
+    if (prm.batch_cursor != nullptr) Xu = reinterpret_cast<const int64_t*>(prm.batch_ptrs[0]) + *prm.batch_cursor * prm.n_pairs * 2;
+    else asm volatile("griddepcontrol.wait;" ::: "memory");
+    const int32_t u0 = checked_id(Xu[2 * jt] - prm.user_base, prm.n_users, prm.err_flag);
+    const int32_t u1 = checked_id(Xu[2 * p_second] - prm.user_base, prm.n_users, prm.err_flag);
+    const float4 eu0 = ldg4(prm.E_user + (size_t)u0 * D + sub * 4);
+    const float4 eu1 = ldg4(prm.E_user + (size_t)u1 * D + sub * 4);
+    asm volatile("griddepcontrol.wait;" ::: "memory");
 
     // ---- A: rows of the CTA's pairs: partial sums + bias, ReLU, dropout, dot with the user row -------------
     for (int rr = hw; rr < npc * R; rr += TM_NT / 16) {
@@ -592,13 +610,21 @@ __global__ void __maxnreg__(64) k_train_mid(const TrainMidParams prm) {
 // =============================================================================================
 // backward: gW / gb partial tiles
 // =============================================================================================
-constexpr int TB_NT = TC_PRODUCERS + 32;   // 16 producer warps + the MMA warp
+// 16 producer warps + the MMA warp + 2 idle warps that only take part in the CTA-wide barriers.  They fix the kernel's
+// occupancy at ONE CTA per SM: at 56 registers (the __maxnreg__ below) a CTA takes 608 x 56 = 34 048 registers, more than
+// half of the SM's 65 536, so two do not fit — as a programmatic dependent of the middle kernel (phases bit 32) the CTAs
+// placed early would otherwise double up on the few free SMs and unbalance the grid.  One CTA still fits beside a CTA of
+// the side-stream sweep (224 x 64 = 14 336 registers, 120 KB of shared memory + this kernel's 96 KB), and none beside a
+// middle-kernel CTA (768 x 64 = 49 152 registers).  tests/test_occupancy.py checks these facts on the built library.
+constexpr int TB_NT = TC_PRODUCERS + 32 + 64;
 
 struct TrainBwdParams {
     const float* E_item;
     const float* Feat;
     const int64_t* X;
     const int64_t* sample_item;
+    const uint64_t* batch_ptrs;  // optional (with batch_cursor): the ids come from batch *batch_cursor of the
+    const int64_t* batch_cursor; //   device-resident epoch, as in k_train_fwd_tc (so they can be read before the wait)
     const float* noise;          // mode 1
     const float* dpre_rows;      // [N, D]
     float* gW_part;              // [n_splits][D][K]
@@ -628,7 +654,7 @@ __device__ __forceinline__ void quad_transpose(float4& a, int j) {
 }
 
 template <int NOISE_MODE>
-__global__ void __launch_bounds__(TB_NT, 2) k_train_bwd_tc(const TrainBwdParams prm) {
+__global__ void __maxnreg__(56) k_train_bwd_tc(const TrainBwdParams prm) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + TT_STAGES * TC_STAGE_BYTES);
     uint64_t* empty_bar = full_bar + TT_STAGES;
@@ -666,27 +692,33 @@ __global__ void __launch_bounds__(TB_NT, 2) k_train_bwd_tc(const TrainBwdParams 
         const int bc = tid & 63, brq = tid >> 6;
         RngKey key_noise = make_rng_key(0, 0, DOMAIN_NOISE);
         if (NOISE_MODE == 2) key_noise = resolve_rng_key(prm.rng, DOMAIN_NOISE);
+        const int64_t *X = prm.X, *si = prm.sample_item;
+        if (prm.batch_cursor != nullptr) {
+            const int64_t b = *prm.batch_cursor, n_pairs = (int64_t)((uint32_t)prm.n_rows / (uint32_t)prm.R);
+            X = reinterpret_cast<const int64_t*>(prm.batch_ptrs[0]) + b * n_pairs * 2;
+            si = reinterpret_cast<const int64_t*>(prm.batch_ptrs[1]) + b * n_pairs * prm.S;
+        }
 
-        // operands of stage st: dpre values (B) and this lane's 4 columns of x for its row (A, before the transpose)
-        auto fetch = [&](int st, float4 (&v)[2], float4& dv) {
-            const int64_t rb = row_lo + (int64_t)st * TC_KC;
-            {
-                const int64_t r0 = rb + brq * 4;
-                const float* src = prm.dpre_rows + (size_t)r0 * D + bc;
-                dv.x = (r0 + 0 < row_hi) ? __ldg(src) : 0.f;
-                dv.y = (r0 + 1 < row_hi) ? __ldg(src + D) : 0.f;
-                dv.z = (r0 + 2 < row_hi) ? __ldg(src + 2 * D) : 0.f;
-                dv.w = (r0 + 3 < row_hi) ? __ldg(src + 3 * D) : 0.f;
-            }
-            const int64_t r = rb + rq * 4 + j;
+        // the B operand of stage st: dpre values, thread = channel bc, rows 4*brq .. 4*brq+3
+        auto fetch_dpre = [&](int st, float4& dv) {
+            const int64_t r0 = row_lo + (int64_t)st * TC_KC + brq * 4;
+            const float* src = prm.dpre_rows + (size_t)r0 * D + bc;
+            dv.x = (r0 + 0 < row_hi) ? __ldg(src) : 0.f;
+            dv.y = (r0 + 1 < row_hi) ? __ldg(src + D) : 0.f;
+            dv.z = (r0 + 2 < row_hi) ? __ldg(src + 2 * D) : 0.f;
+            dv.w = (r0 + 3 < row_hi) ? __ldg(src + 3 * D) : 0.f;
+        };
+        // the A operand of stage st: this lane's 4 columns of x for its row (before the transpose)
+        auto fetch_x = [&](int st, float4 (&v)[2]) {
+            const int64_t r = row_lo + (int64_t)st * TC_KC + rq * 4 + j;
             const bool live = r < row_hi;
             int32_t fi = 0, it = 0;
             if (live) {
                 const uint32_t p = (uint32_t)r / (uint32_t)prm.R;
-                fi = checked_id(prm.X[2 * (int64_t)p + 1], prm.n_items, nullptr);
+                fi = checked_id(X[2 * (int64_t)p + 1], prm.n_items, nullptr);
                 if (mt == 0) {
                     const int z = (int)((uint32_t)r - p * (uint32_t)prm.R) / prm.A;
-                    it = (z == 0) ? fi : checked_id(prm.sample_item[(int64_t)p * prm.S + (z - 1)], prm.n_items, nullptr);
+                    it = (z == 0) ? fi : checked_id(si[(int64_t)p * prm.S + (z - 1)], prm.n_items, nullptr);
                 }
             }
 #pragma unroll
@@ -713,8 +745,8 @@ __global__ void __launch_bounds__(TB_NT, 2) k_train_bwd_tc(const TrainBwdParams 
             }
         };
 
-        // stage st of this CTA: transpose, wait until the MMAs that read its slot have completed, store, publish
-        auto commit = [&](int st, float4 (&v)[2], const float4& dv) {
+        // stage st of this CTA, A operand: transpose, wait until the MMAs that read its slot have completed, store
+        auto store_x = [&](int st, float4 (&v)[2]) {
             const int s = st % TT_STAGES;
             const uint32_t ph = (uint32_t)(st / TT_STAGES) & 1u;
             quad_transpose(v[0], j);
@@ -722,25 +754,55 @@ __global__ void __launch_bounds__(TB_NT, 2) k_train_bwd_tc(const TrainBwdParams 
             tc::mbar_wait(&empty_bar[s], ph ^ 1u);
             uint8_t* a_hi = smem + s * TC_STAGE_BYTES;
             uint8_t* a_lo = a_hi + TC_A_BYTES;
-            uint8_t* b_hi = a_hi + 2 * TC_A_BYTES;
-            uint8_t* b_lo = b_hi + TC_B_BYTES;
 #pragma unroll
             for (int t = 0; t < 2; ++t) {
                 const int m = (cb0 + 2 * t) * 32 + g * 4 + j;      // after the transpose this lane holds column m,
                 store_hi_lo(a_hi, a_lo, core_offset(m, rq * 4), v[t]);   // rows 4*rq .. 4*rq+3 of the stage
             }
+        };
+        // ... B operand (after its A operand): store, publish the stage
+        auto store_dpre = [&](int st, const float4& dv) {
+            const int s = st % TT_STAGES;
+            uint8_t* b_hi = smem + s * TC_STAGE_BYTES + 2 * TC_A_BYTES;
+            uint8_t* b_lo = b_hi + TC_B_BYTES;
             store_hi_lo(b_hi, b_lo, core_offset(bc, brq * 4), dv);
             tc::fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) tc::mbar_arrive(&full_bar[s]);
         };
+        // Launched as a programmatic dependent of the middle kernel (phases bit 32), this CTA may start while that kernel
+        // runs.  Only dpre and the loss terms come from it: with the ids of a device-resident epoch (batch cursor) the A
+        // operands of the first TT_STAGES stages (free ring slots) are built before griddepcontrol.wait, from tables the
+        // step has not written yet.  The wait returns when the middle kernel has completed, which it does only after the
+        // partial-product kernel has (its own wait).  A no-op in a plain launch.
+        const int n_pre = (prm.batch_cursor != nullptr) ? min(n_st, TT_STAGES) : 0;
+        {
+            float4 xp[TT_STAGES][2];
+#pragma unroll
+            for (int st = 0; st < TT_STAGES; ++st)
+                if (st < n_pre) fetch_x(st, xp[st]);
+#pragma unroll
+            for (int st = 0; st < TT_STAGES; ++st)
+                if (st < n_pre) store_x(st, xp[st]);
+        }
+        asm volatile("griddepcontrol.wait;" ::: "memory");
         float4 v[2], dv;
-        if (n_st > 0) fetch(0, v, dv);
-        for (int st = 0; st < n_st; ++st) {
+        {
+            float4 dp[TT_STAGES];
+#pragma unroll
+            for (int st = 0; st < TT_STAGES; ++st)
+                if (st < n_pre) fetch_dpre(st, dp[st]);
+            if (n_pre < n_st) { fetch_x(n_pre, v); fetch_dpre(n_pre, dv); }
+#pragma unroll
+            for (int st = 0; st < TT_STAGES; ++st)
+                if (st < n_pre) store_dpre(st, dp[st]);
+        }
+        for (int st = n_pre; st < n_st; ++st) {
             // the next stage's operands are in flight while this one is transposed, stored and multiplied
             float4 vn[2], dvn;
-            if (st + 1 < n_st) fetch(st + 1, vn, dvn);
-            commit(st, v, dv);
+            if (st + 1 < n_st) { fetch_x(st + 1, vn); fetch_dpre(st + 1, dvn); }
+            store_x(st, v);
+            store_dpre(st, dv);
             if (st + 1 < n_st) {
                 v[0] = vn[0]; v[1] = vn[1]; dv = dvn;
             }
@@ -753,7 +815,7 @@ __global__ void __launch_bounds__(TB_NT, 2) k_train_bwd_tc(const TrainBwdParams 
             acc = warp_sum(acc);
             if (lane == 0) prm.out_loss[0] = acc * prm.loss_scale;
         }
-    } else {
+    } else if (warp == TC_PRODUCERS / 32) {
         // ===== MMA issuer =====
         if (lane == 0) {
             for (int st = 0; st < n_st; ++st) {
@@ -931,7 +993,8 @@ static int launch_fwd_tc(const dccf_dims* dims, const float* E_item, const float
 static int launch_bwd_tc(const dccf_dims* dims, const float* E_item, const float* Feat, const int64_t* X,
                          const int64_t* sample_item, int64_t n_pairs, const dccf_rng* rng, const float* ws_dpre,
                          float* gW_part, float* gb_part, const float* loss_terms, int64_t n_loss_terms,
-                         float loss_scale, float* out_loss, cudaStream_t stream) {
+                         float loss_scale, float* out_loss, cudaStream_t stream, const dccf_batch_ref* batch = nullptr,
+                         bool programmatic = false) {
     static PerDeviceOnce attr_once;
     if (attr_once.need()) {
         int rc = opt_in_smem(k_train_bwd_tc<0>, "dccf_train_bwd_tc");
@@ -943,6 +1006,7 @@ static int launch_bwd_tc(const dccf_dims* dims, const float* E_item, const float
     const int F = dims->feat_dim, K = D + F, Z = dims->n_samples + 1, R = Z * dims->n_attr;
     TrainBwdParams prm;
     prm.E_item = E_item; prm.Feat = Feat; prm.X = X; prm.sample_item = sample_item; prm.noise = rng->noise;
+    prm.batch_ptrs = batch ? batch->epoch_ptrs_dev : nullptr; prm.batch_cursor = batch ? batch->cursor_dev : nullptr;
     prm.dpre_rows = ws_dpre; prm.gW_part = gW_part; prm.gb_part = gb_part; prm.n_rows = n_pairs * R;
     prm.loss_terms = loss_terms; prm.out_loss = out_loss; prm.n_loss_terms = n_loss_terms; prm.loss_scale = loss_scale;
     prm.n_items = dims->n_items; prm.F = F; prm.S = dims->n_samples; prm.A = dims->n_attr; prm.R = R; prm.K = K;
@@ -950,11 +1014,22 @@ static int launch_bwd_tc(const dccf_dims* dims, const float* E_item, const float
     prm.rng.seed = rng->seed; prm.rng.offset = rng->offset; prm.rng.offset_dev = rng->offset_dev;
     int32_t n_mtiles, n_splits;
     bwd_geometry(prm.n_rows, K, &n_mtiles, &n_splits, &prm.rows_per_split);
-    const dim3 grid((unsigned)n_mtiles, (unsigned)n_splits);
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)n_mtiles, (unsigned)n_splits); cfg.blockDim = dim3(TB_NT);
+    cfg.dynamicSmemBytes = TT_SMEM_BYTES; cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = programmatic ? 1 : 0;
+    cudaError_t le;
     switch (rng->noise_mode) {
-        case 0: k_train_bwd_tc<0><<<grid, TB_NT, TT_SMEM_BYTES, stream>>>(prm); break;
-        case 1: k_train_bwd_tc<1><<<grid, TB_NT, TT_SMEM_BYTES, stream>>>(prm); break;
-        default: k_train_bwd_tc<2><<<grid, TB_NT, TT_SMEM_BYTES, stream>>>(prm); break;
+        case 0: le = cudaLaunchKernelEx(&cfg, k_train_bwd_tc<0>, prm); break;
+        case 1: le = cudaLaunchKernelEx(&cfg, k_train_bwd_tc<1>, prm); break;
+        default: le = cudaLaunchKernelEx(&cfg, k_train_bwd_tc<2>, prm); break;
+    }
+    if (le != cudaSuccess) {
+        set_error("k_train_bwd_tc: launch failed: %s", cudaGetErrorString(le));
+        return DCCF_ERR_CUDA;
     }
     DCCF_CHECK_LAUNCH("k_train_bwd_tc");
     return DCCF_OK;
@@ -1042,7 +1117,9 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     cudaStream_t stream = (cudaStream_t)stream_;
     int rc = check_fwd_args("dccf_train_fwd_bwd_tc", dims, expo, rng, sample_item, n_pairs);
     DCCF_CHECK_ARG(batch == nullptr || (batch->epoch_ptrs_dev != nullptr && batch->cursor_dev != nullptr), "dccf_train_fwd_bwd_tc: batch needs both pointers");
-    DCCF_CHECK_ARG(phases >= 1 && phases <= 15 && (phases & 7) != 0, "dccf_train_fwd_bwd_tc: phases is a mask of 1 (partial products), 2 (middle kernel), 4 (dW / db), + 8 (programmatic launch of phase 1)");
+    DCCF_CHECK_ARG(phases >= 1 && phases <= 63 && (phases & 7) != 0, "dccf_train_fwd_bwd_tc: phases is a mask of 1 (partial products), 2 (middle kernel), 4 (dW / db), + 8 / 16 / 32 (programmatic launch of phase 1 / 2 / 4)");
+    DCCF_CHECK_ARG(!(phases & 16) || (phases & 3) == 3, "dccf_train_fwd_bwd_tc: phases + 16 needs phases 1 and 2 in the same call");
+    DCCF_CHECK_ARG(!(phases & 32) || (phases & 6) == 6, "dccf_train_fwd_bwd_tc: phases + 32 needs phases 2 and 4 in the same call");
     DCCF_CHECK_ARG((expo_e == nullptr) == (expo_den == nullptr), "dccf_train_fwd_bwd_tc: expo_e and expo_den go together");
     if (rc != DCCF_OK) return rc;
     DCCF_CHECK_ARG(loss_mode == 0 || loss_mode == 1, "dccf_train_fwd_bwd_tc: loss_mode must be 0 (BPR) or 1 (MSE)");
@@ -1079,6 +1156,7 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     TrainMidParams mid;
     mid.ex = *expo; mid.E_user = E_user; mid.W = W; mid.bias = b; mid.X = X; mid.sample_item = sample_item; mid.Y = Y;
     mid.mask = rng->mask; mid.pre_part = ws_pre_part; mid.expo_e = expo_e; mid.expo_den = expo_den;
+    mid.batch_ptrs = batch ? batch->epoch_ptrs_dev : nullptr; mid.batch_cursor = batch ? batch->cursor_dev : nullptr;
     mid.out_pred = out_pred; mid.loss_terms = ws_loss_terms;
     mid.dpre_rows = ws_dpre; mid.gu_rec = gu_rec; mid.gi_rec = gi_rec; mid.rec_keys_u = rec_keys_u; mid.rec_keys_i = rec_keys_i;
     mid.save_h = save_h; mid.save_w = save_w; mid.err_flag = err_flag; mid.n_pairs = n_pairs; mid.n_rows = n_pairs * R;
@@ -1090,11 +1168,21 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     mid.rng.seed = rng->seed; mid.rng.offset = rng->offset; mid.rng.offset_dev = rng->offset_dev;
     const int64_t n_terms = (loss_mode == 0) ? n_pairs / 2 : n_pairs;
     if (phases & 2) {
-        k_train_mid<<<(unsigned)n_terms, TM_NT, smem, stream>>>(mid);
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)n_terms); cfg.blockDim = dim3(TM_NT); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = attr; cfg.numAttrs = (phases & 16) ? 1 : 0;
+        const cudaError_t le = cudaLaunchKernelEx(&cfg, k_train_mid, mid);
+        if (le != cudaSuccess) {
+            set_error("k_train_mid: launch failed: %s", cudaGetErrorString(le));
+            return DCCF_ERR_CUDA;
+        }
         DCCF_CHECK_LAUNCH("k_train_mid");
     }
     if (!(phases & 4)) return DCCF_OK;
 
     return launch_bwd_tc(dims, E_item, Feat, X, sample_item, n_pairs, rng, ws_dpre, gW_part, gb_part, ws_loss_terms,
-                         n_terms, loss_mode == 0 ? 1.f : 1.f / (float)n_pairs, out_loss, stream);
+                         n_terms, loss_mode == 0 ? 1.f : 1.f / (float)n_pairs, out_loss, stream, batch, (phases & 32) != 0);
 }

@@ -196,8 +196,9 @@ def train_fwd_bwd_tc(dims, E_user, E_item, Feat, W, b, expo, X, sample_item, Y, 
     """Forward + BPR/MSE loss + backward of a training step: partial products, fused per-loss-term middle kernel,
     dW / db tiles (3 launches, 4 when the W operand images must be rebuilt).  batch = (epoch_ptrs_dev, cursor_dev): the
     partial-product kernel takes its ids from the device-resident epoch itself (X / sample_item are then the staged
-    copies another launch is writing; the later kernels read those).  phases + 8: the partial-product kernel starts as
-    a programmatic dependent of the kernel launched before it on the stream (see include/dccf_b200.h)."""
+    copies another launch is writing; the later kernels read those).  phases + 8 / 16 / 32: the partial-product /
+    middle / dW kernel starts as a programmatic dependent of the kernel launched before it on the stream (see
+    include/dccf_b200.h)."""
     lib = _lib.load()
     n_pairs = X.shape[0]
     ref = None

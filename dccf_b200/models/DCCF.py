@@ -477,7 +477,9 @@ class DCCF(DMF):
             rec['gi_rec'], rec['keys_u'], rec['keys_i'], None, None, expo_e, expo_den, self._err_flag)
         pdl = 8 if (programmatic and w_image_valid) else 0     # phase 1 beside the kernel launched just before it
         if between is None:
-            kernels.train_fwd_bwd_tc(*args, phases=7 | pdl, batch=batch)
+            # one chain: the middle and dW kernels are programmatic dependents of the kernel before them, and do their
+            # prologues while it runs.  (The data-parallel step records an event between them: plain launches.)
+            kernels.train_fwd_bwd_tc(*args, phases=7 | pdl | (16 | 32 if pdl else 0), batch=batch)
         else:                       # kernel by kernel, with the caller's stream plumbing after each
             for phase in (1, 2, 4):
                 kernels.train_fwd_bwd_tc(*args, phases=phase | (pdl if phase == 1 else 0), batch=batch)

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 35
+#define DCCF_ABI_VERSION 36
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -202,12 +202,16 @@ int dccf_train_bwd_tc(const dccf_dims* dims, const float* E_user, const float* E
  *        (cudaLaunchAttributeProgrammaticStreamSerialization): it starts as soon as that kernel — dccf_adam_link_ids,
  *        which signals griddepcontrol.launch_dependents first thing — has started, reads nothing it writes (use
  *        `batch` when the ids are being staged by it) and does not complete before it has; needs w_image_valid.
- *        The middle kernel and the dW / db kernel are always plain launches
+ *        + 16: the middle kernel is a programmatic dependent of the partial-product kernel (needs phases 1 and 2):
+ *        its barrier-free prologue (W_i, b, the RNG key; with `batch` the user rows) runs before it waits.
+ *        + 32: the dW / db kernel is a programmatic dependent of the middle kernel (needs phases 2 and 4): barriers,
+ *        tensor memory and, with `batch`, the x operand of its first stages are set up before it waits for dpre.
+ *        Each kernel completes only after the kernel it depends on has, so the chain stays ordered
  *   batch (optional): the partial-product kernel (phase 1) takes its ids from batch *cursor_dev of a device-resident
  *        epoch (epoch_ptrs_dev[0..1] = base addresses of X_epoch [n, P, 2] / sample_epoch [n, P, S], the arrays
  *        dccf_link_extra's staging reads) instead of X / sample_item — it then does not have to wait for the launch
- *        that stages them (dccf_adam_link_ids), which runs beside it (phases + 8); phases 2 and 4 read X /
- *        sample_item, i.e. the staged copies
+ *        that stages them (dccf_adam_link_ids), which runs beside it (phases + 8); phases 2 and 4 read the same ids
+ *        through it before their wait (phases + 16 / + 32) and X / sample_item, the staged copies, after it
  * Needs dccf_train_fused_smem_bytes(S, A, loss_mode) <= 200 KB of shared memory per CTA (else use the two calls
  * above). */
 typedef struct dccf_batch_ref { const uint64_t* epoch_ptrs_dev; const int64_t* cursor_dev; } dccf_batch_ref;
