@@ -11,7 +11,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
-ABI_VERSION = 36
+ABI_VERSION = 37
 DIM = 64
 
 
@@ -68,7 +68,7 @@ class DpSync(ctypes.Structure):
 
 class LinkExtra(ctypes.Structure):
     _fields_ = [('epoch_ptrs_dev', ctypes.c_void_p), ('cursor_dev', ctypes.c_void_p), ('X_out', ctypes.c_void_p),
-                ('sample_item_out', ctypes.c_void_p), ('stage_counter', ctypes.c_void_p),
+                ('sample_item_out', ctypes.c_void_p), ('Y_out', ctypes.c_void_p), ('stage_counter', ctypes.c_void_p),
                 ('pf_user', ctypes.c_void_p * 3), ('pf_item', ctypes.c_void_p * 3), ('pf_feat', ctypes.c_void_p),
                 ('pf_dense', ctypes.c_void_p * 4), ('pf_dense_bytes', ctypes.c_int64 * 4),
                 ('sync', ctypes.POINTER(DpSync)), ('rec_row_user', ctypes.c_void_p), ('rec_row_item', ctypes.c_void_p)]
@@ -114,7 +114,7 @@ _SIGNATURES = {
                                          _P, _P]),
     'dccf_train_fused_smem_bytes': (ctypes.c_int64, [ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]),
     'dccf_train_fwd_bwd_tc': (ctypes.c_int, [ctypes.POINTER(Dims), _P, _P, _P, _P, _P, ctypes.POINTER(Expo), _P, _P, _P,
-                                             ctypes.c_int64, ctypes.POINTER(Rng), ctypes.c_int32, _P, _P, _P,
+                                             ctypes.c_int64, ctypes.c_int64, ctypes.POINTER(Rng), ctypes.c_int32, _P, _P, _P,
                                              ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
                                              ctypes.POINTER(BatchRef), ctypes.c_int32, _P, _P]),
     'dccf_adam_sweep': (ctypes.c_int, [_P, _P, _P, ctypes.c_int64, _P, _P, ctypes.c_int64, _P, _P,
@@ -139,7 +139,7 @@ _SIGNATURES = {
     'dccf_debug_timeline_train': (ctypes.c_int, [_P]),
     'dccf_debug_timeline_adam': (ctypes.c_int, [_P]),
     'dccf_debug_timeline_dp': (ctypes.c_int, [_P]),
-    'dccf_stage_batch': (ctypes.c_int, [_P, _P, ctypes.c_int64, ctypes.c_int32, _P, _P, _P]),
+    'dccf_stage_batch': (ctypes.c_int, [_P, _P, ctypes.c_int64, ctypes.c_int32, _P, _P, _P, _P]),
     'dccf_state_advance': (ctypes.c_int, [_P, _P, ctypes.c_uint64, _P]),
     'dccf_dp_push': (ctypes.c_int, [_P, ctypes.c_int64, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int64, _P, _P, _P]),
     'dccf_dp_push_fold': (ctypes.c_int, [_P, ctypes.c_int64, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int64, _P, _P,

@@ -598,7 +598,12 @@ __global__ void __launch_bounds__(256) k_link_ids(const LinkIdsArgs a) {
             const int64_t* sis = si + (int64_t)seg * seg_stride_s;
             if (slot == 0) {
                 const int64_t uid = Xs[2 * p];
-                if (staged) a.extra.X_out[2 * p] = uid;
+                if (staged) {
+                    a.extra.X_out[2 * p] = uid;
+                    // rating prediction: the pair's label, from the label epoch in slot 6
+                    if (a.extra.Y_out != nullptr)
+                        a.extra.Y_out[p] = reinterpret_cast<const float*>(a.extra.epoch_ptrs_dev[6])[s_batch * a.n_pairs + p];
+                }
                 if (do_link && !(a.user_seg >= 0 && seg != a.user_seg)) {
                     const int32_t u = checked_id(uid - a.user_base, a.n_users, nullptr);
                     const int32_t r = (int32_t)((a.user_seg >= 0 ? 0 : (int64_t)seg * a.n_pairs) + p);
@@ -915,11 +920,11 @@ __global__ void k_state_advance(int32_t* step_dev, uint64_t* offset_dev, uint64_
 }
 
 // Copy batch number *cursor of a device-resident epoch ([n_batches, P, 2] ids and [n_batches, P, S] confounder
-// draws, base addresses read from device memory) into the step graph's static input buffers, then advance
-// the cursor: a replayed graph walks through the epoch without any host-side copy.
+// draws, with Y_out also [n_batches, P] labels; base addresses read from device memory) into the step graph's static
+// input buffers, then advance the cursor: a replayed graph walks through the epoch without any host-side copy.
 __global__ void __launch_bounds__(1024) k_stage_batch(const uint64_t* __restrict__ epoch_ptrs, int64_t* cursor,
                                                       int64_t n_x, int64_t n_s, int64_t* __restrict__ X_out,
-                                                      int64_t* __restrict__ si_out) {
+                                                      int64_t* __restrict__ si_out, float* __restrict__ Y_out) {
     tl_begin(6);
     tl_end(6);
     const int64_t b = *cursor;
@@ -950,6 +955,10 @@ __global__ void __launch_bounds__(1024) k_stage_batch(const uint64_t* __restrict
     } else {
         for (int64_t i = threadIdx.x; i < n_x; i += blockDim.x) X_out[i] = X_src[i];
         for (int64_t i = threadIdx.x; i < n_s; i += blockDim.x) si_out[i] = s_src[i];
+    }
+    if (Y_out != nullptr) {
+        const float* y_src = reinterpret_cast<const float*>(epoch_ptrs[6]) + b * (n_x >> 1);
+        for (int64_t i = threadIdx.x; i < (n_x >> 1); i += blockDim.x) Y_out[i] = y_src[i];
     }
     __syncthreads();
     if (threadIdx.x == 0) *cursor = b + 1;
@@ -1212,6 +1221,7 @@ extern "C" int dccf_adam_link_ids(const dccf_dims* dims, const int64_t* X, const
     DCCF_CHECK_ARG(!staged || epoch_global || (n_seg <= 1 && extra->cursor_dev && (dims->n_samples == 0 || extra->sample_item_out)),
                    "dccf_adam_link_ids: staging needs n_seg <= 1, the cursor and the output buffers");
     DCCF_CHECK_ARG(!epoch_global || (extra->cursor_dev != nullptr && n_seg >= 1), "dccf_adam_link_ids: the epoch-wide link needs the cursor and n_seg >= 1");
+    DCCF_CHECK_ARG(extra == nullptr || extra->Y_out == nullptr || (staged && !epoch_global), "dccf_adam_link_ids: Y_out needs staging (epoch_ptrs_dev and X_out)");
     if (n_pairs <= 0) return DCCF_OK;
     LinkIdsArgs a;
     a.X = X; a.sample_item = sample_item; a.n_pairs = n_pairs; a.S = dims->n_samples; a.A = dims->n_attr;
@@ -1224,7 +1234,7 @@ extern "C" int dccf_adam_link_ids(const dccf_dims* dims, const int64_t* X, const
         a.extra = *extra;
     } else {
         a.extra.epoch_ptrs_dev = nullptr; a.extra.cursor_dev = nullptr; a.extra.X_out = nullptr;
-        a.extra.sample_item_out = nullptr; a.extra.stage_counter = nullptr; a.extra.pf_feat = nullptr; a.extra.sync = nullptr;
+        a.extra.sample_item_out = nullptr; a.extra.Y_out = nullptr; a.extra.stage_counter = nullptr; a.extra.pf_feat = nullptr; a.extra.sync = nullptr;
         a.extra.rec_row_user = nullptr; a.extra.rec_row_item = nullptr;
         for (int k = 0; k < 3; ++k) { a.extra.pf_user[k] = nullptr; a.extra.pf_item[k] = nullptr; }
         for (int k = 0; k < 4; ++k) { a.extra.pf_dense[k] = nullptr; a.extra.pf_dense_bytes[k] = 0; }
@@ -1387,7 +1397,7 @@ extern "C" int dccf_adam_touched(const dccf_adam_table* tables, int32_t n_tables
 }
 
 extern "C" int dccf_stage_batch(const uint64_t* epoch_ptrs_dev, int64_t* cursor_dev, int64_t n_pairs, int32_t n_samples,
-                                int64_t* X_out, int64_t* sample_item_out, void* stream_) {
+                                int64_t* X_out, int64_t* sample_item_out, float* Y_out, void* stream_) {
     DCCF_CHECK_ARG(epoch_ptrs_dev && cursor_dev && X_out && (n_samples == 0 || sample_item_out), "dccf_stage_batch: null argument");
     DCCF_CHECK_ARG(n_pairs >= 0 && n_samples >= 0, "dccf_stage_batch: negative size");
     if (n_pairs == 0) return DCCF_OK;
@@ -1397,7 +1407,7 @@ extern "C" int dccf_stage_batch(const uint64_t* epoch_ptrs_dev, int64_t* cursor_
         carve_once.mark();
     }
     k_stage_batch<<<1, 1024, 0, (cudaStream_t)stream_>>>(epoch_ptrs_dev, cursor_dev, n_pairs * 2, n_pairs * n_samples, X_out,
-                                                         sample_item_out);
+                                                         sample_item_out, Y_out);
     DCCF_CHECK_LAUNCH("k_stage_batch");
     return DCCF_OK;
 }

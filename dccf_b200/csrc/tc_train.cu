@@ -383,6 +383,7 @@ struct TrainMidParams {
     float* save_w;               // optional
     int32_t* err_flag;
     int64_t n_pairs, n_rows;
+    int64_t mse_pairs;           // MSE: the pairs the mean is over (world * n_pairs in a data-parallel step)
     int32_t n_users, user_base, n_items, S, A, R, Z, K;
     int32_t n_ksplits, mask_mode, loss_mode;
     float keep_prob, drop_scale, inv_A;
@@ -524,7 +525,7 @@ __global__ void __maxnreg__(64) k_train_mid(const TrainMidParams prm) {
         if (tid == 0) prm.loss_terms[jt] = (d > 0.f) ? log1pf(expf(-d)) : (-d + log1pf(expf(d)));
     } else {
         const float d = pred_s[0] - __ldg(prm.Y + jt);
-        dp0 = 2.f * d / (float)prm.n_pairs;
+        dp0 = 2.f * d / (float)prm.mse_pairs;
         if (tid == 0) prm.loss_terms[jt] = d * d;
     }
 
@@ -1107,8 +1108,8 @@ extern "C" int64_t dccf_train_fused_smem_bytes(int32_t n_samples, int32_t n_attr
 
 extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user, const float* E_item, const float* Feat,
                                      const float* W, const float* b, const dccf_expo* expo, const int64_t* X,
-                                     const int64_t* sample_item, const float* Y, int64_t n_pairs, const dccf_rng* rng,
-                                     int32_t loss_mode, float* out_pred, float* out_loss, float* ws_wimg,
+                                     const int64_t* sample_item, const float* Y, int64_t n_pairs, int64_t mse_pairs,
+                                     const dccf_rng* rng, int32_t loss_mode, float* out_pred, float* out_loss, float* ws_wimg,
                                      int32_t w_image_valid, float* ws_pre_part, float* ws_dpre, float* ws_loss_terms,
                                      float* gW_part, float* gb_part, float* gu_rec, float* gi_rec, int32_t* rec_keys_u,
                                      int32_t* rec_keys_i, float* save_h, float* save_w, const float* expo_e,
@@ -1121,6 +1122,7 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     DCCF_CHECK_ARG(!(phases & 16) || (phases & 3) == 3, "dccf_train_fwd_bwd_tc: phases + 16 needs phases 1 and 2 in the same call");
     DCCF_CHECK_ARG(!(phases & 32) || (phases & 6) == 6, "dccf_train_fwd_bwd_tc: phases + 32 needs phases 2 and 4 in the same call");
     DCCF_CHECK_ARG((expo_e == nullptr) == (expo_den == nullptr), "dccf_train_fwd_bwd_tc: expo_e and expo_den go together");
+    DCCF_CHECK_ARG(mse_pairs == 0 || mse_pairs >= n_pairs, "dccf_train_fwd_bwd_tc: mse_pairs=%lld is below n_pairs=%lld (0: n_pairs)", (long long)mse_pairs, (long long)n_pairs);
     if (rc != DCCF_OK) return rc;
     DCCF_CHECK_ARG(loss_mode == 0 || loss_mode == 1, "dccf_train_fwd_bwd_tc: loss_mode must be 0 (BPR) or 1 (MSE)");
     DCCF_CHECK_ARG(E_user && E_item && Feat && W && b && X && out_pred && out_loss && ws_wimg && ws_pre_part && ws_dpre &&
@@ -1160,6 +1162,7 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     mid.out_pred = out_pred; mid.loss_terms = ws_loss_terms;
     mid.dpre_rows = ws_dpre; mid.gu_rec = gu_rec; mid.gi_rec = gi_rec; mid.rec_keys_u = rec_keys_u; mid.rec_keys_i = rec_keys_i;
     mid.save_h = save_h; mid.save_w = save_w; mid.err_flag = err_flag; mid.n_pairs = n_pairs; mid.n_rows = n_pairs * R;
+    mid.mse_pairs = mse_pairs > 0 ? mse_pairs : n_pairs;
     mid.n_users = dims->n_users; mid.user_base = dims->user_base; mid.n_items = dims->n_items; mid.S = dims->n_samples;
     mid.A = dims->n_attr; mid.R = R; mid.Z = Z; mid.K = K; mid.n_ksplits = n_ks; mid.mask_mode = rng->mask_mode;
     mid.loss_mode = loss_mode; mid.keep_prob = 1.0f - rng->p_drop;
@@ -1184,5 +1187,5 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     if (!(phases & 4)) return DCCF_OK;
 
     return launch_bwd_tc(dims, E_item, Feat, X, sample_item, n_pairs, rng, ws_dpre, gW_part, gb_part, ws_loss_terms,
-                         n_terms, loss_mode == 0 ? 1.f : 1.f / (float)n_pairs, out_loss, stream, batch, (phases & 32) != 0);
+                         n_terms, loss_mode == 0 ? 1.f : 1.f / (float)mid.mse_pairs, out_loss, stream, batch, (phases & 32) != 0);
 }

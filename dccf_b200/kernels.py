@@ -192,13 +192,13 @@ def train_fused_supported(n_samples, n_attr, loss_mode):
 def train_fwd_bwd_tc(dims, E_user, E_item, Feat, W, b, expo, X, sample_item, Y, rng, loss_mode, out_pred, out_loss,
                      ws_wimg, w_image_valid, ws_pre_part, ws_dpre, ws_loss_terms, gW_part, gb_part, gu_rec, gi_rec,
                      rec_keys_u, rec_keys_i, save_h=None, save_w=None, expo_e=None, expo_den=None, err_flag=None, phases=7,
-                     batch=None):
+                     batch=None, mse_pairs=0):
     """Forward + BPR/MSE loss + backward of a training step: partial products, fused per-loss-term middle kernel,
     dW / db tiles (3 launches, 4 when the W operand images must be rebuilt).  batch = (epoch_ptrs_dev, cursor_dev): the
     partial-product kernel takes its ids from the device-resident epoch itself (X / sample_item are then the staged
     copies another launch is writing; the later kernels read those).  phases + 8 / 16 / 32: the partial-product /
     middle / dW kernel starts as a programmatic dependent of the kernel launched before it on the stream (see
-    include/dccf_b200.h)."""
+    include/dccf_b200.h).  mse_pairs: the pairs the MSE mean is over (0: this call's; world * P data parallel)."""
     lib = _lib.load()
     n_pairs = X.shape[0]
     ref = None
@@ -206,7 +206,8 @@ def train_fwd_bwd_tc(dims, E_user, E_item, Feat, W, b, expo, X, sample_item, Y, 
         ref = _lib.BatchRef()
         ref.epoch_ptrs_dev, ref.cursor_dev = ptr(batch[0]).value, ptr(batch[1]).value
     check(lib.dccf_train_fwd_bwd_tc(ctypes.byref(dims), ptr(E_user), ptr(E_item), ptr(Feat), ptr(W), ptr(b),
-                                    ctypes.byref(expo), ptr(X), ptr(sample_item), ptr(Y), n_pairs, ctypes.byref(rng),
+                                    ctypes.byref(expo), ptr(X), ptr(sample_item), ptr(Y), n_pairs, int(mse_pairs),
+                                    ctypes.byref(rng),
                                     int(loss_mode), ptr(out_pred), ptr(out_loss), ptr(ws_wimg), int(bool(w_image_valid)),
                                     ptr(ws_pre_part), ptr(ws_dpre), ptr(ws_loss_terms), ptr(gW_part), ptr(gb_part),
                                     ptr(gu_rec), ptr(gi_rec), ptr(rec_keys_u), ptr(rec_keys_i), ptr(save_h), ptr(save_w),
@@ -321,16 +322,19 @@ def adam_csr_build(tables):
 
 def make_link_extra(stage=None, prefetch_user=None, prefetch_item=None, prefetch_feat=None, prefetch_dense=None,
                     sync=None, counter=None, rec_rows=None, epoch_global=None):
-    """Extras of dccf_adam_link_ids.  stage = (epoch_ptrs_dev, cursor_dev, X_out, si_out, counter): the batch is read
-    from a device-resident epoch (replaces dccf_stage_batch).  prefetch_user / prefetch_item = up to three [rows, D]
-    tensors each (parameter and the optimizer state it has), prefetch_feat = Feat, prefetch_dense = up to four tensors: what the
-    step will touch, requested into L2 ahead of its use.  epoch_global = (epoch_ptrs_dev with six slots, cursor_dev): the
+    """Extras of dccf_adam_link_ids.  stage = (epoch_ptrs_dev, cursor_dev, X_out, si_out, counter[, Y_out]): the batch
+    is read from a device-resident epoch (replaces dccf_stage_batch); with Y_out also its labels (epoch_ptrs_dev slot 6).
+    prefetch_user / prefetch_item = up to three [rows, D] tensors each (parameter and the optimizer state it has),
+    prefetch_feat = Feat, prefetch_dense = up to four tensors: what the step will touch, requested into L2 ahead of its
+    use.  epoch_global = (epoch_ptrs_dev, cursor_dev): the
     data-parallel link reads every rank's ids of the current batch from an epoch-wide gather (no per-step id exchange)."""
     e = LinkExtra()
     if stage is not None:
-        ep, cur, X_out, si_out, counter = stage
+        ep, cur, X_out, si_out, counter = stage[:5]
         e.epoch_ptrs_dev, e.cursor_dev = ptr(ep).value, ptr(cur).value
         e.X_out, e.sample_item_out, e.stage_counter = ptr(X_out).value, ptr(si_out).value, ptr(counter).value
+        if len(stage) > 5 and stage[5] is not None:
+            e.Y_out = ptr(stage[5]).value
     if epoch_global is not None:        # data-parallel link from the epoch-wide gather of every rank's ids
         ep, cur = epoch_global
         e.epoch_ptrs_dev, e.cursor_dev = ptr(ep).value, ptr(cur).value
@@ -398,10 +402,10 @@ def train_prep_w_image(W, feat_dim, w_image):
     LAUNCHES[0] += 1
 
 
-def stage_batch(epoch_ptrs_dev, cursor_dev, n_pairs, n_samples, X_out, si_out):
+def stage_batch(epoch_ptrs_dev, cursor_dev, n_pairs, n_samples, X_out, si_out, Y_out=None):
     lib = _lib.load()
     check(lib.dccf_stage_batch(ptr(epoch_ptrs_dev), ptr(cursor_dev), int(n_pairs), int(n_samples), ptr(X_out), ptr(si_out),
-                               stream_ptr()), 'dccf_stage_batch')
+                               ptr(Y_out), stream_ptr()), 'dccf_stage_batch')
     LAUNCHES[0] += 1
 
 

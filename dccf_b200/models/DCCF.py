@@ -434,6 +434,9 @@ class DCCF(DMF):
         return rec
 
     def _launch_bwd(self, call, loss_mode, Y):
+        if loss_mode == 1 and self._dp is not None:
+            # this backward divides by the local batch: a data-parallel MSE step takes the fused step's global divisor
+            raise RuntimeError('data-parallel --rank 0 training needs the fused step (dccf_train_fwd_bwd_tc)')
         N = call['N']
         D = self.ui_vector_size
         F = self.feature_embedding.shape[1]
@@ -456,7 +459,9 @@ class DCCF(DMF):
     def _launch_fwd_bwd(self, call, loss_mode, Y, rec=None, w_image_valid=False, expo_e=None, expo_den=None,
                         between=None, batch=None, programmatic=False):
         """Forward + loss + backward of one step through dccf_train_fwd_bwd_tc (three launches; the activations
-        never leave shared memory).  Returns (prediction, gradient buffers)."""
+        never leave shared memory).  Data parallel, the MSE mean is over the global batch of world * P pairs: the ranks'
+        gradients and loss terms then sum to those of one GPU on the concatenated batch.  Returns (prediction, gradient
+        buffers)."""
         P, N = call['P'], call['N']
         D = self.ui_vector_size
         F = self.feature_embedding.shape[1]
@@ -475,14 +480,15 @@ class DCCF(DMF):
             w_image_valid, self._buf('ws_pre_part', (n_ks, N, D), torch.float32), self._buf('ws_dpre', (N, D), torch.float32),
             self._buf('ws_loss_terms', (P,), torch.float32), rec['gW_part'], rec['gb_part'], rec['gu_rec'],
             rec['gi_rec'], rec['keys_u'], rec['keys_i'], None, None, expo_e, expo_den, self._err_flag)
+        mse_pairs = rec['exchange'].world * P if 'exchange' in rec else 0
         pdl = 8 if (programmatic and w_image_valid) else 0     # phase 1 beside the kernel launched just before it
         if between is None:
             # one chain: the middle and dW kernels are programmatic dependents of the kernel before them, and do their
             # prologues while it runs.  (The data-parallel step records an event between them: plain launches.)
-            kernels.train_fwd_bwd_tc(*args, phases=7 | pdl | (16 | 32 if pdl else 0), batch=batch)
+            kernels.train_fwd_bwd_tc(*args, phases=7 | pdl | (16 | 32 if pdl else 0), batch=batch, mse_pairs=mse_pairs)
         else:                       # kernel by kernel, with the caller's stream plumbing after each
             for phase in (1, 2, 4):
-                kernels.train_fwd_bwd_tc(*args, phases=phase | (pdl if phase == 1 else 0), batch=batch)
+                kernels.train_fwd_bwd_tc(*args, phases=phase | (pdl if phase == 1 else 0), batch=batch, mse_pairs=mse_pairs)
                 between(phase)
         call['pred'] = pred
         return pred, rec
@@ -1043,7 +1049,8 @@ class DCCF(DMF):
     use_cuda_graph = True
     def _build_step_graph(self, P, rank_mode, p_drop, opt, staged):
         """Capture forward + backward + (exchange) + Adam + counter advance for a batch of P pairs.  `staged`:
-        the graph's first node copies the batch from a device-resident epoch (dccf_stage_batch)."""
+        the batch is copied from a device-resident epoch (by k_link_ids, or dccf_stage_batch as the graph's first
+        node) — with rank_mode 0 its labels too."""
         dev = self.uid_embeddings.weight.device
         S = self.sample_num
         # ids and confounder draws of the step in ONE buffer [X (P x 2) | sample_item (P x S)]: a batch that arrives from
@@ -1054,7 +1061,8 @@ class DCCF(DMF):
              'step_dev': torch.zeros(1, dtype=torch.int32, device=dev),
              'offset_dev': torch.zeros(1, dtype=torch.int64, device=dev), 'synced': None}
         if staged:
-            g['epoch_ptrs'] = torch.zeros(6, dtype=torch.int64, device=dev)     # [X, si, X_all, si_all, stride_X, stride_si]
+            # [X, si, X_all, si_all, stride_X, stride_si, Y (rank_mode 0)]
+            g['epoch_ptrs'] = torch.zeros(7, dtype=torch.int64, device=dev)
             g['cursor'] = torch.zeros(1, dtype=torch.int64, device=dev)
             g['stage_counter'] = torch.zeros(1, dtype=torch.int32, device=dev)
         if self._dp is not None and self._split_step_ok(0 if rank_mode == 1 else 1, P):
@@ -1081,10 +1089,10 @@ class DCCF(DMF):
             # the step has no id exchange), by a launch of its own otherwise
             epoch_ids = staged and split and self._dp is not None
             if staged and not split:
-                kernels.stage_batch(g['epoch_ptrs'], g['cursor'], P, S, g['X'], g['si'])
+                kernels.stage_batch(g['epoch_ptrs'], g['cursor'], P, S, g['X'], g['si'], Yg)
             if split:
                 # the W operand images are kept current by dccf_adam_touched (checked before every replay)
-                stage = (g['epoch_ptrs'], g['cursor'], g['X'], g['si'], g['stage_counter']) if staged else None
+                stage = (g['epoch_ptrs'], g['cursor'], g['X'], g['si'], g['stage_counter'], Yg) if staged else None
                 g['epoch_ids'] = epoch_ids
                 pred, loss = self._fused_split_step(call, loss_mode, Yg, opt, hp, True, overlap=True,
                                                     counters=(g['step_dev'], g['offset_dev']), stage=stage,
@@ -1199,21 +1207,29 @@ class DCCF(DMF):
         self._check_ready()
         return bool(self._graph_allowed(P))
 
-    def begin_resident_epoch(self, X_epoch, sample_epoch, dropout, opt=None):
+    def begin_resident_epoch(self, X_epoch, sample_epoch, dropout, opt=None, Y_epoch=None):
         """Training over a device-resident epoch: X_epoch [n, P, 2] and sample_epoch [n, P, S] int64 CUDA tensors
         (all batches of P pairs; the confounder block is ONE torch.randint(item_num, (n*P, S)) call, which yields
         the same numbers as n per-batch calls on the same generator).  Returns a callable: each call runs the next
         batch as one CUDA-graph launch — the batch is fetched by a kernel through a device-side cursor, so the
-        host does nothing per step but launch.  BPR (rank 1) only.  Returns None when graphs cannot be used."""
+        host does nothing per step but launch.  Without Y_epoch the batches are BPR (rank 1) batches; with Y_epoch
+        [n, P] (float32 CUDA, the labels) they are rating-prediction (rank 0, MSE) batches, labels fetched beside the
+        ids.  Returns None when graphs cannot be used."""
         opt = opt or self.optimizer
         if not isinstance(opt, FusedAdamState) or not self.use_cuda_graph:
             return None
         self._check_ready()
         n, P = X_epoch.shape[0], X_epoch.shape[1]
+        rank_mode = 1 if Y_epoch is None else 0
+        if Y_epoch is not None:
+            if tuple(Y_epoch.shape) != (n, P) or Y_epoch.dtype != torch.float32 or Y_epoch.device != X_epoch.device:
+                raise ValueError('Y_epoch must be float32 [%d, %d] on %s, got %s %s on %s'
+                                 % (n, P, X_epoch.device, Y_epoch.dtype, tuple(Y_epoch.shape), Y_epoch.device))
+            Y_epoch = Y_epoch.contiguous()
         if not self._graph_allowed(P) or n == 0:
             return None
         p_drop = float(dropout)
-        key = (P, 1, p_drop, opt, True, self._dp is not None)
+        key = (P, rank_mode, p_drop, opt, True, self._dp is not None)
         graphs = self.__dict__.setdefault('_graphs', {})
         state = {'next': 0}
         if key not in graphs:
@@ -1221,17 +1237,24 @@ class DCCF(DMF):
             saved = self.use_cuda_graph
             self.use_cuda_graph = False
             try:
-                first = self.train_step({'X': X_epoch[0], 'rank': 1, 'train': True, 'dropout': p_drop,
-                                         'sample_item': sample_epoch[0]}, opt)
+                fd = {'X': X_epoch[0], 'rank': rank_mode, 'train': True, 'dropout': p_drop,
+                      'sample_item': sample_epoch[0]}
+                if Y_epoch is not None:
+                    fd['Y'] = Y_epoch[0]
+                first = self.train_step(fd, opt)
             finally:
                 self.use_cuda_graph = saved
             state['next'] = 1
             state['first'] = first
-            graphs[key] = self._build_step_graph(P, 1, p_drop, opt, staged=True)
+            graphs[key] = self._build_step_graph(P, rank_mode, p_drop, opt, staged=True)
         g = graphs[key]
         X_epoch, sample_epoch = X_epoch.contiguous(), sample_epoch.contiguous()
-        ptrs = [X_epoch.data_ptr(), sample_epoch.data_ptr(), 0, 0, 0, 0]
+        ptrs = [X_epoch.data_ptr(), sample_epoch.data_ptr(), 0, 0, 0, 0, 0]
         keep = [X_epoch, sample_epoch]
+        if Y_epoch is not None:
+            # the labels stay on this rank: only its own middle kernel reads them
+            ptrs[6] = Y_epoch.data_ptr()
+            keep.append(Y_epoch)
         if g.get('epoch_ids'):
             # every rank's batches of this epoch (chunk), gathered ONCE: [world, n, P, 2] / [world, n, P, S]
             import torch.distributed as dist
@@ -1240,7 +1263,7 @@ class DCCF(DMF):
             si_all = torch.empty((world,) + tuple(sample_epoch.shape), dtype=torch.int64, device=X_epoch.device)
             dist.all_gather_into_tensor(X_all, X_epoch, group=self._dp['group'])
             dist.all_gather_into_tensor(si_all, sample_epoch, group=self._dp['group'])
-            ptrs[2:] = [X_all.data_ptr(), si_all.data_ptr(), X_epoch.numel(), sample_epoch.numel()]
+            ptrs[2:6] = [X_all.data_ptr(), si_all.data_ptr(), X_epoch.numel(), sample_epoch.numel()]
             keep += [X_all, si_all]
         g['epoch_ptrs'].copy_(torch.tensor(ptrs, dtype=torch.int64))
         g['cursor'].fill_(state['next'])

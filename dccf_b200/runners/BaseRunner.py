@@ -209,16 +209,17 @@ class BaseRunner(object):
         world = self._world(model)
         suspended = None
         if world > 1:
-            if not (fused and hasattr(model, 'begin_resident_epoch') and data_processor.rank == 1):
+            if not (fused and hasattr(model, 'begin_resident_epoch')):
                 raise RuntimeError('data-parallel training (torchrun) supports only the fused step of DCCF (GD, '
-                                   'Adagrad or Adam) with --rank 1: not other models, torch optimizers or --rank 0')
+                                   'Adagrad or Adam): not other models or torch optimizers')
             from ..dist import sync_host_rng
             sync_host_rng(model)            # sharded evaluation left the ranks' generators at different positions
         if fused and hasattr(model, 'begin_resident_epoch') and (len(batches) > 2 or world > 1) \
-                and data_processor.rank == 1 and batches[0]['X'].is_cuda:
+                and batches[0]['X'].is_cuda:
             # Equal-size batches run from a device-resident epoch: the confounder draws of all of them are ONE
             # torch.randint call (same CPU-generator stream as the reference's per-batch calls, DCCF.py:72) and
-            # each step is a single CUDA-graph launch that fetches its batch through a device-side cursor.
+            # each step is a single CUDA-graph launch that fetches its batch (with --rank 0 also its labels) through a
+            # device-side cursor.
             # Data parallel (world > 1): global step k = batches k*world .. k*world + world - 1, one per rank; every
             # rank draws the confounders of all of them (generators stay in step) and keeps its own slice.
             from ..dist import rank_slice_of_draws, step_partition
@@ -241,7 +242,13 @@ class BaseRunner(object):
                 X_epoch = torch.stack([batches[i]['X'] for i in mine[done:done + m]])
                 draws = model.draw_confounders(m * world * P0).view(m * world, P0, model.sample_num)
                 draws = rank_slice_of_draws(draws, world, rank) if world > 1 else draws
-                step = model.begin_resident_epoch(X_epoch, draws.to(X_epoch.device, non_blocking=True), self.dropout)
+                draws = draws.to(X_epoch.device, non_blocking=True)
+                if data_processor.rank == 1:
+                    step = model.begin_resident_epoch(X_epoch, draws, self.dropout)
+                else:
+                    # rating prediction (MSE): this rank's own labels beside its batches
+                    Y_epoch = torch.stack([batches[i]['Y'] for i in mine[done:done + m]]).float()
+                    step = model.begin_resident_epoch(X_epoch, draws, self.dropout, Y_epoch=Y_epoch)
                 if step is None:
                     if world > 1:
                         raise RuntimeError('data-parallel training needs the CUDA-graph step (peer-memory exchange)')

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 36
+#define DCCF_ABI_VERSION 37
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -212,14 +212,18 @@ int dccf_train_bwd_tc(const dccf_dims* dims, const float* E_user, const float* E
  *        dccf_link_extra's staging reads) instead of X / sample_item — it then does not have to wait for the launch
  *        that stages them (dccf_adam_link_ids), which runs beside it (phases + 8); phases 2 and 4 read the same ids
  *        through it before their wait (phases + 16 / + 32) and X / sample_item, the staged copies, after it
+ *   mse_pairs: the number of pairs the MSE mean is taken over (0: n_pairs).  A data-parallel step passes world * n_pairs,
+ *        so that d loss / d pred = 2 (pred - Y) / mse_pairs and the loss term is the rank's share of the mean over the
+ *        global batch; counts below n_pairs are rejected.  BPR ignores it.  The middle kernel reads Y after its wait
+ *        (Y may be the staged copy of a device-resident label epoch, dccf_link_extra.Y_out)
  * Needs dccf_train_fused_smem_bytes(S, A, loss_mode) <= 200 KB of shared memory per CTA (else use the two calls
  * above). */
 typedef struct dccf_batch_ref { const uint64_t* epoch_ptrs_dev; const int64_t* cursor_dev; } dccf_batch_ref;
 int64_t dccf_train_fused_smem_bytes(int32_t n_samples, int32_t n_attr, int32_t loss_mode);
 int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user, const float* E_item, const float* Feat,
                           const float* W, const float* b, const dccf_expo* expo, const int64_t* X,
-                          const int64_t* sample_item, const float* Y, int64_t n_pairs, const dccf_rng* rng,
-                          int32_t loss_mode, float* out_pred, float* out_loss, float* ws_wimg,
+                          const int64_t* sample_item, const float* Y, int64_t n_pairs, int64_t mse_pairs,
+                          const dccf_rng* rng, int32_t loss_mode, float* out_pred, float* out_loss, float* ws_wimg,
                           int32_t w_image_valid, float* ws_pre_part, float* ws_dpre, float* ws_loss_terms,
                           float* gW_part, float* gb_part, float* gu_rec, float* gi_rec, int32_t* rec_keys_u,
                           int32_t* rec_keys_i, float* save_h, float* save_w, const float* expo_e,
@@ -357,7 +361,9 @@ typedef struct dccf_dp_sync {
  *   staging (epoch_ptrs_dev != NULL): the step reads its batch from a device-resident epoch — what dccf_stage_batch does
  *     in a launch of its own: X / sample_item arguments are ignored, the batch is [*cursor] of the arrays whose
  *     addresses sit in epoch_ptrs_dev {X_epoch [n,P,2], sample_epoch [n,P,S]}; every id is copied into X_out /
- *     sample_item_out (the buffers the later kernels of the step read) by the thread that links it.  The cursor is NOT
+ *     sample_item_out (the buffers the later kernels of the step read) by the thread that links it.  Y_out (optional,
+ *     rating prediction): the labels of the batch, float32 from the label epoch Y_epoch [n,P] whose address sits in
+ *     epoch_ptrs_dev[6], are copied into Y_out [P] by the thread that copies the pair's user id.  The cursor is NOT
  *     moved here: the partial-product kernel may be reading the same batch beside this launch (dccf_batch_ref);
  *     dccf_adam_touched (advance_cursor_dev) moves it when the step is over.  Needs n_seg <= 1.
  *   L2 prefetch (any pointer may be NULL): the rows this step will touch — the pairs' user rows, the slot items' rows
@@ -367,7 +373,7 @@ typedef struct dccf_dp_sync {
  *   sync: data-parallel link of the GLOBAL step — wait for the peers' ids in the prologue, hand the id buffer back in
  *     the last CTA (stage_counter: int32 CTA counter, zero on entry / exit). */
 typedef struct dccf_link_extra {
-    const uint64_t* epoch_ptrs_dev; int64_t* cursor_dev; int64_t* X_out; int64_t* sample_item_out;
+    const uint64_t* epoch_ptrs_dev; int64_t* cursor_dev; int64_t* X_out; int64_t* sample_item_out; float* Y_out;
     int32_t* stage_counter;
     const float* pf_user[3];     /* E_user, exp_avg, exp_avg_sq   [n_users, D] */
     const float* pf_item[3];     /* E_item, exp_avg, exp_avg_sq   [n_items, D] */
@@ -391,10 +397,11 @@ int dccf_adam_touched(const dccf_adam_table* tables, int32_t n_tables, const dcc
                       uint64_t* advance_offset_dev, int64_t* advance_cursor_dev, const dccf_dp_sync* sync, void* stream);
 int dccf_train_prep_w_image(const float* W, int32_t feat_dim, float* w_image, void* stream);
 /* First node of a captured training step that reads its inputs from a device-resident epoch:
- * epoch_ptrs_dev = device array {address of X_epoch [n_batches,P,2], address of sample_epoch [n_batches,P,S]},
- * cursor_dev = device int64 batch counter (copied batch *cursor, then incremented). */
+ * epoch_ptrs_dev = device array {address of X_epoch [n_batches,P,2], address of sample_epoch [n_batches,P,S]; with
+ * Y_out also slot 6 = address of the label epoch Y_epoch [n_batches,P] float32}, cursor_dev = device int64 batch
+ * counter (copied batch *cursor, then incremented).  Y_out (optional): the batch's labels (rating prediction). */
 int dccf_stage_batch(const uint64_t* epoch_ptrs_dev, int64_t* cursor_dev, int64_t n_pairs, int32_t n_samples,
-                     int64_t* X_out, int64_t* sample_item_out, void* stream);
+                     int64_t* X_out, int64_t* sample_item_out, float* Y_out, void* stream);
 /* step_dev[0] += 1 ; offset_dev[0] += offset_inc  (either pointer may be NULL) — the last node
  * of a captured training step, so that a replay sees t+1 and a fresh rng counter. */
 int dccf_state_advance(int32_t* step_dev, uint64_t* offset_dev, uint64_t offset_inc, void* stream);

@@ -2,10 +2,11 @@
 single-GPU step on the concatenated batch, replicas stay bit-identical, user-sharded evaluation equals the
 single-GPU evaluation.  Prints 'DP CHECK OK' on rank 0.
 
-    torchrun --nproc-per-node 2 tools/dp_check.py [--optimizer adam|gd|adagrad]
+    torchrun --nproc-per-node 2 tools/dp_check.py [--optimizer adam|gd|adagrad] [--rank 0|1]
 
 --optimizer: the fused optimizer of both runs (default adam); its state (exp_avg for Adam, state_sum for Adagrad) is
-compared as well."""
+compared as well.  --rank: the task of src/main.py, 1 (default) top-N ranking with the BPR loss, 0 rating prediction
+with the MSE loss — there the loss of a global step is the mean over the pairs of all ranks, compared as well."""
 import argparse
 import os
 import sys
@@ -43,7 +44,9 @@ def close(a, b, tol, what):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--optimizer', choices=('adam', 'gd', 'adagrad'), default='adam')
-    kind = ap.parse_args().optimizer
+    ap.add_argument('--rank', type=int, choices=(0, 1), default=1)
+    cli = ap.parse_args()
+    kind, task = cli.optimizer, cli.rank
     rank, world, local = int(os.environ['RANK']), int(os.environ['WORLD_SIZE']), int(os.environ['LOCAL_RANK'])
     torch.cuda.set_device(local)
     dist.init_process_group('nccl', device_id=torch.device('cuda', local))
@@ -53,17 +56,23 @@ def main():
     params, X, si, noise, mask = random_problem(17, U, I, F, P, S, A, std, drop)
     R = (S + 1) * A
     b = P // 2
-    # rank r owns positives [r*b_loc, (r+1)*b_loc) and their negatives
-    pos = np.arange(rank * b_loc, (rank + 1) * b_loc)
-    pairs = np.concatenate([pos, b + pos])
+    if task == 1:
+        # rank r owns positives [r*b_loc, (r+1)*b_loc) and their negatives
+        pos = np.arange(rank * b_loc, (rank + 1) * b_loc)
+        pairs = np.concatenate([pos, b + pos])
+        labels = np.zeros(P, dtype=np.float32)
+    else:
+        # rank r owns pairs [r*2*b_loc, (r+1)*2*b_loc) with their ratings
+        pairs = np.arange(rank * 2 * b_loc, (rank + 1) * 2 * b_loc)
+        labels = np.random.RandomState(3).uniform(1.0, 5.0, P).astype(np.float32)
     rows = (pairs[:, None] * R + np.arange(R)[None, :]).reshape(-1)
     model = make_model(params, S, A, std)
     model.enable_data_parallel(p2p=os.environ.get('DCCF_DP_P2P', '1') == '1')
     model.optimizer = model.make_fused_optimizer(lr=1e-3, l2=1e-4, kind=kind)
     steps = 2
     for t in range(steps):
-        fd = {'X': torch.from_numpy(X[pairs]).cuda(), 'rank': 1, 'train': True, 'dropout': drop,
-              'Y': torch.zeros(len(pairs)).cuda(), 'sample_item': torch.from_numpy(si[pairs]),
+        fd = {'X': torch.from_numpy(X[pairs]).cuda(), 'rank': task, 'train': True, 'dropout': drop,
+              'Y': torch.from_numpy(labels[pairs]).cuda(), 'sample_item': torch.from_numpy(si[pairs]),
               'noise': torch.from_numpy(noise[rows]), 'dropout_mask': torch.from_numpy(mask[rows])}
         out = model.train_step(fd)
     say(rank, 'dp steps done (exchange=%s), loss %.6f' % (model._exchange_for(len(pairs)).mode, float(out['loss'])))
@@ -78,7 +87,8 @@ def main():
     single = make_model(params, S, A, std)
     single.optimizer = single.make_fused_optimizer(lr=1e-3, l2=1e-4, kind=kind)
     for t in range(steps):
-        fd = {'X': torch.from_numpy(X).cuda(), 'rank': 1, 'train': True, 'dropout': drop, 'Y': torch.zeros(P).cuda(),
+        fd = {'X': torch.from_numpy(X).cuda(), 'rank': task, 'train': True, 'dropout': drop,
+              'Y': torch.from_numpy(labels).cuda(),
               'sample_item': torch.from_numpy(si), 'noise': torch.from_numpy(noise),
               'dropout_mask': torch.from_numpy(mask)}
         out1 = single.train_step(fd)
@@ -96,8 +106,8 @@ def main():
     say(rank, 'equality with the single-GPU step ok')
     # DP steps on the library's own rng streams keep the replicas identical too
     for t in range(4):
-        fd = {'X': torch.from_numpy(X[pairs]).cuda(), 'rank': 1, 'train': True, 'dropout': drop,
-              'Y': torch.zeros(len(pairs)).cuda(), 'sample_item': torch.from_numpy(si[pairs])}
+        fd = {'X': torch.from_numpy(X[pairs]).cuda(), 'rank': task, 'train': True, 'dropout': drop,
+              'Y': torch.from_numpy(labels[pairs]).cuda(), 'sample_item': torch.from_numpy(si[pairs])}
         model.train_step(fd)
     for k, v in model_params(model).items():
         t = torch.from_numpy(v).cuda()
@@ -126,7 +136,7 @@ def main():
     assert np.abs(np.array(got_m) - np.array(want_m)).max() < 1e-9, (got_m, want_m)
     dist.barrier()
     if rank == 0:
-        print('DP CHECK OK world=%d optimizer=%s' % (world, kind))
+        print('DP CHECK OK world=%d optimizer=%s rank=%d' % (world, kind, task))
     dist.destroy_process_group()
 
 
