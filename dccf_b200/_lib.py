@@ -11,7 +11,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
-ABI_VERSION = 37
+ABI_VERSION = 38
 DIM = 64
 
 
@@ -151,7 +151,7 @@ _SIGNATURES = {
     'dccf_full_scores_splits': (ctypes.c_int32, [ctypes.c_int32, ctypes.c_int32]),
     'dccf_full_scores_ws_floats': (ctypes.c_int64, [ctypes.c_int32]),
     'dccf_full_scores': (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, _P, _P, _P, _P, _P, ctypes.c_float, _P,
-                                        ctypes.c_int32, _P, _P, _P, _P, _P, _P]),
+                                        ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, _P]),
     'dccf_sample_negatives': (ctypes.c_int, [_P, _P, _P, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int64,
                                              ctypes.c_int64, _P, _P, _P, _P, _P]),
     'dccf_confounder_draw': (ctypes.c_int, [_P, _P, _P, ctypes.c_int64, ctypes.c_int64, _P]),
@@ -160,6 +160,8 @@ _SIGNATURES = {
     'dccf_rank_eval_ws_bytes': (ctypes.c_int64, [ctypes.c_int64]),
     'dccf_rank_eval_multi': (ctypes.c_int, [_P, _P, _P, _P, _P, ctypes.c_int64, ctypes.POINTER(ctypes.c_int32),
                                             ctypes.c_int32, _P, _P, _P, _P, _P, _P]),
+    'dccf_topk_metrics': (ctypes.c_int, [_P, ctypes.c_int64, ctypes.c_int32, _P, _P, ctypes.POINTER(ctypes.c_int32),
+                                         ctypes.c_int32, _P, _P, _P, _P, _P]),
 }
 
 _LIB = None

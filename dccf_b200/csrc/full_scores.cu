@@ -62,6 +62,8 @@ struct FsParams {
     int64_t* topk_id;        // [2*splits,U,k]
     int32_t n_users, n_items, k;
     int32_t tiles_per_split, n_tiles;
+    const int64_t* excl_off;     // [U+1] CSR over the rows of A (EXCL only)
+    const int32_t* excl_items;   // each row's excluded items, ascending, unique, < n_items
 };
 
 // byte offset of 4 consecutive k values of row r inside a hi (or lo) half of an item-tile image
@@ -101,7 +103,8 @@ __global__ void __launch_bounds__(128) k_fs_prep_b(const float* __restrict__ B, 
 }
 
 // TOPK: fused per-user top-k (k <= KCAP); the matrix is written when prm.out is given (either or both).
-template <bool TOPK, int KCAP>
+// EXCL (with TOPK, without the matrix): each row's items in prm.excl_off / prm.excl_items score -inf and never rank.
+template <bool TOPK, int KCAP, bool EXCL>
 __global__ void __launch_bounds__(FS_NT, 1) k_full_scores(const FsParams prm) {
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t* stage0 = smem;
@@ -228,6 +231,22 @@ __global__ void __launch_bounds__(FS_NT, 1) k_full_scores(const FsParams prm) {
         for (int j = 0; j < KCAP; ++j) { top_s[j] = -INFINITY; top_i[j] = -1; }
         const int k = prm.k;
         float* my_out = out_s + warp * 32 * FS_OUT_LD;
+        // exclusion cursor: this thread's items arrive in ascending id order, so the row's sorted list is merged
+        // against them.  nxt = the first listed item not yet passed; one binary search places it at the split's
+        // first item, and every read stays inside [c, c_end) whatever the list holds.
+        int64_t c = 0, c_end = 0;
+        int32_t nxt = INT32_MAX;
+        if (EXCL && valid) {
+            c = __ldg(prm.excl_off + u);
+            c_end = __ldg(prm.excl_off + u + 1);
+            const int32_t first = t_lo * FS_BN;
+            int64_t hi = c_end;
+            while (c < hi) {
+                const int64_t mid = (c + hi) >> 1;
+                if (__ldg(prm.excl_items + mid) < first) c = mid + 1; else hi = mid;
+            }
+            if (c < c_end) nxt = __ldg(prm.excl_items + c);
+        }
         for (int t = t_lo; t < t_hi; ++t) {
             const int n = t - t_lo, a = n & 1;
             const uint32_t ph = (uint32_t)(n >> 1) & 1u;
@@ -247,6 +266,15 @@ __global__ void __launch_bounds__(FS_NT, 1) k_full_scores(const FsParams prm) {
             float v[32];
 #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(rm[j]) + __uint_as_float(rc[j]);
+            uint32_t excl_mask = 0;     // bit j: item i0 + j is excluded
+            if (EXCL) {
+                const int32_t lo32 = (int32_t)i0;
+                while (nxt < lo32 + 32) {                   // items below i0 (the other column half's) are passed over
+                    if (nxt >= lo32) excl_mask |= 1u << (nxt - lo32);
+                    ++c;
+                    nxt = (c < c_end) ? __ldg(prm.excl_items + c) : INT32_MAX;
+                }
+            }
             if (TOPK) {
                 // columns beyond the catalogue (last tile only) never rank; NaN never compares greater and stays out
                 const int64_t live = (int64_t)prm.n_items - i0;
@@ -254,6 +282,7 @@ __global__ void __launch_bounds__(FS_NT, 1) k_full_scores(const FsParams prm) {
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
                     if (live < 32 && j >= live) v[j] = -INFINITY;
+                    if (EXCL && (excl_mask >> j & 1u)) v[j] = -INFINITY;   // compile-time j: v stays in registers
                     best = fmaxf(best, v[j]);
                 }
                 if (best > top_s[0]) {
@@ -369,7 +398,8 @@ extern "C" int64_t dccf_full_scores_ws_floats(int32_t n_items) {
 extern "C" int dccf_full_scores(int32_t n_users, int32_t n_items, const float* A, const float* B,
                                 const float* row_bias, const float* col_bias, const float* col_scale, float g,
                                 float* out, int32_t k, float* topk_score, int64_t* topk_id, float* ws_score,
-                                int64_t* ws_id, float* ws_items, void* stream_) {
+                                int64_t* ws_id, float* ws_items, const int64_t* excl_off, const int32_t* excl_items,
+                                void* stream_) {
     cudaStream_t stream = (cudaStream_t)stream_;
     DCCF_CHECK_ARG(A && B, "dccf_full_scores: null factor matrix");
     DCCF_CHECK_ARG(out || (topk_score && topk_id), "dccf_full_scores: nothing to produce (out and top-k both null)");
@@ -377,6 +407,9 @@ extern "C" int dccf_full_scores(int32_t n_users, int32_t n_items, const float* A
     DCCF_CHECK_ARG(topk_score == nullptr || (k >= 1 && k <= FS_KMAX), "dccf_full_scores: fused top-k supports 1 <= k <= %d, got %d", FS_KMAX, k);
     DCCF_CHECK_ARG(ws_items != nullptr && (reinterpret_cast<uintptr_t>(ws_items) & 127) == 0,
                    "dccf_full_scores: ws_items (dccf_full_scores_ws_floats(n_items) floats, 128-byte aligned) is required");
+    DCCF_CHECK_ARG((excl_off == nullptr) == (excl_items == nullptr), "dccf_full_scores: exclusion needs both excl_off and excl_items");
+    DCCF_CHECK_ARG(excl_off == nullptr || (topk_score != nullptr && out == nullptr),
+                   "dccf_full_scores: known-item exclusion applies to the fused top-k only (out must be NULL)");
     if (n_users <= 0 || n_items <= 0) return DCCF_OK;
     const int lists = dccf_full_scores_splits(n_users, n_items);
     const int splits = lists / 2;
@@ -388,11 +421,15 @@ extern "C" int dccf_full_scores(int32_t n_users, int32_t n_items, const float* A
     prm.tiles_per_split = (prm.n_tiles + splits - 1) / splits;
     prm.topk_score = topk_score ? ws_score : nullptr;
     prm.topk_id = topk_score ? ws_id : nullptr;
+    prm.excl_off = excl_off;
+    prm.excl_items = excl_items;
     static PerDeviceOnce attr_once;
     if (attr_once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_full_scores<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_full_scores<true, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_full_scores<true, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
+        cudaError_t e = cudaFuncSetAttribute(k_full_scores<false, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_full_scores<true, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_full_scores<true, 16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_full_scores<true, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_full_scores<true, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FS_SMEM);
         if (e != cudaSuccess) {
             set_error("dccf_full_scores: cannot opt in to %u bytes of shared memory: %s", FS_SMEM, cudaGetErrorString(e));
             return DCCF_ERR_CUDA;
@@ -402,9 +439,12 @@ extern "C" int dccf_full_scores(int32_t n_users, int32_t n_items, const float* A
     k_fs_prep_b<<<(unsigned)prm.n_tiles, 128, 0, stream>>>(B, col_bias, col_scale, n_items, ws_items);
     DCCF_CHECK_LAUNCH("k_fs_prep_b");
     dim3 grid((unsigned)((n_users + FS_BM - 1) / FS_BM), (unsigned)splits);
-    if (!topk_score) k_full_scores<false, 1><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
-    else if (k <= 8) k_full_scores<true, 8><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
-    else k_full_scores<true, 16><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
+    if (!topk_score) k_full_scores<false, 1, false><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
+    else if (excl_off) {
+        if (k <= 8) k_full_scores<true, 8, true><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
+        else k_full_scores<true, 16, true><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
+    } else if (k <= 8) k_full_scores<true, 8, false><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
+    else k_full_scores<true, 16, false><<<grid, FS_NT, FS_SMEM, stream>>>(prm);
     DCCF_CHECK_LAUNCH("k_full_scores");
     if (topk_score) {
         k_topk_merge<<<(unsigned)((n_users + 127) / 128), 128, 0, stream>>>(ws_score, ws_id, lists, n_users, k, topk_score, topk_id);

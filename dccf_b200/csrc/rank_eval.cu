@@ -22,6 +22,8 @@
 // Order: score descending, then item id ascending, then row ascending — a total order, so the result is
 // deterministic (the reference's quicksort leaves ties unordered).  NaN scores rank last, as pandas does.
 // k_rank_select (any k <= 1024): the k-rounds selection kernel, kept for k > 16.
+// k_topk_metrics: the same metrics for full-catalogue top-k lists (dccf_full_scores with known-item exclusion) against
+// each user's held-out positives, summed over users in the same fixed order.
 #include <math.h>
 
 #include "common.cuh"
@@ -445,9 +447,127 @@ __global__ void __launch_bounds__(RANK_WARPS * 32) k_rank_select(
     }
 }
 
+// Metrics of ranked full-catalogue lists: one warp per user, lane t looks up the item at rank t in the user's sorted
+// positives (binary search; the list has at most 16 entries, the positives are few).  The label at rank t is 1 for a hit;
+// the ideal list puts the n_pos positives first.  Per-user values, per-warp accumulation and the sums over users follow
+// k_rank_stream exactly (its code is repeated here, not shared, so that the ranker's instructions stay what they are).
+__global__ void __launch_bounds__(RANK_WARPS * 32) k_topk_metrics(
+    const int64_t* __restrict__ topk_id, int64_t n_users, int32_t k_list, const int64_t* __restrict__ pos_off,
+    const int32_t* __restrict__ pos_items, const RankKs ks, double* __restrict__ out_metrics,
+    double* __restrict__ part_sums, int32_t* __restrict__ cta_counter, double* __restrict__ out_sums,
+    unsigned long long* __restrict__ out_count) {
+    __shared__ double acc_s[RANK_WARPS][RANK_MAX_NK * RANK_NCOL];
+    __shared__ int s_last;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int ncol = ks.n_k * RANK_NCOL;
+    if (lane < RANK_MAX_NK * RANK_NCOL) acc_s[warp][lane] = 0.0;
+    __syncwarp();
+    const int kmax = ks.kmax;
+    const int64_t n_warps = (int64_t)gridDim.x * RANK_WARPS;
+    unsigned long long counted = 0;
+
+    for (int64_t g = (int64_t)blockIdx.x * RANK_WARPS + warp; g < n_users; g += n_warps) {   // warp-uniform
+        const int64_t lo = pos_off[g], hi = pos_off[g + 1];
+        const int64_t n_pos = hi - lo;
+        if (n_pos <= 0) {
+            if (out_metrics != nullptr && lane < ncol) out_metrics[g * ncol + lane] = __longlong_as_double(0x7ff8000000000000LL);
+            continue;
+        }
+        float my_label = 0.f;
+        if (lane < k_list) {
+            const int64_t id = __ldg(topk_id + g * k_list + lane);
+            if (id >= 0) {
+                int64_t a = lo, b = hi;
+                while (a < b) {
+                    const int64_t mid = (a + b) >> 1;
+                    if ((int64_t)__ldg(pos_items + mid) < id) a = mid + 1; else b = mid;
+                }
+                my_label = (a < hi && (int64_t)__ldg(pos_items + a) == id) ? 1.f : 0.f;
+            }
+        }
+        double dcg = 0.0, idcg = 0.0, hit_sum = 0.0;
+        int next_k = 0;
+#pragma unroll 1
+        for (int t = 0; t < kmax; ++t) {
+            const float lab = __shfl_sync(0xffffffffu, my_label, t);
+            const double inv = c_inv_log2_pos[t];
+            dcg += (lab == 0.f) ? 0.0 : inv;
+            idcg += (t < n_pos) ? inv : 0.0;
+            hit_sum += (double)lab;
+            while (next_k < ks.n_k && ks.k[next_k] == t + 1) {     // ks ascending
+                if (lane == 0) {
+                    const double k = (double)(t + 1), np = (double)n_pos;
+                    double m[RANK_NCOL];
+                    m[0] = dcg / idcg;                  // idcg > 0: n_pos >= 1
+                    m[1] = (hit_sum > 0.0) ? 1.0 : 0.0;
+                    m[2] = hit_sum / k;
+                    m[3] = hit_sum / np;
+                    m[4] = 2.0 * hit_sum / (k + np);
+#pragma unroll
+                    for (int q = 0; q < RANK_NCOL; ++q) {
+                        if (out_metrics != nullptr) out_metrics[(g * ks.n_k + next_k) * RANK_NCOL + q] = m[q];
+                        acc_s[warp][next_k * RANK_NCOL + q] += m[q];
+                    }
+                }
+                ++next_k;
+            }
+        }
+        ++counted;
+        __syncwarp();
+    }
+    if (out_count != nullptr && lane == 0 && counted > 0) atomicAdd(out_count, counted);    // integer: order-free
+
+    // ---- sums over users in a fixed order: warps of the CTA, then (last CTA) the CTAs in index order ------
+    if (out_sums == nullptr) return;
+    __syncthreads();
+    if ((int)threadIdx.x < ncol) {
+        double v = 0.0;
+        for (int w = 0; w < RANK_WARPS; ++w) v += acc_s[w][threadIdx.x];
+        part_sums[(size_t)blockIdx.x * (RANK_MAX_NK * RANK_NCOL) + threadIdx.x] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        const int32_t prev = atomicAdd(cta_counter, 1);
+        s_last = (prev == (int32_t)gridDim.x - 1) ? 1 : 0;
+        if (s_last) {
+            __threadfence();
+            *cta_counter = 0;
+        }
+    }
+    __syncthreads();
+    if (!s_last) return;
+    for (int col = warp; col < ncol; col += RANK_WARPS) {
+        double v = 0.0;
+        for (int b = lane; b < (int)gridDim.x; b += 32) v += __ldcg(part_sums + (size_t)b * (RANK_MAX_NK * RANK_NCOL) + col);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (lane == 0) out_sums[col] = v;
+    }
+}
+
 }  // namespace dccf
 
 using namespace dccf;
+
+// the c_log2_pos / c_inv_log2_pos tables, once per device
+static int install_log2_tables(const char* who) {
+    static PerDeviceOnce table_once;
+    if (!table_once.need()) return DCCF_OK;
+    double h[16], hi[16];
+    for (int t = 0; t < 16; ++t) {
+        h[t] = log2((double)(t + 2));
+        hi[t] = 1.0 / h[t];
+    }
+    cudaError_t e = cudaMemcpyToSymbol(c_log2_pos, h, sizeof(h));
+    if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_inv_log2_pos, hi, sizeof(hi));
+    if (e != cudaSuccess) {
+        set_error("%s: cannot install the log2 table: %s", who, cudaGetErrorString(e));
+        return DCCF_ERR_CUDA;
+    }
+    table_once.mark();
+    return DCCF_OK;
+}
 
 extern "C" int64_t dccf_rank_eval_ws_bytes(int64_t n_users) {
     (void)n_users;
@@ -477,21 +597,8 @@ extern "C" int dccf_rank_eval_multi(const float* scores, const float* labels, co
         if (out_sums) cudaMemsetAsync(out_sums, 0, sizeof(double) * n_k * RANK_NCOL, stream);
         return DCCF_OK;
     }
-    static PerDeviceOnce table_once;
-    if (table_once.need()) {
-        double h[16], hi[16];
-        for (int t = 0; t < 16; ++t) {
-            h[t] = log2((double)(t + 2));
-            hi[t] = 1.0 / h[t];
-        }
-        cudaError_t e = cudaMemcpyToSymbol(c_log2_pos, h, sizeof(h));
-        if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_inv_log2_pos, hi, sizeof(hi));
-        if (e != cudaSuccess) {
-            set_error("dccf_rank_eval_multi: cannot install the log2 table: %s", cudaGetErrorString(e));
-            return DCCF_ERR_CUDA;
-        }
-        table_once.mark();
-    }
+    const int rc = install_log2_tables("dccf_rank_eval_multi");
+    if (rc != DCCF_OK) return rc;
     int64_t ctas = (n_users + RANK_WARPS - 1) / RANK_WARPS;
     if (ctas > 148 * 4) ctas = 148 * 4;
     double* part = reinterpret_cast<double*>(ws);
@@ -516,5 +623,47 @@ extern "C" int dccf_rank_eval(const float* scores, const float* labels, const in
     k_rank_select<<<(unsigned)((n_users + RANK_WARPS - 1) / RANK_WARPS), RANK_WARPS * 32, 0, stream>>>(
         scores, labels, iids, cand_rows, user_off, n_users, k, out_topk_iid, out_topk_row, out_metrics);
     DCCF_CHECK_LAUNCH("k_rank_select");
+    return DCCF_OK;
+}
+
+extern "C" int dccf_topk_metrics(const int64_t* topk_id, int64_t n_users, int32_t k_list, const int64_t* pos_off,
+                                 const int32_t* pos_items, const int32_t* ks_host, int32_t n_k, double* out_metrics, void* ws,
+                                 double* out_sums, int64_t* out_count, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    DCCF_CHECK_ARG(topk_id && pos_off, "dccf_topk_metrics: null buffer");
+    DCCF_CHECK_ARG(k_list >= 1 && k_list <= RANK_STREAM_MAX_K, "dccf_topk_metrics: list length %d outside [1,%d]", k_list, RANK_STREAM_MAX_K);
+    DCCF_CHECK_ARG(ks_host && n_k >= 1 && n_k <= RANK_MAX_NK, "dccf_topk_metrics: 1 to %d values of k per call", RANK_MAX_NK);
+    DCCF_CHECK_ARG(out_metrics || out_sums || out_count, "dccf_topk_metrics: no output requested");
+    DCCF_CHECK_ARG(out_sums == nullptr || ws != nullptr, "dccf_topk_metrics: the sums need the workspace (dccf_rank_eval_ws_bytes)");
+    RankKs ks;
+    ks.n_k = n_k;
+    for (int i = 0; i < RANK_MAX_NK; ++i) ks.k[i] = 0;
+    for (int i = 0; i < n_k; ++i) {
+        DCCF_CHECK_ARG(ks_host[i] >= 1 && ks_host[i] <= k_list, "dccf_topk_metrics: k=%d outside [1,%d] (the list length)", ks_host[i], k_list);
+        DCCF_CHECK_ARG(i == 0 || ks_host[i] > ks_host[i - 1], "dccf_topk_metrics: the values of k must be strictly ascending");
+        ks.k[i] = ks_host[i];
+    }
+    ks.kmax = ks.k[n_k - 1];
+    if (out_count) {
+        const cudaError_t e = cudaMemsetAsync(out_count, 0, sizeof(int64_t), stream);
+        if (e != cudaSuccess) {
+            set_error("dccf_topk_metrics: cannot clear the user count: %s", cudaGetErrorString(e));
+            return DCCF_ERR_CUDA;
+        }
+    }
+    if (n_users <= 0) {
+        if (out_sums) cudaMemsetAsync(out_sums, 0, sizeof(double) * n_k * RANK_NCOL, stream);
+        return DCCF_OK;
+    }
+    const int rc = install_log2_tables("dccf_topk_metrics");
+    if (rc != DCCF_OK) return rc;
+    int64_t ctas = (n_users + RANK_WARPS - 1) / RANK_WARPS;
+    if (ctas > 148 * 4) ctas = 148 * 4;
+    double* part = reinterpret_cast<double*>(ws);
+    int32_t* counter = ws ? reinterpret_cast<int32_t*>(reinterpret_cast<uint8_t*>(ws) + (size_t)(148 * 4) * RANK_MAX_NK * RANK_NCOL * sizeof(double)) : nullptr;
+    k_topk_metrics<<<(unsigned)ctas, RANK_WARPS * 32, 0, stream>>>(topk_id, n_users, k_list, pos_off, pos_items, ks, out_metrics,
+                                                                   part, counter, out_sums,
+                                                                   reinterpret_cast<unsigned long long*>(out_count));
+    DCCF_CHECK_LAUNCH("k_topk_metrics");
     return DCCF_OK;
 }

@@ -455,9 +455,10 @@ def rank_eval_multi(scores, labels, iids, cand_rows, user_off, ks, out_metrics=N
 _FS_WS = {}
 
 
-def full_scores(A, B, row_bias=None, col_bias=None, col_scale=None, g=0.0, materialise=True, k=0):
+def full_scores(A, B, row_bias=None, col_bias=None, col_scale=None, g=0.0, materialise=True, k=0, exclude=None):
     """Full-catalogue scoring on the tensor cores (dccf_full_scores).  Returns (matrix [U,I] or None,
-    topk_score [U,k] or None, topk_id [U,k] or None)."""
+    topk_score [U,k] or None, topk_id [U,k] or None).  exclude = (off int64 [U+1], items int32) CUDA tensors: each
+    row's known items, dropped from its top-k (not with the matrix)."""
     lib = _lib.load()
     U, I = A.shape[0], B.shape[0]
     dev = A.device
@@ -474,10 +475,28 @@ def full_scores(A, B, row_bias=None, col_bias=None, col_scale=None, g=0.0, mater
     items = _FS_WS.get(key)
     if items is None:
         items = _FS_WS[key] = torch.empty(int(lib.dccf_full_scores_ws_floats(I)), dtype=torch.float32, device=dev)
+    eo, ei = exclude if exclude is not None else (None, None)
+    if ei is not None and ei.numel() == 0:      # no listed item anywhere: a valid address that is never read
+        ei = torch.zeros(1, dtype=torch.int32, device=dev)
     check(lib.dccf_full_scores(U, I, ptr(A), ptr(B), ptr(row_bias), ptr(col_bias), ptr(col_scale), float(g), ptr(out),
-                               int(k), ptr(ts), ptr(ti), ptr(ws), ptr(wi), ptr(items), stream_ptr()), 'dccf_full_scores')
+                               int(k), ptr(ts), ptr(ti), ptr(ws), ptr(wi), ptr(items), ptr(eo), ptr(ei), stream_ptr()),
+          'dccf_full_scores')
     LAUNCHES[0] += 3 if k > 0 else 2
     return out, ts, ti
+
+
+def topk_metrics(topk_id, pos_off, pos_items, ks, out_metrics=None, out_sums=None, out_count=None):
+    """Every metric at every k of `ks` (ascending, <= 4 values, each <= the list length) of ranked top-k lists against
+    each user's sorted positives (dccf_topk_metrics, one launch): per-user values [n_users, n_k, 5], their sums over the
+    users with a positive [n_k, 5] and / or the number of those users (int64 [1])."""
+    lib = _lib.load()
+    n_users, k_list = topk_id.shape
+    arr = (ctypes.c_int32 * len(ks))(*[int(k) for k in ks])
+    ws = rank_workspace(topk_id.device) if out_sums is not None else None
+    check(lib.dccf_topk_metrics(ptr(topk_id), int(n_users), int(k_list), ptr(pos_off), ptr(pos_items), arr, len(ks),
+                                ptr(out_metrics), ptr(ws), ptr(out_sums), ptr(out_count), stream_ptr()),
+          'dccf_topk_metrics')
+    LAUNCHES[0] += 1 if n_users > 0 else 0
 
 
 def dp_push(send, seg, peer_bases, world, rank, flag_off, epoch_dev, cta_counter):

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 37
+#define DCCF_ABI_VERSION 38
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -447,6 +447,22 @@ int dccf_rank_eval_multi(const float* scores, const float* labels, const int64_t
                          const int64_t* user_off, int64_t n_users, const int32_t* ks, int32_t n_k,
                          int64_t* out_topk_iid, int32_t* out_topk_row, double* out_metrics, void* ws,
                          double* out_sums, void* stream);
+/* Ranking metrics of full-catalogue top-k lists (dccf_full_scores with known-item exclusion) against held-out
+ * positives, with the definitions of dccf_rank_eval_multi applied to the ranked list of every rankable item (label 1
+ * for a positive):
+ *   topk_id  [n_users, k_list] int64: score descending, ties by item id ascending, -1 padded; 1 <= k_list <= 16
+ *   pos_off  [n_users+1] int64, pos_items int32: each user's positives, ascending and unique (a CSR over the same rows)
+ *   ks       HOST array of n_k (1..4) strictly ascending values of k, each <= k_list
+ *   ndcg = DCG / IDCG with IDCG = sum_{j < min(n_pos, k)} 1 / log2(j + 2); hit; precision = hits / k;
+ *   recall = hits / n_pos; f1 = 2 hits / (k + n_pos).  Users with n_pos == 0 are not counted.
+ *   out_metrics [n_users, n_k, 5] f64 (may be NULL; NaN in the rows of users not counted)
+ *   out_sums    [n_k, 5] f64, summed in a fixed order as dccf_rank_eval_multi does (may be NULL)
+ *   out_count   device int64: the number of users counted (may be NULL)
+ *   ws          the workspace of dccf_rank_eval_multi (dccf_rank_eval_ws_bytes, zero on first use); required with
+ *               out_sums */
+int dccf_topk_metrics(const int64_t* topk_id, int64_t n_users, int32_t k_list, const int64_t* pos_off,
+                      const int32_t* pos_items, const int32_t* ks, int32_t n_k, double* out_metrics, void* ws,
+                      double* out_sums, int64_t* out_count, void* stream);
 
 /* ---- data-parallel gradient exchange over NVLink peer memory (new: the reference is single-GPU) ----- */
 /* Every rank owns a symmetric buffer of floats: [ recv: world*seg | flag area of dccf_dp_flag_floats() words ] mapped on
@@ -490,12 +506,17 @@ int dccf_dp_done(const uint64_t* peer_bases, int32_t world, int32_t rank, int64_
  *              split and half of an item tile, merged by a second launch); required with topk_score
  *   ws_items:  dccf_full_scores_ws_floats(n_items) floats, 128-byte aligned: the item side pre-split into the TF32 hi / lo
  *              operand images the tensor cores read (written once per call by k_fs_prep_b, streamed by the GEMM's
- *              CTAs with cp.async.bulk) */
+ *              CTAs with cp.async.bulk)
+ *   excl_off [U+1] int64, excl_items int32: known-item exclusion for the fused top-k, a CSR over the rows of A (each
+ *              row's items ascending, unique, < n_items); those items never enter the row's list, and a row with fewer
+ *              than k other items is -1 padded.  Both NULL: no exclusion.  Rejected together with `out`.  A list
+ *              that is not sorted may fail to exclude some of its items but is never read outside [off[u], off[u+1]). */
 int32_t dccf_full_scores_splits(int32_t n_users, int32_t n_items);
 int64_t dccf_full_scores_ws_floats(int32_t n_items);
 int dccf_full_scores(int32_t n_users, int32_t n_items, const float* A, const float* B, const float* row_bias,
                      const float* col_bias, const float* col_scale, float g, float* out, int32_t k,
-                     float* topk_score, int64_t* topk_id, float* ws_score, int64_t* ws_id, float* ws_items, void* stream);
+                     float* topk_score, int64_t* topk_id, float* ws_score, int64_t* ws_id, float* ws_items,
+                     const int64_t* excl_off, const int32_t* excl_items, void* stream);
 
 /* ---- host side: exact replay of the reference's negative sampler ---------------------------- */
 /* Replaces the Python loop of src/data_processor/DataProcessor.py:446-524 draw for draw.  HOST pointers.
