@@ -1134,18 +1134,25 @@ extern "C" int dccf_train_fwd_bwd_tc(const dccf_dims* dims, const float* E_user,
     const int Z = dims->n_samples + 1, R = Z * dims->n_attr, K = D + dims->feat_dim;
     const size_t smem = train_mid_smem_floats(R, Z, loss_mode == 0 ? 2 : 1) * sizeof(float);
     DCCF_CHECK_ARG(smem <= 200 * 1024, "dccf_train_fwd_bwd_tc: S=%d A=%d need %zu bytes of shared memory per CTA; use dccf_train_fwd_tc + dccf_train_bwd_tc", dims->n_samples, dims->n_attr, smem);
-    static size_t smem_opted = 0;
-    if (smem_opted == 0) {
+    // the middle kernel's carveout and the largest dynamic shared memory opted in so far, per device (indexed as
+    // PerDeviceOnce): an opt-in made on one GPU does not carry over to the next one a process drives
+    struct MidSmemOptIn { bool carveout; size_t bytes; };
+    static MidSmemOptIn mid_opted[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    MidSmemOptIn& opted = mid_opted[dev & 63];
+    if (!opted.carveout) {
         cudaFuncSetAttribute(k_train_mid, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        smem_opted = 48 * 1024;
+        opted.carveout = true;
+        opted.bytes = 48 * 1024;
     }
-    if (smem > smem_opted) {
+    if (smem > opted.bytes) {
         cudaError_t e = cudaFuncSetAttribute(k_train_mid, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) {
             set_error("dccf_train_fwd_bwd_tc: cannot opt in to %zu bytes of shared memory: %s", smem, cudaGetErrorString(e));
             return DCCF_ERR_CUDA;
         }
-        smem_opted = smem;
+        opted.bytes = smem;
     }
     int32_t n_ks = fwd_ksplits_for(n_pairs * R, K / TC_KC);
     if (phases & 1) {
