@@ -11,7 +11,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
-ABI_VERSION = 38
+ABI_VERSION = 39
 DIM = 64
 
 
@@ -126,6 +126,7 @@ _SIGNATURES = {
                                        ctypes.POINTER(Adam), _P]),
     'dccf_adam_step': (ctypes.c_int, [ctypes.POINTER(AdamTable), ctypes.c_int32, ctypes.POINTER(AdamTensor),
                                       ctypes.c_int32, ctypes.POINTER(Adam), _P]),
+    'dccf_adam_blocks': (ctypes.c_int32, [ctypes.c_int32, _P, _P, ctypes.c_int32, _P, ctypes.c_int32, _P, _P]),
     'dccf_adam_link_ids': (ctypes.c_int, [ctypes.POINTER(Dims), _P, _P, ctypes.c_int64, ctypes.c_int32, ctypes.c_int64,
                                           ctypes.c_int32, _P, _P, _P, _P, ctypes.POINTER(Expo), _P, _P, _P, _P,
                                           ctypes.POINTER(LinkExtra), _P]),

@@ -54,10 +54,20 @@ __device__ __forceinline__ AdamScalars resolve_adam(const AdamHost& h) {
     return s;
 }
 
+// clip_grad_value_: clamp to [-clip, clip], NaN stays NaN as in torch.clamp (fmaxf / fminf would turn it into -clip, and
+// a diverged step would go on with finite parameters).  The .NaN forms of max / min cost what fmaxf / fminf cost; finite
+// values and +-inf clip as before.
+__device__ __forceinline__ float clip_value(float g, float clip) {
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(g), "f"(-clip));
+    asm("min.NaN.f32 %0, %0, %1;" : "+f"(r) : "f"(clip));
+    return r;
+}
+
 // one element of the update; g_sparse is the data-dependent part of the gradient
 __device__ __forceinline__ void adam_elem(float& p, float& m, float& v, float g_sparse, const AdamScalars& s) {
     float g = __fadd_rn(g_sparse, __fmul_rn(s.two_l2, p));       // + d/dp (l2 * sum p^2)
-    if (s.clip > 0.f) g = fminf(fmaxf(g, -s.clip), s.clip);      // clip_grad_value_
+    if (s.clip > 0.f) g = clip_value(g, s.clip);                 // clip_grad_value_
     g = fmaf(s.wd, p, g);                                        // Adam weight_decay: g + wd * p
     m = fmaf(s.w1, __fsub_rn(g, m), m);                          // exp_avg.lerp_(g, 1 - beta1)
     v = __fmul_rn(v, s.beta2);                                   // exp_avg_sq.mul_(beta2)
@@ -99,7 +109,7 @@ template <int R> __device__ __forceinline__ void rule_elem(float& p, float& m, f
         adam_elem(p, m, v, g_sparse, s);
     } else {
         float g = __fadd_rn(g_sparse, __fmul_rn(s.two_l2, p));   // same preamble as adam_elem
-        if (s.clip > 0.f) g = fminf(fmaxf(g, -s.clip), s.clip);
+        if (s.clip > 0.f) g = clip_value(g, s.clip);
         g = fmaf(s.wd, p, g);                                    // weight_decay: g + wd * p
         if constexpr (R == RULE_GD) {
             p = fmaf(s.step_size, g, p);                         // SGD: param.add_(g, alpha = -lr)
@@ -1105,9 +1115,39 @@ extern "C" int dccf_state_advance(int32_t* step_dev, uint64_t* offset_dev, uint6
     return DCCF_OK;
 }
 
+// CTAs of one table's range in a launch of `mode` (see marshal_adam).  total_rows / n_rec_all: over every table of the
+// launch.
+static int64_t table_blocks(int mode, int64_t n_rows, int64_t total_rows, int64_t n_rec, int64_t n_rec_all) {
+    int64_t want;
+    if (mode == 2) {
+        // 16 records (half-warps) per 256-thread CTA per trip; ALL tables and dense tensors of the launch together stay
+        // within one wave (three 256-thread CTAs of this kernel fit an SM: 444, of which the dense tensors take up to
+        // 149) — a second wave started only when first-wave CTAs retired (data-parallel steps: 533 CTAs)
+        const int64_t table_budget = 148 * 3 - 150;
+        want = (n_rec + 15) / 16;
+        const int64_t share = n_rec_all > 0 ? (table_budget * n_rec + n_rec_all - 1) / n_rec_all : 0;
+        if (want > share) want = share;
+        if (want < 1 && n_rec > 0) want = 1;
+    } else {
+        // CTAs for the table sweeps, shared in proportion to the row counts (mode 3: the wide untouched-row sweep)
+        const int64_t budget = (mode == 1) ? 148 : 148 * 8;
+        want = (n_rows + 31) / 32;                           // 32 rows per 256-thread CTA per trip
+        const int64_t share = total_rows > 0 ? (budget * n_rows + total_rows - 1) / total_rows : 0;
+        if (want > share) want = share;
+        if (want < 1 && n_rows > 0) want = 1;
+    }
+    return want;
+}
+
+// CTAs of one dense tensor's range (every mode)
+static int64_t dense_blocks(int64_t n) {
+    const int64_t want = (n + 255) / 256;
+    return want > 148 ? 148 : want;
+}
+
 // Validate and marshal the table / tensor descriptors.  mode 0: k_adam_all (sweep blocks over all rows);
 // 1: k_adam_untouched (sweep blocks, at most one 256-thread CTA per SM so that a tensor-core CTA of the forward /
-// backward fits beside it); 2: k_adam_touched (one half-warp per record).
+// backward fits beside it); 2: k_adam_touched (one half-warp per record); 3: the wide k_adam_untouched.
 static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t n_tables, const dccf_adam_tensor* dense,
                         int32_t n_dense, const dccf_adam* hp, int mode, AdamAllArgs& a, int32_t* blocks_out,
                         int32_t* link_blocks_out) {
@@ -1120,10 +1160,12 @@ static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t 
     DCCF_CHECK_ARG((n_tables == 0 || tables) && (n_dense == 0 || dense), "%s: null descriptor array", who);
     a.n_tables = n_tables;
     a.n_dense = n_dense;
-    int64_t total_rows = 0;
-    for (int i = 0; i < n_tables; ++i) total_rows += tables[i].n_rows > 0 ? tables[i].n_rows : 0;
+    int64_t total_rows = 0, n_rec_all = 0;
+    for (int i = 0; i < n_tables; ++i) {
+        total_rows += tables[i].n_rows > 0 ? tables[i].n_rows : 0;
+        n_rec_all += (int64_t)tables[i].n_seg * tables[i].seg_len;
+    }
     int32_t blocks = 0, link_blocks = 0;
-    const int64_t budget = (mode == 1) ? 148 : 148 * 8;   // CTAs for the table sweeps, shared in proportion to the row counts (mode 3: the wide untouched-row sweep)
     for (int i = 0; i < n_tables; ++i) {
         const dccf_adam_table& t = tables[i];
         DCCF_CHECK_ARG(t.table && t.head && (t.m || !need_m) && (t.v || !need_v), "%s: table %d has a null buffer (rule %d)", who, i, hp->rule);
@@ -1140,24 +1182,7 @@ static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t 
         const int n_csr = (t.rec_row != nullptr) + (t.csr_off != nullptr) + (t.csr != nullptr) + (t.csr_pool != nullptr);
         DCCF_CHECK_ARG(n_csr == 0 || n_csr == 4, "%s: table %d: the CSR buffers (rec_row, csr_off, csr, csr_pool) go together", who, i);
         o.rec_row = t.rec_row; o.csr_off = t.csr_off; o.csr = t.csr; o.csr_pool = t.csr_pool;
-        int64_t want;
-        if (mode == 2) {
-            // 16 records (half-warps) per 256-thread CTA per trip; ALL tables and dense tensors of the launch together stay
-            // within one wave (three 256-thread CTAs of this kernel fit an SM: 444, of which the dense tensors take up to
-            // 149) — a second wave started only when first-wave CTAs retired (data-parallel steps: 533 CTAs)
-            int64_t n_rec_all = 0;
-            for (int j = 0; j < n_tables; ++j) n_rec_all += (int64_t)tables[j].n_seg * tables[j].seg_len;
-            const int64_t table_budget = 148 * 3 - 150;
-            want = (n_rec + 15) / 16;
-            const int64_t share = n_rec_all > 0 ? (table_budget * n_rec + n_rec_all - 1) / n_rec_all : 0;
-            if (want > share) want = share;
-            if (want < 1 && n_rec > 0) want = 1;
-        } else {
-            want = (o.n_rows + 31) / 32;                           // 32 rows per 256-thread CTA per trip
-            int64_t share = total_rows > 0 ? (budget * o.n_rows + total_rows - 1) / total_rows : 0;
-            if (want > share) want = share;
-            if (want < 1 && o.n_rows > 0) want = 1;
-        }
+        const int64_t want = table_blocks(mode, o.n_rows, total_rows, n_rec, n_rec_all);
         o.block_lo = blocks; o.block_n = (int32_t)want; blocks += (int32_t)want;
         o.link_lo = link_blocks; o.link_n = (int32_t)((n_rec + 255) / 256); link_blocks += o.link_n;
     }
@@ -1168,13 +1193,35 @@ static int marshal_adam(const char* who, const dccf_adam_table* tables, int32_t 
         AdamDenseArgs& o = a.d[i];
         o.p = d.p; o.m = d.m; o.v = d.v; o.n = d.n > 0 ? d.n : 0; o.g_parts = d.g_parts; o.n_parts = d.n_parts;
         o.part_stride = d.part_stride;
-        int64_t want = (o.n + 255) / 256;
-        if (want > 148) want = 148;
+        const int64_t want = dense_blocks(o.n);
         o.block_lo = blocks; o.block_n = (int32_t)want; blocks += (int32_t)want;
     }
     *blocks_out = blocks;
     *link_blocks_out = link_blocks;
     return DCCF_OK;
+}
+
+extern "C" int32_t dccf_adam_blocks(int32_t mode, const int64_t* n_rows, const int64_t* n_rec, int32_t n_tables,
+                                    const int64_t* n_dense_elems, int32_t n_dense, int32_t* block_lo, int32_t* block_n) {
+    if (mode < 0 || mode > 3 || n_tables < 0 || n_tables > ADAM_MAX_T || n_dense < 0 || n_dense > ADAM_MAX_T ||
+        (n_tables > 0 && (n_rows == nullptr || n_rec == nullptr)) || (n_dense > 0 && n_dense_elems == nullptr) ||
+        (n_tables + n_dense > 0 && (block_lo == nullptr || block_n == nullptr)))
+        return -1;
+    int64_t total_rows = 0, n_rec_all = 0;
+    for (int i = 0; i < n_tables; ++i) {
+        if (n_rows[i] < 0 || n_rec[i] < 0) return -1;
+        total_rows += n_rows[i];
+        n_rec_all += n_rec[i];
+    }
+    for (int i = 0; i < n_dense; ++i)
+        if (n_dense_elems[i] < 0) return -1;
+    int32_t blocks = 0;
+    for (int i = 0; i < n_tables + n_dense; ++i) {
+        const int64_t want = i < n_tables ? table_blocks(mode, n_rows[i], total_rows, n_rec[i], n_rec_all)
+                                          : dense_blocks(n_dense_elems[i - n_tables]);
+        block_lo[i] = blocks; block_n[i] = (int32_t)want; blocks += (int32_t)want;
+    }
+    return blocks;
 }
 
 extern "C" int dccf_adam_step(const dccf_adam_table* tables, int32_t n_tables, const dccf_adam_tensor* dense,

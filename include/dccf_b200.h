@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 38
+#define DCCF_ABI_VERSION 39
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -303,6 +303,13 @@ typedef struct dccf_adam_tensor {
 } dccf_adam_tensor;
 int dccf_adam_step(const dccf_adam_table* tables, int32_t n_tables, const dccf_adam_tensor* dense,
                    int32_t n_dense, const dccf_adam* hp, void* stream);
+/* Host only, no CUDA call: the CTA ranges one launch of the optimizer step gives its tensors — tables first (n_rows,
+ * n_rec records each), then dense tensors (n_dense_elems each).  mode 0: dccf_adam_step; 1: dccf_adam_untouched
+ * (threads_per_cta >= 0); 2: dccf_adam_touched and dccf_adam_csr_build; 3: dccf_adam_untouched (threads_per_cta < 0,
+ * the wide sweep).  Only mode 2 reads n_rec; modes 0, 1 and 3 share the CTAs by n_rows.  Writes block_lo / block_n
+ * [n_tables + n_dense] and returns the grid size; -1 on a bad argument (a negative count among them). */
+int32_t dccf_adam_blocks(int32_t mode, const int64_t* n_rows, const int64_t* n_rec, int32_t n_tables,
+                         const int64_t* n_dense_elems, int32_t n_dense, int32_t* block_lo, int32_t* block_n);
 /* The same optimizer step split around the backward pass: the rows a step does not touch (99 % of both
  * embedding tables; their gradient is the l2 / weight-decay term only) are swept by dccf_adam_untouched on a
  * second stream WHILE the forward and backward run; the touched rows, W and b follow the backward.
