@@ -156,11 +156,11 @@ def make_problem(case, seed=0):
 # ------------------------------------------------------------------------------------------------------------------
 # float64 reference and its elementwise bounds
 # ------------------------------------------------------------------------------------------------------------------
-def reference(pb, noise, mask, mse_pairs, splits, save_h=None, c=C, W=None, b=None):
-    """float64 value of every output of one step, and what its bound is made of.  noise / mask: the float32 values the
-    kernels use (None: mode 0); mse_pairs: the MSE divisor; splits: [(row_lo, row_hi)] of the gW / gb partials;
-    save_h: the kernel's activations, which decide the gates of the kink elements.  W / b override pb's in the forward
-    only (the comparator's negative controls)."""
+def forward_reference(pb, noise, mask, save_h=None, c=C, W=None, b=None, noise_exact=False):
+    """float64 value of the forward (pre, h, w, s, pred) and what its bound is made of.  noise / mask: the float32
+    values the kernels use (None: mode 0); save_h: the kernel's activations, which decide the gates of the kink
+    elements.  W / b override pb's (the comparator's negative controls).  noise_exact: the kernel multiplies eps itself
+    into W_f (the tensor-core scorer) instead of the rounded sum fl(Feat + eps)."""
     S, A, F = pb['S'], pb['A'], pb['F']
     Z = S + 1
     R = Z * A
@@ -182,12 +182,12 @@ def reference(pb, noise, mask, mse_pairs, splits, save_h=None, c=C, W=None, b=No
     if noise is not None:
         # the kernels add the noise in float32: x = fl(Feat + eps), which the oracle then sees exactly
         feat = pb['Feat'][np.repeat(X[:, 1], R)]
-        noise_eff = (feat + noise).astype(np.float64) - feat.astype(np.float64)
+        noise_eff = noise.astype(np.float64) if noise_exact else \
+            (feat + noise).astype(np.float64) - feat.astype(np.float64)
     m = np.ones((N, D)) if mask is None else mask.astype(np.float64)
     fwd = O.predict(params, X, pb['si'], noise_eff, None if mask is None else m, A, dtype=np.float64, expo=expo)
-    x, pre, h, w, s, pred, items = fwd['x'], fwd['pre'], fwd['h'], fwd['w'], fwd['s'], fwd['pred'], fwd['items']
+    x, pre, h, w, items = fwd['x'], fwd['pre'], fwd['h'], fwd['w'], fwd['items']
     u = X[:, 0]
-    W64 = pb['W'].astype(np.float64)            # the backward's W (gi) is always the step's own
 
     absP = np.abs(x) @ np.abs(params['W']).T + np.abs(params['b'])
     kink = (np.abs(pre) <= c * UNIT * absP) & (m != 0)
@@ -205,6 +205,21 @@ def reference(pb, noise, mask, mse_pairs, splits, save_h=None, c=C, W=None, b=No
     else:
         v_abs = np.zeros_like(v)
     rho = 1.0 + np.abs(v - v.max(axis=1, keepdims=True)) + v_abs + v_abs.max(axis=1, keepdims=True)
+    return {'P': P, 'Z': Z, 'R': R, 'A': A, 'N': N, 'x': x, 'pre': pre, 'h': h, 'w': w, 's': fwd['s'],
+            'pred': fwd['pred'], 'save_h': h, 'save_w': w, 'm': m, 'absP': absP, 'kink': kink, 'gpos': gpos, 'gv': gv,
+            'live': live, 'rho': rho, 'eu_r': np.repeat(params['E_user'][u], R, axis=0), 'fwd': fwd, 'params': params,
+            'X': X, 'noise_eff': noise_eff, 'items': items, 'u': u}
+
+
+def reference(pb, noise, mask, mse_pairs, splits, save_h=None, c=C, W=None, b=None):
+    """float64 value of every output of one step, and what its bound is made of.  noise / mask: the float32 values the
+    kernels use (None: mode 0); mse_pairs: the MSE divisor; splits: [(row_lo, row_hi)] of the gW / gb partials;
+    save_h: the kernel's activations, which decide the gates of the kink elements.  W / b override pb's in the forward
+    only (the comparator's negative controls)."""
+    ref = forward_reference(pb, noise, mask, save_h=save_h, c=c, W=W, b=b)
+    P, Z, R, A, N = ref['P'], ref['Z'], ref['R'], ref['A'], ref['N']
+    x, h, w, pred, gv, eu_r, u = ref['x'], ref['h'], ref['w'], ref['pred'], ref['gv'], ref['eu_r'], ref['u']
+    W64 = pb['W'].astype(np.float64)            # the backward's W (gi) is always the step's own
 
     if pb['loss'] == 0:
         hb = P // 2
@@ -220,26 +235,24 @@ def reference(pb, noise, mask, mse_pairs, splits, save_h=None, c=C, W=None, b=No
         loss = float(np.sum(d * d) / mse_pairs)
     ds = dp[:, None] * w / A                                                   # [P, Z]
     ds_r = np.repeat(ds.reshape(-1), A)                                        # [N]
-    eu_r = np.repeat(params['E_user'][u], R, axis=0)                           # [N, D]
     dpre = ds_r[:, None] * eu_r * gv
     gu = (ds_r[:, None] * h).reshape(P, R, D).sum(axis=1)
     gi = (dpre.reshape(P, Z, A, D).sum(axis=2) @ W64[:, :D]).reshape(P * Z, D)
     gW = np.stack([dpre[lo:hi].T @ x[lo:hi] for lo, hi in splits])
     gb = np.stack([dpre[lo:hi].sum(axis=0) for lo, hi in splits])
 
-    return {'P': P, 'Z': Z, 'R': R, 'A': A, 'N': N, 'x': x, 'pre': pre, 'h': h, 'w': w, 's': s, 'pred': pred,
-            'save_h': h, 'save_w': w,
-            'm': m, 'absP': absP, 'kink': kink, 'gpos': gpos, 'gv': gv, 'live': live, 'rho': rho, 'loss_mode': pb['loss'],
-            'd': d, 'sig': sig, 'g': g, 'dp': dp, 'mse_pairs': mse_pairs, 'loss': loss, 'ds': ds, 'ds_r': ds_r,
-            'eu_r': eu_r, 'dpre': dpre, 'gu': gu, 'gi': gi, 'gW': gW, 'gb': gb, 'W': W64, 'splits': splits,
-            'ku': u.astype(np.int32), 'ki': items.reshape(-1).astype(np.int32), 'fwd': fwd, 'params': params,
-            'X': X, 'noise_eff': noise_eff}
+    ref.update({'loss_mode': pb['loss'], 'd': d, 'sig': sig, 'g': g, 'dp': dp, 'mse_pairs': mse_pairs, 'loss': loss,
+                'ds': ds, 'ds_r': ds_r, 'dpre': dpre, 'gu': gu, 'gi': gi, 'gW': gW, 'gb': gb, 'W': W64,
+                'splits': splits, 'ku': u.astype(np.int32), 'ki': ref['items'].reshape(-1).astype(np.int32)})
+    return ref
 
 
-def bounds(ref, eps):
-    """Elementwise error bounds of every output for a relative unit eps (= C * 2^-20), first order: each stage's bound
-    is eps times its absolute-value computation, plus its inputs' bounds carried through it, plus ULPS of the value."""
-    P, Z, R, A, N = ref['P'], ref['Z'], ref['R'], ref['A'], ref['N']
+def forward_bounds(ref, eps):
+    """Elementwise error bounds of the forward's outputs (save_h, save_w, pred) for a relative unit eps (= C * 2^-20),
+    first order: each stage's bound is eps times its absolute-value computation, plus its inputs' bounds carried
+    through it, plus ULPS of the value.  Also returns the bound of the row scores (Bs) and the softmax's relative
+    bound (rel_w), which the backward's bounds carry on."""
+    P, R, A = ref['P'], ref['R'], ref['A']
     h, w, s, m, eu_r = ref['h'], ref['w'], ref['s'], ref['m'], ref['eu_r']
     aeu = np.abs(eu_r)
     B = {}
@@ -248,13 +261,22 @@ def bounds(ref, eps):
     Bs = (Bh * aeu).sum(axis=1) + eps * (np.abs(h) * aeu).sum(axis=1)                       # [N] row scores
     rho = ref['rho']
     rel_w = eps * (rho + (w * rho).sum(axis=1, keepdims=True) + 1.0)                        # softmax, relative
-    Bw = rel_w * w + ULPS * w
-    B['save_w'] = Bw
+    B['save_w'] = rel_w * w + ULPS * w
     wr = np.repeat(w / A, A, axis=1)                                                        # [P, R]
     sr = np.abs(s.reshape(P, R))
-    Bpred = (wr * (Bs.reshape(P, R) + sr * np.repeat(rel_w, A, axis=1))).sum(axis=1) + eps * (wr * sr).sum(axis=1) \
-        + ULPS * np.abs(ref['pred'])
-    B['pred'] = Bpred
+    B['pred'] = (wr * (Bs.reshape(P, R) + sr * np.repeat(rel_w, A, axis=1))).sum(axis=1) \
+        + eps * (wr * sr).sum(axis=1) + ULPS * np.abs(ref['pred'])
+    return B, Bs, rel_w
+
+
+def bounds(ref, eps):
+    """Elementwise error bounds of every output for a relative unit eps (= C * 2^-20), first order: each stage's bound
+    is eps times its absolute-value computation, plus its inputs' bounds carried through it, plus ULPS of the value."""
+    P, Z, R, A, N = ref['P'], ref['Z'], ref['R'], ref['A'], ref['N']
+    h, w, s, m, eu_r = ref['h'], ref['w'], ref['s'], ref['m'], ref['eu_r']
+    aeu = np.abs(eu_r)
+    B, Bs, rel_w = forward_bounds(ref, eps)
+    Bh, Bw, Bpred = B['save_h'], B['save_w'], B['pred']
     dp = ref['dp']
     if ref['loss_mode'] == 0:
         hb = P // 2
@@ -292,16 +314,17 @@ def bounds(ref, eps):
 OUTPUTS = ('pred', 'loss', 'save_h', 'save_w', 'dpre', 'gu', 'gi', 'gW', 'gb')
 
 
-def compare(got, ref, c=C):
-    """got: numpy outputs of one call (any subset of OUTPUTS, plus 'ku' / 'ki').  Returns (failures, observed): the
+def compare(got, ref, c=C, bounds_fn=bounds, outputs=OUTPUTS):
+    """got: numpy outputs of one call (any subset of `outputs`, plus 'ku' / 'ki').  Returns (failures, observed): the
     list of failed checks (empty = pass) and, per output, the smallest C its elements need (inf: an element that must
-    be exact is not)."""
-    B0 = bounds(ref, 0.0)
-    B1 = bounds(ref, UNIT)
+    be exact is not).  c: one C for every output or a dict of them; bounds_fn(ref, eps) -> {output: bound}."""
+    B0 = bounds_fn(ref, 0.0)
+    B1 = bounds_fn(ref, UNIT)
     fails, observed = [], {}
-    for k in OUTPUTS:
+    for k in outputs:
         if k not in got:
             continue
+        ck = c[k] if isinstance(c, dict) else c
         y = np.asarray(got[k], np.float64)
         r = np.asarray(ref[k], np.float64)
         if y.shape != r.shape:
@@ -314,12 +337,12 @@ def compare(got, ref, c=C):
         excess = err - b0
         need = np.where(excess <= 0, 0.0, np.where(slope > 0, excess / np.where(slope > 0, slope, 1.0), np.inf))
         observed[k] = float(need.max()) if need.size else 0.0
-        bad = ~(err <= b0 + c * slope)
+        bad = ~(err <= b0 + ck * slope)
         if bad.any():
             i = np.unravel_index(int(np.argmax(np.where(bad, need, -1.0))), y.shape) if y.ndim else ()
             fails.append('%s: %d of %d elements outside the bound; worst at %s: kernel %r, reference %r, bound %.3g '
                          '(needs C = %.3g)' % (k, int(bad.sum()), bad.size, tuple(int(t) for t in i), float(y[i]),
-                                               float(r[i]), float(b0[i] + c * slope[i]), float(need[i])))
+                                               float(r[i]), float(b0[i] + ck * slope[i]), float(need[i])))
     for k in ('ku', 'ki'):
         if k in got and not np.array_equal(np.asarray(got[k]), ref[k]):
             fails.append('%s: record keys differ at %d places' % (k, int((np.asarray(got[k]) != ref[k]).sum())))
