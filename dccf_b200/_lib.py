@@ -11,7 +11,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libdccf_b200.so')
-ABI_VERSION = 39
+ABI_VERSION = 40
 DIM = 64
 
 
@@ -153,6 +153,13 @@ _SIGNATURES = {
     'dccf_full_scores_ws_floats': (ctypes.c_int64, [ctypes.c_int32]),
     'dccf_full_scores': (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, _P, _P, _P, _P, _P, ctypes.c_float, _P,
                                         ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'dccf_mf_step_ctas': (ctypes.c_int32, [ctypes.c_int64]),
+    'dccf_mf_step': (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, _P, _P, _P, _P, _P, _P, ctypes.c_float, _P, _P,
+                                    ctypes.c_int64, ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    'dccf_mf_bias_grad': (ctypes.c_int, [ctypes.POINTER(AdamTable), ctypes.POINTER(AdamTable), _P, _P, _P, _P,
+                                         ctypes.c_int32, ctypes.c_float, _P, _P]),
+    'dccf_mf_scores': (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(Expo), _P, _P, ctypes.c_int64, _P,
+                                      _P, _P]),
     'dccf_sample_negatives': (ctypes.c_int, [_P, _P, _P, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int64,
                                              ctypes.c_int64, _P, _P, _P, _P, _P]),
     'dccf_confounder_draw': (ctypes.c_int, [_P, _P, _P, ctypes.c_int64, ctypes.c_int64, _P]),

@@ -415,6 +415,44 @@ def state_advance(step_dev, offset_dev, offset_inc=1):
     LAUNCHES[0] += 1
 
 
+def mf_step_ctas(n_pairs):
+    """Number of CTA partials (global_bias gradient, loss) of dccf_mf_step for a batch of n_pairs."""
+    return int(_lib.load().dccf_mf_step_ctas(int(n_pairs)))
+
+
+def mf_step(E_user, E_item, user_bias, item_bias, global_bias, propensity, M, X, Y, loss_mode, out_pred, gu_rec, gi_rec,
+            gb_rec, keys_u, keys_i, g_part, loss_part, err_flag=None):
+    """Forward, loss and backward of one BiasedMF / IPSBiasedMF batch (dccf_mf_step, one launch)."""
+    lib = _lib.load()
+    n_pairs = X.shape[0]
+    check(lib.dccf_mf_step(E_user.shape[0], E_item.shape[0], ptr(E_user), ptr(E_item), ptr(user_bias), ptr(item_bias),
+                           ptr(global_bias), ptr(propensity), float(M), ptr(X), ptr(Y), n_pairs, int(loss_mode),
+                           ptr(out_pred), ptr(gu_rec), ptr(gi_rec), ptr(gb_rec), ptr(keys_u), ptr(keys_i), ptr(g_part),
+                           ptr(loss_part), ptr(err_flag), stream_ptr()), 'dccf_mf_step')
+    LAUNCHES[0] += 1 if n_pairs > 0 else 0
+
+
+def mf_bias_grad(user_table, item_table, gb_rec, g_user_bias, g_item_bias, loss_part, n_loss_part, loss_scale, out_loss):
+    """Dense bias gradients from the CSR record lists of the two embedding tables (AdamTable descriptors) and the loss
+    (dccf_mf_bias_grad, one launch)."""
+    lib = _lib.load()
+    check(lib.dccf_mf_bias_grad(ctypes.byref(user_table), ctypes.byref(item_table), ptr(gb_rec), ptr(g_user_bias),
+                                ptr(g_item_bias), ptr(loss_part), int(n_loss_part), float(loss_scale), ptr(out_loss),
+                                stream_ptr()), 'dccf_mf_bias_grad')
+    LAUNCHES[0] += 1
+
+
+def mf_scores(factors, global_bias, X, out, err_flag=None):
+    """Predictions of the pairs X [P, 2] from IPS-MF factors (make_expo keys; global_bias a device tensor)."""
+    lib = _lib.load()
+    e = make_expo(ipsmf=dict(factors, mf_global_bias=0.0))
+    n_pairs = X.shape[0]
+    check(lib.dccf_mf_scores(factors['mf_user'].shape[0], factors['mf_item'].shape[0], ctypes.byref(e), ptr(global_bias),
+                             ptr(X), n_pairs, ptr(out), ptr(err_flag), stream_ptr()), 'dccf_mf_scores')
+    LAUNCHES[0] += 1 if n_pairs > 0 else 0
+    return out
+
+
 def rank_eval(scores, labels, iids, cand_rows, user_off, k, out_metrics, out_topk_iid=None, out_topk_row=None):
     """One k; cand_rows None = rows already grouped by user (candidate c is row c)."""
     lib = _lib.load()

@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define DCCF_ABI_VERSION 39
+#define DCCF_ABI_VERSION 40
 #define DCCF_DIM 64 /* u_vector_size == i_vector_size compiled into the kernels */
 
 typedef enum dccf_status {
@@ -524,6 +524,36 @@ int dccf_full_scores(int32_t n_users, int32_t n_items, const float* A, const flo
                      const float* col_bias, const float* col_scale, float g, float* out, int32_t k,
                      float* topk_score, int64_t* topk_id, float* ws_score, int64_t* ws_id, float* ws_items,
                      const int64_t* excl_off, const int32_t* excl_items, void* stream);
+
+/* ---- exposure models: BiasedMF / IPSBiasedMF training and scoring ------------------------------- */
+/* The model whose U x I prediction is <ds>.ips_expo_prob.npy (README.md:27-29; src/models/IPSBiasedMF.py:37-57):
+ *   pred = (<p_u, q_i> + b_u + b_i + g) / max(propensity_i, M)      (BiasedMF: propensity 1, M = 1)
+ * One training step is the split optimizer step above with S = 0 (record p = user row and item row of pair p):
+ *   dccf_adam_link_ids (CSR counting mode) -> dccf_adam_untouched -> dccf_adam_csr_build -> dccf_mf_step ->
+ *   dccf_mf_bias_grad -> dccf_adam_touched(tables: E_user, E_item; dense: user_bias [U], item_bias [I] with one partial
+ *   each, global_bias [1] with the dccf_mf_step_ctas(P) CTA partials, part_stride 1).
+ * dccf_mf_step: forward, loss and backward of one batch in one launch (loss_mode 0 BPR over [pos ; neg] halves, P even;
+ *   1 MSE mean against Y [P]).  global_bias is a DEVICE pointer to the 0-d parameter (graph replay).
+ *   out_pred [P]; gu_rec / gi_rec [P, D]: d loss / d p_u, d loss / d q_i of pair p; gb_rec [P]: d loss / d pred / max(prop, M)
+ *   (the gradient of b_u, b_i and g from pair p); rec_keys_u / rec_keys_i [P] int32: the rows (out-of-range ids are
+ *   clamped to row 0 and raise err_flag, as dccf_adam_link_ids clamps them); g_part / loss_part
+ *   [dccf_mf_step_ctas(P)]: per-CTA sums of gb_rec and of the loss terms.
+ * dccf_mf_bias_grad: dense d loss / d b_u [U] and d loss / d b_i [I] — the scalar records of each row summed in ascending
+ *   record index through the CSR that dccf_adam_csr_build built for `user` / `item` (0 for untouched rows) — and
+ *   out_loss[0] = loss_scale * sum of the loss partials in index order.  Between dccf_adam_csr_build and dccf_adam_touched.
+ * dccf_mf_scores: out[p] = pred of pair X[p] with the arithmetic of the DCCF kernels' exposure mode 1; factors->
+ *   mf_global_bias is ignored, the value is read from global_bias (device). */
+int32_t dccf_mf_step_ctas(int64_t n_pairs);
+int dccf_mf_step(int32_t n_users, int32_t n_items, const float* E_user, const float* E_item, const float* user_bias,
+                 const float* item_bias, const float* global_bias, const float* propensity, float min_propensity,
+                 const int64_t* X, const float* Y, int64_t n_pairs, int32_t loss_mode, float* out_pred, float* gu_rec,
+                 float* gi_rec, float* gb_rec, int32_t* rec_keys_u, int32_t* rec_keys_i, float* g_part, float* loss_part,
+                 int32_t* err_flag, void* stream);
+int dccf_mf_bias_grad(const dccf_adam_table* user, const dccf_adam_table* item, const float* gb_rec, float* g_user_bias,
+                      float* g_item_bias, const float* loss_part, int32_t n_loss_part, float loss_scale, float* out_loss,
+                      void* stream);
+int dccf_mf_scores(int32_t n_users, int32_t n_items, const dccf_expo* factors, const float* global_bias, const int64_t* X,
+                   int64_t n_pairs, float* out, int32_t* err_flag, void* stream);
 
 /* ---- host side: exact replay of the reference's negative sampler ---------------------------- */
 /* Replaces the Python loop of src/data_processor/DataProcessor.py:446-524 draw for draw.  HOST pointers.

@@ -46,11 +46,13 @@ from dccf_b200.data_loaders.DataLoader import DataLoader  # noqa: E402,F401
 from dccf_b200.models.BaseModel import BaseModel  # noqa: E402,F401
 from dccf_b200.models.RecModel import RecModel  # noqa: E402,F401
 from dccf_b200.models.DCCF import DCCF  # noqa: E402,F401
+from dccf_b200.models.BiasedMF import BiasedMF  # noqa: E402,F401
+from dccf_b200.models.IPSBiasedMF import IPSBiasedMF  # noqa: E402,F401
 from dccf_b200.runners.BaseRunner import BaseRunner  # noqa: E402,F401
 from dccf_b200.data_processor.DataProcessor import DataProcessor  # noqa: E402,F401
 
 _CLASSES = {'DataLoader': DataLoader, 'BaseModel': BaseModel, 'RecModel': RecModel, 'DCCF': DCCF,
-            'BaseRunner': BaseRunner, 'DataProcessor': DataProcessor}
+            'BiasedMF': BiasedMF, 'IPSBiasedMF': IPSBiasedMF, 'BaseRunner': BaseRunner, 'DataProcessor': DataProcessor}
 
 
 def _resolve(name):
@@ -144,8 +146,14 @@ def main(argv=None):
     if init_args.model_name in ['BaseModel']:
         model = model_name(label_min=data_loader.label_min, label_max=data_loader.label_max,
                            feature_num=len(features), random_seed=args.random_seed, model_path=args.model_path)
-    elif init_args.model_name in ['RecModel']:
+    elif init_args.model_name in ['RecModel', 'BiasedMF']:
         model = model_name(label_min=data_loader.label_min, label_max=data_loader.label_max, feature_num=0,
+                           user_num=data_loader.user_num, item_num=data_loader.item_num,
+                           u_vector_size=args.u_vector_size, i_vector_size=args.i_vector_size,
+                           random_seed=args.random_seed, model_path=args.model_path)
+    elif init_args.model_name in ['IPSBiasedMF']:
+        model = model_name(path=data_loader.path, dataset=data_loader.dataset, M=args.M,
+                           label_min=data_loader.label_min, label_max=data_loader.label_max, feature_num=0,
                            user_num=data_loader.user_num, item_num=data_loader.item_num,
                            u_vector_size=args.u_vector_size, i_vector_size=args.i_vector_size,
                            random_seed=args.random_seed, model_path=args.model_path)
