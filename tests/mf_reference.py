@@ -73,6 +73,40 @@ def gradients(params, X, Y, rank, prop=None, M=1.0, biases=True):
     return loss, pred, grads, mags, loss_mag
 
 
+def pairs(params, X, Y, rank, prop=None, M=1.0):
+    """Per-pair float64 terms of k_mf_step with tight first-order magnitudes (the `abs` of `gradients` bounds the
+    sigmoid's slope by 1/4; here it is sigma (1 - sigma), so that a pair far in the tail is judged on its own scale):
+    {'pred', 'scale', 'r' (the bias record d loss / d pred / scale), 'term' (the pair's loss term; 0 on the negative half
+    of a BPR batch), 'gu' [P, D] = r q_i, 'gi' [P, D] = r p_u} and 'A_<name>' for each: |x_fp32 - x| <~ 2^-24 A_x."""
+    P = len(X)
+    u, i = X[:, 0], X[:, 1]
+    pred, s, mag = forward(params, X, prop, M)
+    A_pred = mag + np.abs(pred)
+    if rank == 1:
+        b = P // 2
+        x = pred[:b] - pred[b:]
+        A_x = A_pred[:b] + A_pred[b:] + np.abs(x)
+        with np.errstate(over='ignore'):
+            sig = 1.0 / (1.0 + np.exp(x))                        # sigmoid(-x)
+        slope = sig * (1.0 - sig)
+        dl = np.concatenate([-sig, sig])
+        A_dl = np.concatenate([sig + slope * A_x] * 2)
+        t = np.logaddexp(0.0, -x)
+        term = np.concatenate([t, np.zeros(b)])
+        A_term = np.concatenate([t + sig * A_x, np.zeros(b)])
+    else:
+        e = pred - np.asarray(Y, np.float64)
+        A_e = A_pred + np.abs(np.asarray(Y, np.float64)) + np.abs(e)
+        dl, A_dl = 2.0 * e / P, 2.0 * A_e / P
+        term, A_term = e * e, 2.0 * np.abs(e) * A_e
+    r = dl / s
+    A_r = A_dl / s + np.abs(r)
+    pu, qi = params['E_user'][u], params['E_item'][i]
+    gu, gi = r[:, None] * qi, r[:, None] * pu
+    return {'pred': pred, 'A_pred': A_pred, 'scale': s, 'r': r, 'A_r': A_r, 'term': term, 'A_term': A_term,
+            'gu': gu, 'A_gu': A_r[:, None] * np.abs(qi) + np.abs(gu), 'gi': gi, 'A_gi': A_r[:, None] * np.abs(pu) + np.abs(gi)}
+
+
 def apply_rule(p, st, gs, t, hp, kind):
     """One element-wise update of the runner's step; returns (new p, new state, g after l2 / clip / weight decay)."""
     g = np.clip(gs + 2.0 * hp['l2'] * p, -hp.get('clip', 50.0), hp.get('clip', 50.0)) + hp['weight_decay'] * p
